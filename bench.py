@@ -4,6 +4,7 @@ NDCG@10 / Recall@20 on a synthetic ML-25M-shape matrix (BASELINE.json configs[1]
 
   python bench.py --gpus N --steps K --warmup W            # this repo, N GPUs (torchrun for N > 1)
   python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle restatement)
+  python bench.py --steps K --warmup W --dump-outputs DIR  # also writes the last timed step's results to DIR/*.npy
 
 One "step" = one full pass: fit of this rank's item rows, all-gather of the pruned similarity lists
 (N > 1), scoring + top-20 + NDCG@10 / Recall@20 of this rank's users, all-reduce of the metric sums.
@@ -32,7 +33,7 @@ N_LIST = 20
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (full passes); the e2e leg times as many")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--shape", default="ml25m", help="ml100k | ml1m | ml25m | netflix | msd | large (recpack_b200/synth.py SHAPES)")
@@ -44,7 +45,14 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--ref-fraction", type=float, default=0.02, help="fraction of a full pass one step of the reference arm / CPU baseline does")
     ap.add_argument("--cpu-procs", type=int, default=0, help="worker processes of --impl reference's setup (0 = one per host core, at most 64)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs); "
+                                                          "one GPU only")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl b200 and --gpus 1")
+    return args
 
 
 def make_data(args):
@@ -369,6 +377,10 @@ def run_gpu(args):
         step_ms.append(ms)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        if world > 1:
+            raise SystemExit("--dump-outputs needs a single process (--gpus 1)")
+        dump_outputs(args.dump_outputs, fit_out, top_out, red)
     if args.trace:  # one more step with the library's marks on (after the timed region)
         eng.trace(True)
         one_step(False)
@@ -389,7 +401,7 @@ def run_gpu(args):
     # ---- end to end through the public classes, host inputs (N = 1 rank-local: each rank does its shard)
     e2e = None
     if not args.no_e2e and world == 1:
-        e2e = run_e2e(args, train, test_out, eng, steps=max(3, min(args.steps, 5)))
+        e2e = run_e2e(args, train, test_out, eng, steps=args.steps)
     elif not args.no_e2e:
         # N > 1: the same sharded step through the C ABI with HOST input buffers (pinned), every copy inside the
         # timed region, wall clock bracketed by barriers, max over ranks
@@ -404,7 +416,7 @@ def run_gpu(args):
         h_top_len = torch.empty((nU,), dtype=torch.int32).pin_memory()
         e_times = []
         e_red = None
-        for s_ in range(max(3, min(args.steps, 5)) + 1):
+        for s_ in range(args.steps + 1):
             barrier()
             t0 = time.perf_counter()
             eng.fit_topk(U, I, hx_ptr.numpy(), hx_idx.numpy(), K_NEIGH, similarity=SIM, item_begin=ib, item_end=ie, out=fit_out)
@@ -503,6 +515,45 @@ def run_gpu(args):
         _emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 60_000_000  # all files of --dump-outputs together stay below 64 MB (.npy headers included)
+
+
+def dump_outputs(out_dir, fit_out, top_out, red):
+    """What the last timed step computed, as DIR/<name>.npy in float64 (ids and counts are exact):
+
+      metric_sums                          [sum of NDCG@10, sum of Recall@20, evaluated users]
+      topn_users, topn_idx, topn_len       top-N lists (-1 padded) of every user, or of a seeded sample of users
+      fit_items, fit_idx, fit_val, fit_len top-K similarity lists (-1 padded) of every item row, or of a seeded sample
+
+    The samples depend only on the shape and the arguments, so two builds run with the same arguments write
+    the same rows and their files can be compared one to one."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+
+    def sample(n, row_bytes):
+        keep = min(n, max(1, DUMP_BYTES // 2 // row_bytes))  # half for the top-N lists, half for the similarity lists
+        if keep == n:
+            return np.arange(n, dtype=np.int64)
+        return np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+
+    def rows_of(t, sel):
+        return t[torch.from_numpy(sel).to(t.device)].cpu().numpy().astype(np.float64)
+
+    nU, N = top_out["idx"].shape
+    I, K = fit_out["idx"].shape
+    users = sample(nU, 8 * (N + 2))
+    items = sample(I, 8 * (2 * K + 2))
+    arrays = {
+        "metric_sums": np.asarray(red, dtype=np.float64),
+        "topn_users": users.astype(np.float64), "topn_idx": rows_of(top_out["idx"], users), "topn_len": rows_of(top_out["len"], users),
+        "fit_items": items.astype(np.float64), "fit_idx": rows_of(fit_out["idx"], items), "fit_val": rows_of(fit_out["val"], items),
+        "fit_len": rows_of(fit_out["len"], items),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_e2e(args, train, test_out, eng, steps):

@@ -594,18 +594,21 @@ def ref_fraction_split_mask(user_ix: np.ndarray, in_frac: float, seed: int) -> n
 # --------------------------------------------------------------------------
 # Tie-aware comparison against the unmodified reference (SURVEY.md 8c (3))
 # --------------------------------------------------------------------------
-def compare_topk_tie_aware(ref_S: csr_matrix, got, Xb: csr_matrix, similarity="cosine", rel=1e-5):
+def compare_topk_tie_aware(ref_S: csr_matrix, got, Xb: csr_matrix, similarity="cosine", rel=1e-5, rows=None):
     """Compare reference top-K rows (arbitrary ties) with canonical lists ``got``.
 
     Per row: the sorted kept values must agree to ``rel``; items kept by only one side
     must all sit in the boundary tie group (exact key equal to the K-th exact key, widened
     by 4*c*2^-53 relative because the reference's own sums carry that much rounding noise).
+    Row r of ``ref_S`` is item ``rows[r]`` (default: item r), so a sample of the reference's
+    rows can be checked against the full lists.
     Returns dict(rows_checked, rows_with_diff, max_rel_err)."""
     ref_S = csr_matrix(ref_S)
     n = item_counts(Xb)
     stats = {"rows_checked": 0, "rows_with_diff": 0, "max_rel_err": 0.0}
-    for i in range(ref_S.shape[0]):
-        lo, hi = ref_S.indptr[i], ref_S.indptr[i + 1]
+    for r in range(ref_S.shape[0]):
+        i = r if rows is None else int(rows[r])
+        lo, hi = ref_S.indptr[r], ref_S.indptr[r + 1]
         rj, rv = ref_S.indices[lo:hi], ref_S.data[lo:hi]
         m = int(got["len"][i])
         gj, gv, gc = got["idx"][i, :m], got["val"][i, :m], got["cnt"][i, :m]

@@ -91,7 +91,7 @@ def main():
         X = synth_interactions(U, I, nnz, seed=7)
         train, test_out = weak_generalization_split(X, 0.8, seed=11)
         if name == "mid_cosine":
-            # keep the committed fixture small: inputs + scalar metric values only
+            # keep the committed fixture small: inputs, scalar metric values and a seeded sample of 512 rows of S
             with warnings.catch_warnings():
                 warnings.simplefilter("ignore")
                 algo = ItemKNN(K=K).fit(train)
@@ -100,7 +100,10 @@ def main():
                 out = {}
                 pack("X", train, out)
                 pack("ytrue", test_out, out)
-                pack("S", algo.similarity_matrix_, out)
+                S = csr_matrix(algo.similarity_matrix_)
+                rows = np.sort(np.random.default_rng(0).choice(S.shape[0], size=512, replace=False))
+                pack("S", S[rows], out)
+                out["S_rows"] = rows.astype(np.int64)
                 out["K"] = np.array(K)
                 for cls, tag, k in ((NDCGK, "ndcg", 10), (RecallK, "recall", 20)):
                     m = cls(k)
