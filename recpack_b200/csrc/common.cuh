@@ -43,6 +43,7 @@ enum {
   DBG_MULTI_PASS = 4,  // fit / predict: at least two item-range passes
   DBG_SPLIT_ROWS = 8,  // fit: cut the heaviest rows into pieces even when they are small
   DBG_EXACT_SCORES = 16,  // predict: exact sums for every list even when only the lists are asked for
+  DBG_MANY_PASS = 32,     // predict (top-N): at least four item ranges
 };
 
 }  // namespace rpk

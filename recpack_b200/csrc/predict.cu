@@ -952,17 +952,21 @@ __global__ void __launch_bounds__(1024, 1) k_predict(PredParams p) {
 //      keeps every sum below 2^32, taken from a bound on the user's terms (sum over the history rows of the largest
 //      q of the row's segment).  Each term is within 1 of q / 2^s, so |a_j - score_j / 2^s| <= d (d = history
 //      length): a_x - a_y > 2d proves score_x > score_y.
-//   2. history items are zeroed, then two dense passes over the accumulators (16-byte loads, untouched vectors are
-//      skipped as a whole): a 2048-bin histogram finds the bin of the N-th largest sum, the second pass copies
-//      every item within 2d of that bin's lower edge to the survivor list and clears the accumulators.
-//   3. when the caller wants the lists only (no scores) and the survivors' sums are all more than 2d apart down to
-//      the (N+1)-th, their order is already proven: the sums themselves are written out.  Otherwise a second sweep
-//      over the rows adds the exact q of the survivors (two 20-bit limbs, native atomics) and they are ordered by
-//      their exact scores.
-// k_predict_merge orders the P per-range lists of a user; a user whose lists cannot be ordered with certainty
-// (approximate sums of different ranges too close) is scored again with exact sums.  4 bytes per slot let two CTAs
-// share an SM, so one CTA's latency-bound steps hide behind the other's atomics.  A user whose survivors do not fit
-// the list (huge groups of near-equal scores) is handed to the two-limb kernel.
+//   2. history items are zeroed, then the survivor threshold: either the range's own bound (the N-th largest of the
+//      per-thread maxima, two small histogram rounds) or, once the user's running list holds N entries, the bound
+//      carried from the earlier ranges (the N-th entry's lower end).  One dense pass copies every item at or above
+//      the threshold to the list and clears the accumulators.
+//   3. the survivors are merged into the running list.  Every key is an interval of the exact score: an approximate
+//      sum a stands for [(a - d) * 2^s, (a + d) * 2^s], an exact one for itself.  The list is ordered by upper end;
+//      when every neighbour pair down to the (N+1)-th is separated (or exact), its order is the exact order.
+//      Otherwise a second sweep over the rows adds the exact q of this range's survivors (two 20-bit limbs, native
+//      atomics) while their accumulators are still live.  Scores requested: every survivor takes the second sweep.
+// One work item is a whole user: the P ranges run one after the other on the same accumulators, the history is
+// fetched once, and the list is written out after the last range.  All ranges share one shift s (from the bound
+// over whole rows), so their approximate sums compare as plain integers.  A user whose order the approximate sums
+// of an earlier range (their accumulators are gone) leave open is run again with exact sums throughout.  4 bytes
+// per slot let two CTAs share an SM, so one CTA's latency-bound steps hide behind the other's atomics.  A user whose
+// survivors do not fit the list (huge groups of near-equal scores) is handed to the two-limb kernel.
 struct ExactOrder {
   __device__ __forceinline__ int cmp3(const Entry& a, const Entry& b) const {
     if (a.key != b.key) return a.key > b.key ? 1 : -1;
@@ -973,17 +977,16 @@ struct ExactOrder {
 struct Pred32Params {
   const int* indices;
   const u64* ent;        // model rows in 4-entry blocks, entries (q << 24) | column
-  const int4* blk;       // {first block, blocks, bound of q >> 20, 0} per (row, item range)
+  const int4* blk;       // {first block, blocks, bound of q >> 20, 0} per (row, item range), at row * P + range
   const int4* work_tab;  // {user, history length, row start lo, hi} in processing order
-  const int* n_work;     // non-null: number of work_tab records (device side), replaces U
   int U, P, R, I, N, mask;
-  int exact;             // 1: exact scores for every list (scores requested / second pass over flagged users)
+  int exact;             // 1: exact scores for every list (scores requested)
   int cap;
   int* queue;
-  int* part_idx;         // [U*P x N]
-  u64* part_key;         // exact sums; approximate sums where part_sft >= 0
-  int* part_len;         // [U*P]
-  int* part_sft;         // [U*P] -1: exact keys, s >= 0: keys are 32-bit sums of (q >> s) | 1
+  int* out_idx;          // [U x N] final lists
+  double* out_val;       // [U x N] scores (exact mode), or null
+  int* out_len;          // [U]
+  const ModelScale* scale;
   const unsigned char* item_ok;  // non-null: item filter (1 = may be recommended), padded to a multiple of 4 items
   int* ovf_flag;         // per user: 1 = handed to the two-limb kernel
   int* ovf_count;        // number of such users
@@ -1086,42 +1089,25 @@ __device__ __forceinline__ void sweep_rows(const u64* __restrict__ ent, const Ro
 __device__ __forceinline__ void rank_by_warps(const Entry* src, Entry* dst, int m) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   u64 kf = 0ull;
-  int jf = SENTINEL_IDX;
+  int jf = SENTINEL_IDX, af = 0;
   if (lane < m) {
     kf = src[lane].key;
     jf = src[lane].idx;
+    af = src[lane].aux;
   }
   for (int i = warp; i < m; i += nwarps) {
     const u64 ki = __shfl_sync(0xffffffffu, kf, i);
     const int ji = __shfl_sync(0xffffffffu, jf, i);
+    const int ai = __shfl_sync(0xffffffffu, af, i);
     const unsigned first = __ballot_sync(0xffffffffu, lane < m && (kf > ki || (kf == ki && jf < ji)));
     if (lane == 0) {
       Entry e;
       e.key = ki;
       e.idx = ji;
-      e.aux = 0;
+      e.aux = ai;
       dst[__popc(first)] = e;
     }
   }
-}
-
-// One warp: `sorted` holds m <= 32 entries best first.  Optionally checks that the first min(m - 1, N) neighbouring
-// keys are more than `margin` apart (the approximate sums then prove the order) and -- unless that check fails --
-// writes the first N places of the list.  Returns false when the check failed.
-__device__ __forceinline__ bool warp_check_write(const Entry* sorted, int m, int N, u64 margin, bool check, int* o_idx, u64* o_key) {
-  const int lane = threadIdx.x & 31;
-  if (check) {
-    const int pairs = (m - 1) < N ? (m - 1) : N;
-    bool bad = false;
-    for (int k = lane; k < pairs; k += 32) bad |= sorted[k].key - sorted[k + 1].key <= margin;
-    if (__any_sync(0xffffffffu, bad)) return false;
-  }
-  const int mo = m < N ? m : N;
-  for (int t = lane; t < N; t += 32) {
-    o_idx[t] = t < mo ? sorted[t].idx : -1;
-    o_key[t] = t < mo ? sorted[t].key : 0ull;
-  }
-  return true;
 }
 
 // Orders m entries best first by (key desc, index asc).  Up to SEL_RANK_MAX entries are ranked by counting
@@ -1169,31 +1155,54 @@ __host__ __device__ __forceinline__ size_t a32_fixed_bytes(int cap) {
   return sel_smem_bytes(cap, A32_BINS) + 2 * ((sizeof(RowTab) + 15) / 16) * 16;
 }
 
-// Work distribution: the items are sorted heaviest first; CTA b starts with item b and takes every further item from a
-// shared counter (longest-processing-time scheduling: the few users with five-digit histories then cost their CTAs
-// other items instead of coming on top of an equal share of everything -- that tail bounded the kernel once a rank's
-// shard became small).  The counter is read TWO items ahead by thread 0 and kept in a register, so the atomic's
-// latency hides behind a whole item and the next item can still be staged while the current one is swept.
-// Users with histories of at least A32_EXACT_D rows get their exact sums in the same work item: the margin 2 d of
-// their approximate sums never proves a list, and a second launch for them would run on a handful of CTAs.
+// Lower end of a key's interval (aux = 1: approximate key = upper end, the interval is W wide; aux = 0: exact).
+__device__ __forceinline__ u64 a32_lo(const Entry& e, u64 W) { return e.aux ? (e.key > W ? e.key - W : 0ull) : e.key; }
+
+// Orders list[0..m) best first by (upper end desc, index asc); returns where the result is (list or list2).
+// Barrier before (the entries are in place) and after.
+__device__ __forceinline__ Entry* a32_order(Entry* list, Entry* list2, int m) {
+  if (m <= 32) {
+    rank_by_warps(list, list2, m);
+    __syncthreads();
+    return list2;
+  }
+  return a32_sort(list, list2, m);
+}
+
+// True (in every thread) unless each neighbour pair of the first min(m - 1, N) places is proven: the first one's
+// interval lies strictly above the second one's, or both are exact (then the order by index decides ties).
+__device__ __forceinline__ bool a32_unproven(const Entry* s, int m, int N, u64 W) {
+  const int pairs = (m - 1) < N ? (m - 1) : N;
+  bool bad = false;
+  for (int k = threadIdx.x; k < pairs; k += blockDim.x)
+    if (s[k].aux | s[k + 1].aux) bad |= a32_lo(s[k], W) <= s[k + 1].key;
+  return __syncthreads_or(bad) != 0;
+}
+
+// Work distribution: the users are sorted heaviest first; CTA b starts with user b and takes every further user
+// from a shared counter (longest-processing-time scheduling: the few users with five-digit histories then cost
+// their CTAs other users instead of coming on top of an equal share of everything -- that tail bounded the kernel
+// once a rank's shard became small).  The counter is read TWO users ahead by thread 0, so the atomic's latency
+// hides behind a whole user and the next user can still be staged while the current one is swept.  Users with histories of at least A32_EXACT_D rows get exact sums from the start: the margin 2 d of their
+// approximate sums never proves a list.
 constexpr int A32_EXACT_D = 2048;
 
 __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
   extern __shared__ __align__(16) unsigned char smem[];
-  Entry* list = reinterpret_cast<Entry*>(smem);
+  Entry* list = reinterpret_cast<Entry*>(smem);  // the user's running list, then this range's survivors
   Entry* list2 = list + p.cap;  // SEL_RANK_MAX entries
   int* hist = reinterpret_cast<int*>(smem + sel_list_bytes(p.cap));
   SelShared* sh = reinterpret_cast<SelShared*>(hist + A32_BINS);
   RowTab* rtab = reinterpret_cast<RowTab*>(smem + sel_smem_bytes(p.cap, A32_BINS));
   unsigned* acc = reinterpret_cast<unsigned*>(smem + a32_fixed_bytes(p.cap));
-  __shared__ int s_flag3[3];  // "exact scores needed" of item k lives in s_flag3[k % 3]; reset two items ahead
   __shared__ int4 s_rec[2];
   __shared__ int s_w[2];
   __shared__ u64 s_bsum[2];       // bound of the sums, in units of 2^20: rows beyond the first chunk ...
   __shared__ unsigned s_bsum32[2];  // ... and the first chunk
+  __shared__ int s_pend;            // the user after the next one (thread 0 asks for it one user ahead of its use)
 
-  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5;
-  const int total = (p.n_work ? *p.n_work : p.U) * p.P;
+  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31;
+  const int total = p.U, P = p.P, N = p.N;
   const int G = gridDim.x, bid = blockIdx.x;
   if (bid >= total) return;
   uint4* acc4 = reinterpret_cast<uint4*>(acc);
@@ -1201,26 +1210,32 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
   const int nvec = p.R >> 2;  // R is a multiple of 4
   for (int v = tid; v < nvec; v += nt) acc4[v] = make_uint4(0u, 0u, 0u, 0u);
   for (int b = tid; b < A32_BINS; b += nt) hist[b] = 0;
-  int pend = total;  // thread 0: the item after the next one (fetched one item ahead of its use)
   if (tid == 0) {
     const int w0 = bid;
-    pend = G + atomicAdd(p.queue, 1);
+    s_pend = G + atomicAdd(p.queue, 1);
     s_w[0] = w0;
-    s_rec[0] = p.work_tab[w0 / p.P];
+    s_rec[0] = p.work_tab[w0];
     s_bsum[0] = 0ull;
     s_bsum[1] = 0ull;
     s_bsum32[0] = 0u;
     s_bsum32[1] = 0u;
-    s_flag3[0] = s_flag3[1] = s_flag3[2] = 0;
-    sh->count = 0;
-    sh->bstar = 0;
   }
   __syncthreads();
-  // ---- staging of a work item, in three parts so that its two dependent global loads (history item -> block
-  //      table entry) hide behind other work: part 1 issues the load of this thread's history item, part 2 the
-  //      load of that row's table entry, part 3 writes the row table and adds up the bound of the sums
+  // ---- staging of a user, in three parts so that its two dependent global loads (history item -> block table
+  //      entries) hide behind other work: part 1 issues the load of this thread's history item, part 2 the loads of
+  //      that row's table entries (all P ranges, adjacent), part 3 writes the row table of range 0 and adds up the
+  //      bound of the sums (largest q of each whole row)
   int st_item = -1;
-  int4 st_blk = make_int4(0, 0, 0, 0);
+  int2 st_seg = make_int2(0, 0);
+  unsigned st_bnd = 0;
+  auto row_bound = [&](int item, int2* seg0) {
+    const int4* b = p.blk + (int64_t)item * P;
+    const int4 b0 = __ldg(b);
+    unsigned z = (unsigned)b0.z;
+    for (int q = 1; q < P; ++q) z = max(z, (unsigned)__ldg(b + q).z);
+    if (seg0) *seg0 = make_int2(b0.x, b0.y);
+    return z;
+  };
   auto stage1 = [&](int buf) {
     st_item = -1;
     if (s_w[buf] < total) {
@@ -1230,26 +1245,27 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
     }
   };
   auto stage2 = [&](int buf) {
-    st_blk = make_int4(0, 0, 0, 0);
-    if (st_item >= 0) st_blk = __ldg(p.blk + (int64_t)st_item * p.P + (s_w[buf] % p.P));
+    st_seg = make_int2(0, 0);
+    st_bnd = 0;
+    if (st_item >= 0) st_bnd = row_bound(st_item, &st_seg);
   };
   auto stage3 = [&](int buf) {
     if (s_w[buf] >= total) return;
     const int4 rc = s_rec[buf];
-    const int d2 = rc.y, pass2 = s_w[buf] % p.P;
+    const int d2 = rc.y;
     const int64_t xb2 = ((int64_t)(unsigned)rc.z) | ((int64_t)rc.w << 32);
     RowTab* rt2 = rtab + buf;
     unsigned b32 = 0;  // first chunk: at most 512 terms of at most 2^20 each
     if (tid < d2) {
-      rt2->seg[tid] = make_int2(st_blk.x, st_blk.y);
+      rt2->seg[tid] = st_seg;
       rt2->item[tid] = st_item;
-      b32 = (unsigned)st_blk.z;
+      b32 = st_bnd;
     }
     b32 = __reduce_add_sync(0xffffffffu, b32);
     if (lane == 0 && b32) atomicAdd(&s_bsum32[buf], b32);
     if (d2 > nt) {  // long histories: the rows beyond the first chunk only add to the bound
       u64 bsum = 0;
-      for (int r = tid + nt; r < d2; r += nt) bsum += (u64)(unsigned)__ldg(p.blk + (int64_t)p.indices[xb2 + r] * p.P + pass2).z;
+      for (int r = tid + nt; r < d2; r += nt) bsum += (u64)row_bound(p.indices[xb2 + r], nullptr);
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) bsum += __shfl_xor_sync(0xffffffffu, bsum, o);
       if (lane == 0 && bsum) atomicAdd(&s_bsum[buf], bsum);
@@ -1264,20 +1280,19 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
 #endif
   for (int k = 0;; ++k) {
     const int cur = k & 1, nxt = cur ^ 1;
-    int& s_flag = s_flag3[k % 3];
     const int w = s_w[cur];
     if (w >= total) break;
     const int4 rec = s_rec[cur];
-    const RowTab* rt = rtab + cur;
-    // the next work item: its record is copied into shared memory asynchronously while this item is swept; the
-    // per-item scratch is reset here too (every thread has left the previous item, nobody reads these before the
+    RowTab* rt = rtab + cur;
+    // the next user: its record is copied into shared memory asynchronously while this one's first range is
+    // swept; its bound is reset here too (every thread has left the previous user, nobody reads these before the
     // barrier after the sweep)
     if (tid == 0) {
-      int w_n = pend;                    // asked for while the previous item was processed
-      pend = G + atomicAdd(p.queue, 1);  // used at the top of the next item
+      int w_n = s_pend;                    // asked for while the previous user was processed
+      s_pend = G + atomicAdd(p.queue, 1);  // used at the top of the next user
       if (w_n < total) {
         asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(&s_rec[nxt])),
-                     "l"(p.work_tab + w_n / p.P)
+                     "l"(p.work_tab + w_n)
                      : "memory");
       } else {
         w_n = total;
@@ -1286,21 +1301,26 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
       s_w[nxt] = w_n;
       s_bsum[nxt] = 0ull;
       s_bsum32[nxt] = 0u;
-      s_flag3[(k + 1) % 3] = 0;  // the next item's flag; the previous item's may still be read by slow threads
-      sh->count = 0;
-      sh->bstar = 0;
     }
     const int u = rec.x;
-    const int pass = w % p.P;
-    const int r0 = pass * p.R;
-    const int ns = min(p.R, p.I - r0);
     const int64_t xb = ((int64_t)(unsigned)rec.z) | ((int64_t)rec.w << 32);
     const int d = rec.y;
-    const int64_t slot_out = (int64_t)u * p.P + pass;
-    int* o_idx = p.part_idx + slot_out * p.N;
-    u64* o_key = p.part_key + slot_out * p.N;
     PROF32_MARK(0);
-    // ---- shift of the 32-bit sums from the bound staged with the item
+    if (d == 0) {  // user without history: empty prediction row (algorithms/base.py:123-127)
+      if (tid == 0) asm volatile("cp.async.wait_group 0;" ::: "memory");
+      __syncthreads();
+      stage1(nxt);
+      for (int t = tid; t < N; t += nt) {
+        p.out_idx[(int64_t)u * N + t] = -1;
+        if (p.out_val) p.out_val[(int64_t)u * N + t] = 0.0;
+      }
+      if (tid == 0) p.out_len[u] = 0;
+      stage2(nxt);
+      stage3(nxt);
+      __syncthreads();
+      continue;
+    }
+    // ---- shift of the 32-bit sums from the bound staged with the user
     // B = b20 * 2^20 >= sum over the rows of their largest q; the smallest shift with (B >> sft) + d < 2^32
     const u64 b20 = s_bsum[cur] + (u64)s_bsum32[cur];  // < 2^45 (d < 2^24 rows of at most 2^20 each)
     int sft = 0;
@@ -1316,18 +1336,25 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
     const int sh_a = 24 + sft;
     const unsigned margin = 2u * (unsigned)d;
     const u64 idle = (u64)(unsigned)(p.R + lane) << 2;
-    // ---- sweep 1: approximate sums, one fire-and-forget atomic per entry
-    if (d > 0) {
-      RowTab* rtw = rtab + cur;
+    bool uexact = p.exact != 0 || d >= A32_EXACT_D;
+    bool first = true;   // the user's first range: the next user is staged alongside
+    bool staged = true;  // the row table holds chunk 0 of the current range
+    bool own = false;    // the range takes its own bound even when a carried one exists
+    int r = 0;           // entries of the running list (list[0..r), best first, proven order)
+    for (int pass = 0; pass < P; ++pass) {
+      const int r0 = pass * p.R;
+      const int ns = min(p.R, p.I - r0);
+      if (tid == 0) sh->count = 0;
+      // ---- sweep 1: approximate sums, one fire-and-forget atomic per entry
       for (int c0 = 0; c0 < d; c0 += A32_ROWS) {
         const int n = min(A32_ROWS, d - c0);
-        if (c0 > 0) {
-          __syncthreads();  // the previous chunk's table is still being read
-          for (int r = tid; r < n; r += nt) {
-            const int i = p.indices[xb + c0 + r];
-            const int4 b = __ldg(p.blk + (int64_t)i * p.P + pass);
-            rtw->seg[r] = make_int2(b.x, b.y);
-            rtw->item[r] = i;
+        if (c0 > 0 || !staged) {
+          __syncthreads();  // the previous table is still being read
+          for (int rr = tid; rr < n; rr += nt) {
+            const int i = p.indices[xb + c0 + rr];
+            const int4 b = __ldg(p.blk + (int64_t)i * P + pass);
+            rt->seg[rr] = make_int2(b.x, b.y);
+            rt->item[rr] = i;
           }
           __syncthreads();
         }
@@ -1336,291 +1363,295 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
           asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(acc_s + ((unsigned)e & 0xffffffu)), "r"((unsigned)(e >> sh_a) | 1u) : "memory");
         });
       }
-    }
-    if (tid == 0) asm volatile("cp.async.wait_group 0;" ::: "memory");  // the next item's record has landed
-    __syncthreads();
-    PROF32_MARK(1);
-    stage1(nxt);
-    if (d == 0) {  // user without history: empty prediction row (algorithms/base.py:123-127)
-      for (int t = tid; t < p.N; t += nt) {
-        o_idx[t] = -1;
-        o_key[t] = 0;
-      }
-      if (tid == 0) {
-        p.part_len[slot_out] = 0;
-        p.part_sft[slot_out] = -1;
-      }
-      stage2(nxt);
-      stage3(nxt);
+      staged = d <= A32_ROWS;
+      if (tid == 0) asm volatile("cp.async.wait_group 0;" ::: "memory");  // the next user's record has landed
       __syncthreads();
-      continue;
-    }
-    if (p.mask) {  // pipelines/pipeline.py:174-175 -- before the truncation to N
-      if (d <= A32_ROWS) {
-        if (tid < d) {
-          const int j = rt->item[tid] - r0;
-          if (j >= 0 && j < ns) acc[j] = 0u;
-        }
-      } else {
-        for (int r = tid; r < d; r += nt) {
-          const int j = p.indices[xb + r] - r0;
-          if (j >= 0 && j < ns) acc[j] = 0u;
-        }
-      }
-      __syncthreads();
-    }
-    if (p.item_ok) {  // postprocessing/filters.py:58-101: filtered items are never recommended (4 items per word)
-      const unsigned* ok4 = reinterpret_cast<const unsigned*>(p.item_ok + r0);
-      for (int v = tid; v < nvec; v += nt) {
-        const unsigned okw = 4 * v < ns ? __ldg(ok4 + v) : 0x01010101u;
-        if (okw != 0x01010101u) {
-          uint4 x = acc4[v];
-          if (!(okw & 0xffu)) x.x = 0u;
-          if (!(okw & 0xff00u)) x.y = 0u;
-          if (!(okw & 0xff0000u)) x.z = 0u;
-          if (!(okw & 0xff000000u)) x.w = 0u;
-          acc4[v] = x;
-        }
-      }
-      __syncthreads();
-    }
-    PROF32_MARK(2);
-    // ---- survivors.  A dense pass costs a warp its full instruction stream whenever any of its lanes has work, so
-    //      the per-item work is kept out of it: every thread takes the maximum of its own slots (no branches, no
-    //      atomics), and the N-th largest of these per-thread maxima -- found with one histogram entry per thread,
-    //      64 bins per octave -- is a lower bound of the N-th largest sum (N distinct items reach it).  Everything
-    //      within the margin below that bin survives.
-    unsigned mymax = 0u;
-    for (int v = tid; v < nvec; v += nt) {
-      const uint4 x = acc4[v];
-      mymax = max(mymax, max(max(x.x, x.y), max(x.z, x.w)));
-    }
-    // N-th largest of the 512 per-thread maxima, in two rounds of a 32-bin histogram (octave, then 32 bins inside
-    // the octave).  Every warp scans the 32 bins by itself (one bin per lane), so no warp waits for another one
-    // beyond the two barriers.
-    const int mybin = mymax ? a32_bin(mymax) : -1;  // (octave << 5) | bin inside the octave
-    if (mybin >= 0) atomicAdd(&hist[mybin >> 5], 1);
-    __syncthreads();
-    PROF32_MARK(12);
-    stage2(nxt);
-    int bstar = 0;
-    {
-      const int h1 = hist[lane];
-      int incl = h1;  // maxima in my octave and the higher ones
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int t = __shfl_down_sync(0xffffffffu, incl, o);
-        if (lane + o < 32) incl += t;
-      }
-      const unsigned hit = __ballot_sync(0xffffffffu, incl >= p.N);  // lanes whose octave-and-above hold N maxima
-      if (hit) {
-        const int oct = 31 - __clz(hit);  // the highest such octave holds the N-th largest
-        const int above = __shfl_sync(0xffffffffu, incl - h1, oct);
-        if (mybin >= 0 && (mybin >> 5) == oct) atomicAdd(&hist[32 + (mybin & 31)], 1);
-        __syncthreads();
-        const int h2 = hist[32 + lane];
-        int incl2 = h2;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int t = __shfl_down_sync(0xffffffffu, incl2, o);
-          if (lane + o < 32) incl2 += t;
-        }
-        const unsigned hit2 = __ballot_sync(0xffffffffu, above + incl2 >= p.N);
-        bstar = (oct << 5) | (hit2 ? 31 - __clz(hit2) : 0);
-      } else {
-        __syncthreads();  // fewer than N non-empty threads: everything survives (bstar = 0)
-      }
-    }
-    __syncthreads();  // every warp has read both histograms
-    if (mybin >= 0) {
-      hist[mybin >> 5] = 0;
-      hist[32 + (mybin & 31)] = 0;
-    }
-    const unsigned edge = a32_bin_floor(bstar);
-    const unsigned thr = edge > margin + 1u ? edge - margin : 1u;
-    PROF32_MARK(13);
-    // copy the survivors, clear the accumulators: one compare per vector, the rest only for the few that pass
-    for (int v = tid; v < nvec; v += nt) {
-      const uint4 x = acc4[v];
-      acc4[v] = make_uint4(0u, 0u, 0u, 0u);
-      if (max(max(x.x, x.y), max(x.z, x.w)) < thr) continue;
-      const unsigned xs[4] = {x.x, x.y, x.z, x.w};
-#pragma unroll
-      for (int q = 0; q < 4; ++q)
-        if (xs[q] >= thr) {
-          const int pos = atomicAdd(&sh->count, 1);
-          if (pos < p.cap) {
-            Entry e;
-            e.key = (u64)xs[q];
-            e.idx = r0 + 4 * v + q;
-            e.aux = 0;
-            list[pos] = e;
+      PROF32_MARK(1);
+      if (first) stage1(nxt);
+      // the next range's table entry of this thread's row, written to the table once this range is done
+      const bool pre = d <= A32_ROWS && pass + 1 < P && tid < d;
+      if (pre) asm volatile("prefetch.global.L1 [%0];" ::"l"(p.blk + (int64_t)rt->item[tid] * P + pass + 1));
+      if (p.mask) {  // pipelines/pipeline.py:174-175 -- before the truncation to N
+        if (d <= A32_ROWS) {
+          if (tid < d) {
+            const int j = rt->item[tid] - r0;
+            if (j >= 0 && j < ns) acc[j] = 0u;
+          }
+        } else {
+          for (int rr = tid; rr < d; rr += nt) {
+            const int j = p.indices[xb + rr] - r0;
+            if (j >= 0 && j < ns) acc[j] = 0u;
           }
         }
-    }
-    PROF32_MARK(14);
-    stage3(nxt);
-    __syncthreads();
-    const int m = sh->count;
-    PROF32_MARK(3);
-#ifdef RPK_PHASE_PROF
-    if (tid == 0) {
-      atomicAdd(p.prof + 8, 1ull);
-      atomicAdd(p.prof + 11, (unsigned long long)(m > p.cap ? 0 : m));
-    }
-#endif
-    if (m > p.cap) {  // survivors do not fit: the exact kernel takes the whole user
-      if (tid == 0 && atomicExch(&p.ovf_flag[u], 1) == 0) p.ovf_tab[atomicAdd(p.ovf_count, 1)] = rec;
-      __syncthreads();
-      continue;
-    }
-    const int mo = m < p.N ? m : p.N;
-    bool need_exact = p.exact != 0 || d >= A32_EXACT_D;
-    Entry* surv = list;  // where the survivors are
-    if (!need_exact) {
-      // is the order of the N best (and their separation from the rest) proven by the approximate sums alone?
-      if (m <= 32) {
-        // the usual case: every warp ranks two survivors (a lane per opponent), then one warp checks the gaps and
-        // writes the list
-        rank_by_warps(list, list2, m);
         __syncthreads();
-        if (warp == 0) {
-          const bool sure = warp_check_write(list2, m, p.N, (u64)margin, true, o_idx, o_key);
-          if (lane == 0) {
-            if (sure) {
-              p.part_len[slot_out] = mo;
-              p.part_sft[slot_out] = sft;
-            } else {
-              s_flag = 1;
+      }
+      if (p.item_ok) {  // postprocessing/filters.py:58-101: filtered items are never recommended (4 items per word)
+        const unsigned* ok4 = reinterpret_cast<const unsigned*>(p.item_ok + r0);
+        for (int v = tid; v < nvec; v += nt) {
+          const unsigned okw = 4 * v < ns ? __ldg(ok4 + v) : 0x01010101u;
+          if (okw != 0x01010101u) {
+            uint4 x = acc4[v];
+            if (!(okw & 0xffu)) x.x = 0u;
+            if (!(okw & 0xff00u)) x.y = 0u;
+            if (!(okw & 0xff0000u)) x.z = 0u;
+            if (!(okw & 0xff000000u)) x.w = 0u;
+            acc4[v] = x;
+          }
+        }
+        __syncthreads();
+      }
+      PROF32_MARK(2);
+      // ---- survivor threshold.  Carried: with N entries in the list, an item can only reach the top N when its
+      //      upper end (a + d) * 2^s reaches the N-th entry's lower end L (the order of the list is proven, so the
+      //      lower ends decrease along it): a >= ceil(L / 2^s) - d.  With an approximate N-th entry a_N that is
+      //      a_N - 2d, the rule of a range's own bound.
+      unsigned thr_c = 1u;
+      if (r >= N) {
+        const u64 need = (a32_lo(list[N - 1], (u64)margin << sft) + ((1ull << sft) - 1)) >> sft;
+        thr_c = need > (u64)d + 1 ? (unsigned)min(need - (u64)d, 0xffffffffull) : 1u;
+      }
+      const bool carried = r >= N && !own;
+      unsigned thr = thr_c;
+      if (!carried) {
+        // own bound.  A dense pass costs a warp its full instruction stream whenever any of its lanes has work, so
+        // the per-range work is kept out of it: every thread takes the maximum of its own slots (no branches, no
+        // atomics), and the N-th largest of these per-thread maxima -- found with one histogram entry per thread,
+        // 32 bins per octave -- is a lower bound of the N-th largest sum (N distinct items reach it).  Everything
+        // within the margin below that bin survives.
+        unsigned mymax = 0u;
+        for (int v = tid; v < nvec; v += nt) {
+          const uint4 x = acc4[v];
+          mymax = max(mymax, max(max(x.x, x.y), max(x.z, x.w)));
+        }
+        // N-th largest of the 512 per-thread maxima, in two rounds of a 32-bin histogram (octave, then 32 bins
+        // inside the octave).  Every warp scans the 32 bins by itself (one bin per lane), so no warp waits for
+        // another one beyond the two barriers.
+        const int mybin = mymax ? a32_bin(mymax) : -1;  // (octave << 5) | bin inside the octave
+        if (mybin >= 0) atomicAdd(&hist[mybin >> 5], 1);
+        __syncthreads();
+        PROF32_MARK(12);
+        if (first) stage2(nxt);
+        int bstar = 0;
+        {
+          const int h1 = hist[lane];
+          int incl = h1;  // maxima in my octave and the higher ones
+#pragma unroll
+          for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_down_sync(0xffffffffu, incl, o);
+            if (lane + o < 32) incl += t;
+          }
+          const unsigned hit = __ballot_sync(0xffffffffu, incl >= N);  // lanes whose octave-and-above hold N maxima
+          if (hit) {
+            const int oct = 31 - __clz(hit);  // the highest such octave holds the N-th largest
+            const int above = __shfl_sync(0xffffffffu, incl - h1, oct);
+            if (mybin >= 0 && (mybin >> 5) == oct) atomicAdd(&hist[32 + (mybin & 31)], 1);
+            __syncthreads();
+            const int h2 = hist[32 + lane];
+            int incl2 = h2;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+              const int t = __shfl_down_sync(0xffffffffu, incl2, o);
+              if (lane + o < 32) incl2 += t;
+            }
+            const unsigned hit2 = __ballot_sync(0xffffffffu, above + incl2 >= N);
+            bstar = (oct << 5) | (hit2 ? 31 - __clz(hit2) : 0);
+          } else {
+            __syncthreads();  // fewer than N non-empty threads: everything survives (bstar = 0)
+          }
+        }
+        __syncthreads();  // every warp has read both histograms
+        if (mybin >= 0) {
+          hist[mybin >> 5] = 0;
+          hist[32 + (mybin & 31)] = 0;
+        }
+        const unsigned edge = a32_bin_floor(bstar);
+        thr = max(thr, edge > margin + 1u ? edge - margin : 1u);
+      } else if (first) {
+        stage2(nxt);
+      }
+      PROF32_MARK(13);
+      // copy the survivors behind the running list, clear the accumulators: one compare per vector, the rest only
+      // for the few that pass
+      const int room = p.cap - r;
+      for (int v = tid; v < nvec; v += nt) {
+        const uint4 x = acc4[v];
+        acc4[v] = make_uint4(0u, 0u, 0u, 0u);
+        if (max(max(x.x, x.y), max(x.z, x.w)) < thr) continue;
+        const unsigned xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          if (xs[q] >= thr) {
+            const int pos = atomicAdd(&sh->count, 1);
+            if (pos < room) {
+              Entry e;
+              e.key = ((u64)xs[q] + (u64)d) << sft;
+              e.idx = r0 + 4 * v + q;
+              e.aux = 1;
+              list[r + pos] = e;
             }
           }
-        }
-        __syncthreads();
-        need_exact = s_flag != 0;
-        if (!need_exact) {
-          PROF32_MARK(6);
-          continue;
-        }
-      } else {
-        surv = a32_sort(list, list2, m);
-        const int pairs = (m - 1) < p.N ? (m - 1) : p.N;
-        for (int kk = tid; kk < pairs; kk += nt)
-          if (surv[kk].key - surv[kk + 1].key <= (u64)margin) s_flag = 1;
-        __syncthreads();
-        need_exact = s_flag != 0;
-        if (!need_exact) {
-          for (int t = tid; t < p.N; t += nt) {
-            o_idx[t] = t < mo ? surv[t].idx : -1;
-            o_key[t] = t < mo ? surv[t].key : 0ull;
-          }
-          if (tid == 0) {
-            p.part_len[slot_out] = mo;
-            p.part_sft[slot_out] = sft;
-          }
-          __syncthreads();
-          PROF32_MARK(6);
-          continue;
-        }
       }
-    }
+      PROF32_MARK(14);
+      if (first) stage3(nxt);
+      first = false;
+      __syncthreads();
+      const int m = sh->count;
+      const int tot = r + m;
+      __syncthreads();  // every thread has read the count (thread 0 resets it at the next range)
+      PROF32_MARK(3);
 #ifdef RPK_PHASE_PROF
-    if (tid == 0) atomicAdd(p.prof + 9, 1ull);
+      if (tid == 0) {
+        atomicAdd(p.prof + 10, 1ull);
+        atomicAdd(p.prof + 11, (unsigned long long)(m > room ? 0 : m));
+        if (carried) atomicAdd(p.prof + 17, 1ull);
+      }
 #endif
-    // ---- sweep 2: exact scores of the survivors (slot -> survivor number + 1, key -> exact sum)
-    for (int t = tid; t < m; t += nt) {
-      acc[surv[t].idx - r0] = (unsigned)t + 1u;
-      surv[t].key = 0ull;
-    }
-    __syncthreads();
-    PROF32_MARK(4);
-    const bool limbs = d <= LIMB_CHUNK;  // two 32-bit adds (20-bit limbs) cannot overflow
-    if (m > 0) {
-      RowTab* rtw = rtab + cur;
-      for (int c0 = 0; c0 < d; c0 += A32_ROWS) {
-        const int n = min(A32_ROWS, d - c0);
-        if (d > A32_ROWS) {  // a single chunk is still staged from sweep 1
-          if (c0 > 0) __syncthreads();
-          for (int r = tid; r < n; r += nt) {
-            const int i = p.indices[xb + c0 + r];
-            const int4 b = __ldg(p.blk + (int64_t)i * p.P + pass);
-            rtw->seg[r] = make_int2(b.x, b.y);
-            rtw->item[r] = i;
-          }
-          __syncthreads();
+      if (m > room) {
+        if (carried) {  // the carried bound is too loose for this range: sweep it again and take its own bound
+#ifdef RPK_PHASE_PROF
+          if (tid == 0) atomicAdd(p.prof + 16, 1ull);
+#endif
+          own = true;
+          --pass;
+          continue;
         }
-        sweep_rows(p.ent, rt, n, idle, [&](u64 e) {
-          const unsigned j = ((unsigned)e & 0xffffffu) >> 2;
-          if (j < (unsigned)ns) {
-            const unsigned cn = acc[j];
-            if (cn) {
-              const u64 q = e >> 24;
-              if (limbs) {
-                unsigned* wd = reinterpret_cast<unsigned*>(&surv[cn - 1u].key);
-                atomicAdd(wd, (unsigned)q & LIMB_MASK);
-                atomicAdd(wd + 1, (unsigned)(q >> LIMB_BITS));
-              } else {
-                atomicAdd(&surv[cn - 1u].key, q);
+        // survivors do not fit: the exact kernel takes the whole user
+        if (tid == 0 && atomicExch(&p.ovf_flag[u], 1) == 0) p.ovf_tab[atomicAdd(p.ovf_count, 1)] = s_rec[cur];
+        break;
+      }
+      own = false;
+      // ---- sweep 2: exact scores of the entries of this range in s[0..tot) (slot -> place + 1, key -> exact sum);
+      //      the accumulators are all zero again afterwards
+      auto exact_pass = [&](Entry* s) {
+#ifdef RPK_PHASE_PROF
+        if (tid == 0) atomicAdd(p.prof + 9, 1ull);
+#endif
+        auto mine = [&](const Entry& e) { return e.aux && (unsigned)(e.idx - r0) < (unsigned)ns; };
+        for (int t = tid; t < tot; t += nt)
+          if (mine(s[t])) {
+            acc[s[t].idx - r0] = (unsigned)t + 1u;
+            s[t].key = 0ull;
+          }
+        __syncthreads();
+        PROF32_MARK(4);
+        const bool limbs = d <= LIMB_CHUNK;  // two 32-bit adds (20-bit limbs) cannot overflow
+        for (int c0 = 0; c0 < d; c0 += A32_ROWS) {
+          const int n = min(A32_ROWS, d - c0);
+          if (d > A32_ROWS) {  // a single chunk is still staged from sweep 1
+            if (c0 > 0) __syncthreads();
+            for (int rr = tid; rr < n; rr += nt) {
+              const int i = p.indices[xb + c0 + rr];
+              const int4 b = __ldg(p.blk + (int64_t)i * P + pass);
+              rt->seg[rr] = make_int2(b.x, b.y);
+              rt->item[rr] = i;
+            }
+            __syncthreads();
+          }
+          sweep_rows(p.ent, rt, n, idle, [&](u64 e) {
+            const unsigned j = ((unsigned)e & 0xffffffu) >> 2;
+            if (j < (unsigned)ns) {
+              const unsigned cn = acc[j];
+              if (cn) {
+                const u64 q = e >> 24;
+                if (limbs) {
+                  unsigned* wd = reinterpret_cast<unsigned*>(&s[cn - 1u].key);
+                  atomicAdd(wd, (unsigned)q & LIMB_MASK);
+                  atomicAdd(wd + 1, (unsigned)(q >> LIMB_BITS));
+                } else {
+                  atomicAdd(&s[cn - 1u].key, q);
+                }
               }
             }
+          });
+        }
+        __syncthreads();
+        PROF32_MARK(5);
+        for (int t = tid; t < tot; t += nt)
+          if (mine(s[t])) {
+            acc[s[t].idx - r0] = 0u;
+            if (limbs) {
+              const u64 kv = s[t].key;
+              s[t].key = ((kv >> 32) << LIMB_BITS) + (kv & 0xffffffffull);
+            }
+            s[t].aux = 0;
           }
-        });
+        __syncthreads();
+      };
+      // order the list; approximate keys that leave the order open take the exact pass (scores requested: all
+      // of them, before the first ordering)
+      Entry* s = list;
+      bool restart = false;
+      if (m > 0) {
+        bool due = uexact, done = false;
+        for (;;) {
+          if (due) {
+            exact_pass(s);
+            done = true;
+          }
+          s = a32_order(s, s == list ? list2 : list, tot);
+          if (uexact || !a32_unproven(s, tot, N, (u64)margin << sft)) break;
+          if (done) {  // an approximate key of an earlier range is too close to call
+            restart = true;
+            break;
+          }
+          due = true;
+        }
       }
+      if (restart) {  // the user again, exact throughout
+#ifdef RPK_PHASE_PROF
+        if (tid == 0) atomicAdd(p.prof + 15, 1ull);
+#endif
+        uexact = true;
+        staged = false;
+        r = 0;
+        pass = -1;
+        continue;
+      }
+      const int keep = tot < N ? tot : N;
+      if (pass + 1 == P) {  // the user's list is final
+        const double inv = p.scale->inv;
+        for (int t = tid; t < N; t += nt) {
+          p.out_idx[(int64_t)u * N + t] = t < keep ? s[t].idx : -1;
+          if (p.out_val) p.out_val[(int64_t)u * N + t] = t < keep ? (double)s[t].key * inv : 0.0;
+        }
+        if (tid == 0) p.out_len[u] = keep;
+      } else {
+        if (s != list)
+          for (int t = tid; t < keep; t += nt) list[t] = s[t];
+        if (pre) {
+          const int4 b = __ldg(p.blk + (int64_t)rt->item[tid] * P + pass + 1);
+          rt->seg[tid] = make_int2(b.x, b.y);
+        }
+      }
+      r = keep;
       __syncthreads();
+      PROF32_MARK(6);
     }
-    PROF32_MARK(5);
-    for (int t = tid; t < m; t += nt) {
-      acc[surv[t].idx - r0] = 0u;
-      if (limbs) {
-        const u64 kv = surv[t].key;
-        surv[t].key = ((kv >> 32) << LIMB_BITS) + (kv & 0xffffffffull);
-      }
-    }
+#ifdef RPK_PHASE_PROF
+    if (tid == 0) atomicAdd(p.prof + 8, 1ull);
+#endif
     __syncthreads();
-    if (m <= 32) {
-      Entry* other = surv == list ? list2 : list;
-      rank_by_warps(surv, other, m);
-      __syncthreads();
-      if (warp == 0) warp_check_write(other, m, p.N, 0ull, false, o_idx, o_key);
-    } else {
-      const Entry* fin = a32_sort(surv, surv == list ? list2 : list, m);
-      for (int t = tid; t < p.N; t += nt) {
-        o_idx[t] = t < mo ? fin[t].idx : -1;
-        o_key[t] = t < mo ? fin[t].key : 0ull;
-      }
-    }
-    if (tid == 0) {
-      p.part_len[slot_out] = mo;
-      p.part_sft[slot_out] = -1;
-    }
-    __syncthreads();
-    PROF32_MARK(6);
   }
 }
 
-// One warp per user: merge the P per-range lists (each best-first, exact keys) into the final top-N.
-// Users flagged in `alt_flag` take their lists from the second set (the two-limb kernel's, alt_P ranges).
-// only_a / only_b non-null: only users flagged in either are processed (second pass).
+// One warp per user: merge the P per-range lists of the two-limb kernel (each best-first, exact keys) into the final
+// top-N.  only non-null: only the users flagged there are processed (the ones the 32-bit kernel handed over).
 __global__ void k_predict_finalize(const int* __restrict__ part_idx, const u64* __restrict__ part_sq,
                                    const int* __restrict__ part_len, int64_t U, int P, int N, int* __restrict__ out_idx,
-                                   double* __restrict__ out_val, int* __restrict__ out_len,
-                                   const int* __restrict__ alt_flag, const int* __restrict__ alt_idx,
-                                   const u64* __restrict__ alt_sq, const int* __restrict__ alt_len, int alt_P,
-                                   const int* __restrict__ only_a, const int* __restrict__ only_b,
+                                   double* __restrict__ out_val, int* __restrict__ out_len, const int* __restrict__ only,
                                    const ModelScale* __restrict__ scale) {
   const int lane = threadIdx.x & 31;
   int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const double inv = scale->inv;
   for (int64_t u = warp; u < U; u += nwarps) {
-    if ((only_a || only_b) && !((only_a && only_a[u]) || (only_b && only_b[u]))) continue;
-    const bool alt = alt_flag && alt_flag[u];
-    const int Pu = alt ? alt_P : P;
-    const int PN = Pu * N;
-    const int* pi = (alt ? alt_idx : part_idx) + u * PN;
-    const u64* ps = (alt ? alt_sq : part_sq) + u * PN;
-    const int* pl = (alt ? alt_len : part_len) + u * Pu;
+    if (only && !only[u]) continue;
+    const int PN = P * N;
+    const int* pi = part_idx + u * PN;
+    const u64* ps = part_sq + u * PN;
+    const int* pl = part_len + u * P;
     int tot = 0;
-    for (int q = 0; q < Pu; ++q) tot += pl[q];
+    for (int q = 0; q < P; ++q) tot += pl[q];
     const int m = min(N, tot);
     for (int e = lane; e < PN; e += 32) {
       const int je = pi[e];
@@ -1642,90 +1673,6 @@ __global__ void k_predict_finalize(const int* __restrict__ part_idx, const u64* 
       out_idx[u * N + t] = -1;
       if (out_val) out_val[u * N + t] = 0.0;
     }
-    if (lane == 0) out_len[u] = m;
-  }
-}
-
-// Lists-only mode: the P per-range lists of a user carry exact sums (part_sft < 0) or approximate ones
-// (sums of (q >> s) | 1, part_sft = s).  Every key is an interval of the exact score:
-//   exact:        [E, E]
-//   approximate:  [(a - d) * 2^s, (a + d) * 2^s]        (|a - E / 2^s| <= d, d = history length)
-// One warp per user orders the (at most MERGE_MAX) entries by their upper ends and checks that down to the
-// (N+1)-th every entry's interval lies strictly above the next one's (equal exact scores: ascending index).  Then
-// the order is the exact order and the list is written; otherwise the user is queued for a second, exact pass.
-constexpr int MERGE_MAX = 256;
-constexpr int MERGE_WARPS = 4;
-__global__ void __launch_bounds__(32 * MERGE_WARPS) k_predict_merge(const int* __restrict__ part_idx, const u64* __restrict__ part_key,
-                                                                   const int* __restrict__ part_len, const int* __restrict__ part_sft,
-                                                                   const int64_t* __restrict__ indptr, int64_t U, int P, int N,
-                                                                   int* __restrict__ out_idx, int* __restrict__ out_len,
-                                                                   const int* __restrict__ ovf_flag, int* __restrict__ redo_flag,
-                                                                   int* __restrict__ redo_count, int4* __restrict__ redo_tab) {
-  // per warp: the user's entries as they come (a*) and in order (s*)
-  __shared__ u64 a_lo[MERGE_WARPS][MERGE_MAX], a_hi[MERGE_WARPS][MERGE_MAX];
-  __shared__ u64 s_lo[MERGE_WARPS][MERGE_MAX], s_hi[MERGE_WARPS][MERGE_MAX];
-  __shared__ int a_ix[MERGE_WARPS][MERGE_MAX], s_ix[MERGE_WARPS][MERGE_MAX];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  u64 *alo = a_lo[wib], *ahi = a_hi[wib], *lo = s_lo[wib], *hi = s_hi[wib];
-  int *aix = a_ix[wib], *ix = s_ix[wib];
-  int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  for (int64_t u = warp; u < U; u += nwarps) {
-    if (ovf_flag[u]) continue;  // the two-limb kernel produces this user's lists
-    const int64_t xb = indptr[u];
-    const u64 d = (u64)(indptr[u + 1] - xb);
-    // gather the valid entries of the P lists, densely: range q contributes its first part_len places
-    int tot = 0;
-    __syncwarp();
-    for (int q = 0; q < P; ++q) {
-      const int n = part_len[u * P + q];
-      const int sf = part_sft[u * P + q];
-      for (int t = lane; t < n; t += 32) {
-        const u64 k = part_key[(u * P + q) * N + t];
-        u64 l, h;
-        if (sf < 0) {
-          l = h = k;
-        } else {
-          l = (k > d ? k - d : 0ull) << sf;
-          h = (k + d) > (~0ull >> sf) ? ~0ull : (k + d) << sf;
-        }
-        alo[tot + t] = l;
-        ahi[tot + t] = h;
-        aix[tot + t] = part_idx[(u * P + q) * N + t];
-      }
-      tot += n;
-    }
-    __syncwarp();
-    // rank every entry against all of them: by upper end, then lower end, then index
-    for (int e = lane; e < tot; e += 32) {
-      const u64 l = alo[e], h = ahi[e];
-      const int je = aix[e];
-      int rank = 0;
-      for (int f = 0; f < tot; ++f) {
-        const u64 hf = ahi[f], lf = alo[f];
-        rank += (hf > h) || (hf == h && (lf > l || (lf == l && aix[f] < je)));
-      }
-      lo[rank] = l;
-      hi[rank] = h;
-      ix[rank] = je;
-    }
-    __syncwarp();
-    const int m = min(N, tot);
-    const int pairs = min(tot - 1, N);
-    bool bad = false;
-    for (int k = lane; k < pairs; k += 32) {
-      const bool exact_pair = lo[k] == hi[k] && lo[k + 1] == hi[k + 1];
-      const bool ok = lo[k] > hi[k + 1] || (exact_pair && (hi[k] > hi[k + 1] || ix[k] < ix[k + 1]));
-      bad |= !ok;
-    }
-    if (__any_sync(0xffffffffu, bad)) {
-      if (lane == 0) {
-        redo_flag[u] = 1;
-        redo_tab[atomicAdd(redo_count, 1)] = make_int4((int)u, (int)d, (int)(xb & 0xffffffffll), (int)(xb >> 32));
-      }
-      continue;
-    }
-    for (int t = lane; t < N; t += 32) out_idx[u * N + t] = t < m ? ix[t] : -1;
     if (lane == 0) out_len[u] = m;
   }
 }
@@ -1886,8 +1833,9 @@ static Pred32Geom predict32_geometry(rpk_ctx* c, int N) {
   g.ctas = two ? 2 : 1;
   g.P = two ? P2 : P1;
   int64_t R = two ? R2 : R1;
-  if ((c->flags & DBG_MULTI_PASS) && g.P < 2 && I >= 8) {
-    g.P = 2;
+  const int p_min = (c->flags & DBG_MANY_PASS) ? 4 : ((c->flags & DBG_MULTI_PASS) ? 2 : 1);
+  if (g.P < p_min && I >= 4 * p_min) {
+    g.P = p_min;
     R = ((I + g.P - 1) / g.P + 3) & ~(int64_t)3;
   }
   g.R = (int)R;
@@ -1908,7 +1856,7 @@ static PredWork prepare_work(rpk_ctx* c, int64_t U, const int64_t* indptr) {
   int* order = c->buf<int>("p_order", (size_t)U);
   int* bcnt = c->buf<int>("p_bcnt", 65 * 2 + 4);
   int* boff = bcnt + 65;
-  int* queue = boff + 65;  // [0] two-limb kernel, [1] 32-bit kernel, [2] its second (exact) pass
+  int* queue = boff + 65;  // [0] two-limb kernel, [1] 32-bit kernel
   RPK_CUDA(cudaMemsetAsync(bcnt, 0, sizeof(int) * (65 * 2 + 4), st));
   k_row_lengths<<<ceil_div(U, 256), 256, 0, st>>>(indptr, U, work);
   RPK_LAUNCH_CHECK(c);
@@ -2052,72 +2000,52 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
     if ((c->flags & DBG_WIDE_ACC) || !blocks_fit) {  // debug flag / giant models: every user through the two-limb kernel
       launch_predict(c, pp, g, U, indptr);
       k_predict_finalize<<<fgrid, 256, 0, st>>>(pp.part_idx, pp.part_sq, pp.part_len, U, g.P, N, o_idx.dev, o_val.dev,
-                                                o_len.dev, nullptr, nullptr, nullptr, nullptr, 0, nullptr, nullptr, scale);
+                                                o_len.dev, nullptr, scale);
       RPK_LAUNCH_CHECK(c);
     } else {
-      RPK_REQUIRE(U * (int64_t)g2.P < ((int64_t)1 << 31), "too many (user, item range) work items in one call; split the batch");
       ensure_blocks(c, g2.P, g2.R);
-      // lists only (no scores wanted): the approximate sums settle most lists, the rest are scored again exactly
-      const bool lists_only = o_val.dev == nullptr && (int64_t)g2.P * N <= MERGE_MAX && !(c->flags & DBG_EXACT_SCORES);
       Pred32Params qp;
       qp.indices = indices;
       qp.ent = c->get<u64>("m_ent4");
       qp.blk = c->get<int4>("m_blk");
-      qp.n_work = nullptr;
       qp.U = (int)U;
       qp.P = g2.P;
       qp.R = g2.R;
       qp.I = (int)c->m_I;
       qp.N = N;
       qp.mask = mask_history;
-      qp.exact = lists_only ? 0 : 1;
+      // lists only (no scores wanted): the approximate sums settle most lists, exact sums only where they do not
+      qp.exact = (o_val.dev != nullptr || (c->flags & DBG_EXACT_SCORES)) ? 1 : 0;
       qp.item_ok = item_filter_ptr(c);
       qp.cap = g2.cap;
-      qp.part_idx = c->buf<int>("p_part2_idx", (size_t)U * g2.P * N);
-      qp.part_key = c->buf<u64>("p_part2_sq", (size_t)U * g2.P * N);
-      qp.part_len = c->buf<int>("p_part2_len", (size_t)U * g2.P);
-      qp.part_sft = c->buf<int>("p_part2_sft", (size_t)U * g2.P);
-      // per-user flags: [0, U) handed to the two-limb kernel, [U] their count; [U+1, 2U+1) second exact pass, [2U+1] count
-      int* flags = c->buf<int>("p_ovf_flag", 2 * (size_t)U + 2);
+      qp.out_idx = o_idx.dev;
+      qp.out_val = o_val.dev;
+      qp.out_len = o_len.dev;
+      qp.scale = scale;
+      // per-user flags: [0, U) handed to the two-limb kernel, [U] their count
+      int* flags = c->buf<int>("p_ovf_flag", (size_t)U + 1);
       qp.ovf_flag = flags;
       qp.ovf_count = flags + U;
       qp.ovf_tab = c->buf<int4>("p_ovf_tab", (size_t)U);
-      int* redo_flag = flags + U + 1;
-      int* redo_count = flags + 2 * U + 1;
-      int4* redo_tab = c->buf<int4>("p_redo_tab", (size_t)U);
-      RPK_CUDA(cudaMemsetAsync(flags, 0, sizeof(int) * (2 * (size_t)U + 2), st));
+      RPK_CUDA(cudaMemsetAsync(flags, 0, sizeof(int) * ((size_t)U + 1), st));
       const PredWork w = prepare_work(c, U, indptr);
       qp.work_tab = w.tab;
       qp.queue = w.queue + 1;
       qp.prof = nullptr;
 #ifdef RPK_PHASE_PROF
-      qp.prof = c->buf<unsigned long long>("p_prof32", 16);
-      RPK_CUDA(cudaMemsetAsync(qp.prof, 0, 16 * sizeof(unsigned long long), st));  // 0-6 phases, 8-11 counters, 12-14 inside select
+      qp.prof = c->buf<unsigned long long>("p_prof32", 24);
+      RPK_CUDA(cudaMemsetAsync(qp.prof, 0, 24 * sizeof(unsigned long long), st));  // 0-6 phases, 8-11 and 15-17 counters, 12-14 inside select
 #endif
       RPK_CUDA(cudaFuncSetAttribute(k_predict_a32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g2.smem));
       int occ = 0;
       RPK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_predict_a32, g2.nt, g2.smem));
       RPK_REQUIRE(occ >= 1, "predict kernel does not fit on an SM");
-      const int grid = (int)std::min<int64_t>(U * g2.P, (int64_t)c->sm_count * occ);
+      const int grid = (int)std::min<int64_t>(U, (int64_t)c->sm_count * occ);
       c->mark("predict: layout + work table");
       c->ev_record(4);
       k_predict_a32<<<grid, g2.nt, g2.smem, st>>>(qp);
       RPK_LAUNCH_CHECK(c);
       c->mark("predict: scoring kernel");
-      if (lists_only) {
-        // order the per-range lists; users whose order the approximate sums cannot prove are scored again, exactly
-        const int mgrid = (int)std::min<int64_t>(ceil_div(U, MERGE_WARPS), (int64_t)c->sm_count * 16);
-        k_predict_merge<<<mgrid, 32 * MERGE_WARPS, 0, st>>>(qp.part_idx, qp.part_key, qp.part_len, qp.part_sft, indptr, U, g2.P, N,
-                                                           o_idx.dev, o_len.dev, qp.ovf_flag, redo_flag, redo_count, redo_tab);
-        RPK_LAUNCH_CHECK(c);
-        Pred32Params rp = qp;
-        rp.work_tab = redo_tab;
-        rp.n_work = redo_count;
-        rp.exact = 1;
-        rp.queue = w.queue + 2;
-        k_predict_a32<<<grid, g2.nt, g2.smem, st>>>(rp);
-        RPK_LAUNCH_CHECK(c);
-      }
       // users whose survivors overflowed the list: exact two-limb kernel (normally none; the kernel then exits)
       pp.work_tab = qp.ovf_tab;
       pp.n_work = qp.ovf_count;
@@ -2125,37 +2053,32 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
       launch_predict_kernel(c, pp, g, U);
       c->ev_record(5);
       c->ev_valid[2] = true;
-      c->mark("predict: merge + exact passes");
+      c->mark("predict: exact passes");
 #ifdef RPK_PHASE_PROF
       {
-        unsigned long long h[16];
-        int novf = 0, nredo = 0;
+        unsigned long long h[24];
+        int novf = 0;
         RPK_CUDA(cudaMemcpyAsync(h, qp.prof, sizeof(h), cudaMemcpyDeviceToHost, st));
         RPK_CUDA(cudaMemcpyAsync(&novf, qp.ovf_count, sizeof(int), cudaMemcpyDeviceToHost, st));
-        RPK_CUDA(cudaMemcpyAsync(&nredo, redo_count, sizeof(int), cudaMemcpyDeviceToHost, st));
         RPK_CUDA(cudaStreamSynchronize(st));
         static const char* nm[7] = {"fetch", "bound+sweep1", "mask", "select", "tag", "sweep2", "sort+out"};
         unsigned long long tot = 0;
-        h[3] += 0;
         for (int k = 0; k < 7; ++k) tot += h[k];
         tot += h[12] + h[13] + h[14];
-        fprintf(stderr, "[predict32 phases] grid=%d nt=%d P=%d R=%d smem=%zu occ=%d lists_only=%d items=%llu exact items=%llu survivors/item=%.1f overflow users=%d redo users=%d cycles/item=%.0f\n",
-                grid, g2.nt, g2.P, g2.R, g2.smem, occ, (int)lists_only, h[8], h[9], h[8] ? (double)h[11] / h[8] : 0.0, novf, nredo,
-                h[8] ? (double)tot / h[8] : 0.0);
+        const double us = h[8] ? (double)h[8] : 1.0;
+        fprintf(stderr, "[predict32 phases] grid=%d nt=%d P=%d R=%d smem=%zu occ=%d exact=%d users=%llu ranges=%llu carried ranges=%llu "
+                "carried retries=%llu exact range passes=%llu exact restarts=%llu survivors/user=%.1f overflow users=%d cycles/user=%.0f\n",
+                grid, g2.nt, g2.P, g2.R, g2.smem, occ, qp.exact, h[8], h[10], h[17], h[16], h[9], h[15], (double)h[11] / us, novf,
+                (double)tot / us);
         for (int k = 0; k < 7; ++k)
-          fprintf(stderr, "  %-12s %5.1f%%  %8.0f cycles/item\n", nm[k], 100.0 * h[k] / (tot ? tot : 1), h[8] ? (double)h[k] / h[8] : 0.0);
-        fprintf(stderr, "  select = thread maxima %.0f + boundary bin %.0f + copy/clear %.0f + staging of the next item %.0f cycles/item\n",
-                h[8] ? (double)h[12] / h[8] : 0.0, h[8] ? (double)h[13] / h[8] : 0.0, h[8] ? (double)h[14] / h[8] : 0.0,
-                h[8] ? (double)h[3] / h[8] : 0.0);
+          fprintf(stderr, "  %-12s %5.1f%%  %8.0f cycles/user\n", nm[k], 100.0 * h[k] / (tot ? tot : 1), (double)h[k] / us);
+        fprintf(stderr, "  select = thread maxima %.0f + boundary bin %.0f + copy/clear %.0f + staging of the next user %.0f cycles/user\n",
+                (double)h[12] / us, (double)h[13] / us, (double)h[14] / us, (double)h[3] / us);
       }
 #endif
-      if (lists_only) {
-        k_predict_finalize<<<fgrid, 256, 0, st>>>(qp.part_idx, qp.part_key, qp.part_len, U, g2.P, N, o_idx.dev, o_val.dev, o_len.dev,
-                                                  qp.ovf_flag, pp.part_idx, pp.part_sq, pp.part_len, g.P, qp.ovf_flag, redo_flag, scale);
-      } else {
-        k_predict_finalize<<<fgrid, 256, 0, st>>>(qp.part_idx, qp.part_key, qp.part_len, U, g2.P, N, o_idx.dev, o_val.dev, o_len.dev,
-                                                  qp.ovf_flag, pp.part_idx, pp.part_sq, pp.part_len, g.P, nullptr, nullptr, scale);
-      }
+      // the two-limb kernel's lists of the handed-over users
+      k_predict_finalize<<<fgrid, 256, 0, st>>>(pp.part_idx, pp.part_sq, pp.part_len, U, g.P, N, o_idx.dev, o_val.dev, o_len.dev,
+                                                qp.ovf_flag, scale);
       RPK_LAUNCH_CHECK(c);
     }
   }
