@@ -784,8 +784,16 @@ __global__ void __launch_bounds__(1024, 1) k_predict(PredParams p) {
               if (WIDE) {
                 atomicAdd(&acc64[j], q);
               } else {
-                const unsigned old = atomicAdd(&acc_lo[j], (unsigned)q & LIMB_MASK);
-                atomicAdd(&acc_hi[j], (unsigned)(q >> LIMB_BITS));
+                // a zero low limb would leave the slot looking untouched (a second first touch: the slot twice in
+                // the touched list), so it is added as 2^20 with one less in the high limb -- the same sum, and
+                // LIMB_CHUNK terms of at most 2^20 still fit the low limb
+                unsigned lo = (unsigned)q & LIMB_MASK, hi = (unsigned)(q >> LIMB_BITS);
+                if (lo == 0u) {
+                  lo = 1u << LIMB_BITS;
+                  --hi;
+                }
+                const unsigned old = atomicAdd(&acc_lo[j], lo);
+                atomicAdd(&acc_hi[j], hi);
                 first = old == 0u;
               }
             }
