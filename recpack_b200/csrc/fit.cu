@@ -25,6 +25,12 @@ __device__ unsigned long long g_sel_prof[16];
       sel_tprev = t_now;                                                          \
     }                                                                             \
   } while (0)
+// path counters of one fit call: the SelEvent branches taken by the row kernel's selections, then rows deferred to
+// k_fit_sort_rows and rows merged by k_fit_merge
+#define FIT_EV_DEFERRED 5
+#define FIT_EV_MERGED 6
+__device__ unsigned long long g_fit_ev[8];
+#define SEL_EVENT(src, ev) sel_event(src, ev)
 #endif
 #include "select.cuh"
 
@@ -666,6 +672,14 @@ struct RowCountSrc {
   __device__ __forceinline__ int cmp3(const Entry& a, const Entry& b) const { return sk.cmp3(a, b); }
 };
 
+#ifdef RPK_PHASE_PROF
+// only the selections of the row kernel (its counters are the source) are counted, not those of the merge and the sort
+template <class Src>
+__device__ __forceinline__ void sel_event(const Src&, int) {}
+template <bool PACK16>
+__device__ __forceinline__ void sel_event(const RowCountSrc<PACK16>&, int ev) { atomicAdd(&g_fit_ev[ev], 1ull); }
+#endif
+
 struct PairListSrc {  // (idx, cnt) pairs in global memory, idx < 0 = empty slot
   __device__ __forceinline__ bool has_queue() const { return false; }
   template <class F>
@@ -1131,6 +1145,9 @@ __global__ void __launch_bounds__(1024, 1) k_fit_rows(FitParams p) {
         s_cnt[t] = list[t].aux;
       }
       if (tid == 0) p.scr_len[orow] = m;
+#ifdef RPK_PHASE_PROF
+      if (tid == 0) atomicAdd(&g_fit_ev[FIT_EV_DEFERRED], 1ull);
+#endif
       __syncthreads();
       FIT_MARK(5);
       continue;
@@ -1174,6 +1191,9 @@ __global__ void __launch_bounds__(256) k_fit_merge(MergeParams p) {
       p.out_cnt[row * p.K + t] = t < m ? list[t].aux : 0;
     }
     if (tid == 0) p.out_len[row] = m;
+#ifdef RPK_PHASE_PROF
+    if (tid == 0) atomicAdd(&g_fit_ev[FIT_EV_MERGED], 1ull);
+#endif
     __syncthreads();
   }
 }
@@ -1509,12 +1529,7 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
     const int direct_cap = tiny ? K : std::min(cap, std::max(2 * K, 64));
     const size_t fixed = sel_smem_bytes(cap);
     RPK_REQUIRE((size_t)c->smem_max > fixed + 1024 + 4096, "K too large for shared memory");
-    const size_t avail = (size_t)c->smem_max - fixed - 2048;  // 2 KB slack for static shared memory
     const SimKey sk{n, rnf, pw, nmax, reinterpret_cast<const double*>(pwmin), nullptr, nullptr, mode};
-    // coded reciprocals (1 B per item in shared memory) when the catalogue leaves room for them
-    const bool use_code = mode == 0 && (size_t)I + 65536 < avail && U < ((int64_t)1 << 21);  // code 255 = 2.5M users
-    // (the kernel keeps R * P >= I code bytes: R is rounded up to a multiple of 8 per range)
-    const size_t code_bytes = use_code ? (((size_t)I + 8 * 64 + 15) & ~(size_t)15) : 0;
 
     c->mark("fit: CSC + order + heavy");
     c->span_begin(1);
@@ -1531,11 +1546,29 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
       RPK_CUDA(cudaEventCreateWithFlags(&c->side_ev[0], cudaEventDisableTiming));
       RPK_CUDA(cudaEventCreateWithFlags(&c->side_ev[1], cudaEventDisableTiming));
     }
+#ifdef RPK_PHASE_PROF
+    static const unsigned long long ev_zero[8] = {};
+    RPK_CUDA(cudaMemcpyToSymbolAsync(g_fit_ev, ev_zero, sizeof(ev_zero), 0, cudaMemcpyHostToDevice, st));
+    int geo_P = 0, geo_R = 0, geo_code = 0;
+    size_t geo_smem = 0, geo_static = 0;
+#endif
     RPK_CUDA(cudaEventRecord(c->side_ev[0], st));
     RPK_CUDA(cudaStreamWaitEvent(c->side, c->side_ev[0], 0));
     cudaStream_t main_st = st;
     for (int wide = 1; wide >= 0; --wide) {
       cudaStream_t st = wide ? c->side : main_st;  // shadows the outer stream inside this launch
+      auto kern = wide ? k_fit_rows<false> : k_fit_rows<true>;
+      // the kernel's static tables (popularity-code table, count floors, heavy columns) come out of the same
+      // per-block limit as the dynamic shared memory
+      cudaFuncAttributes fa;
+      RPK_CUDA(cudaFuncGetAttributes(&fa, kern));
+      const size_t static_smem = fa.sharedSizeBytes;
+      RPK_REQUIRE((size_t)c->smem_max > fixed + static_smem + 4096, "K too large for shared memory");
+      const size_t avail = (size_t)c->smem_max - fixed - static_smem;
+      // coded reciprocals (1 B per item in shared memory) when the catalogue leaves room for them
+      const bool use_code = mode == 0 && (size_t)I + 65536 < avail && U < ((int64_t)1 << 21);  // code 255 = 2.5M users
+      // (the kernel keeps R * P >= I code bytes: R is rounded up to a multiple of 8 per range)
+      const size_t code_bytes = use_code ? (((size_t)I + 8 * 64 + 15) & ~(size_t)15) : 0;
       // geometry: item-range passes so that the counters of one pass fit shared memory
       const int bytes_per_item = wide ? 4 : 2;
       int64_t Rmax = (int64_t)((avail - code_bytes) / bytes_per_item) & ~(int64_t)7;
@@ -1544,6 +1577,8 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
       if ((c->flags & DBG_MULTI_PASS) && P < 2 && I >= 16) P = 2;
       const int R = (int)(((I + P - 1) / P + 7) & ~(int64_t)7);
       const size_t smem = fixed + (size_t)R * bytes_per_item + code_bytes;
+      RPK_REQUIRE(smem + static_smem <= (size_t)c->smem_max,
+                  "fit geometry exceeds the shared memory of a block (dynamic + static)");
       const int nt = R >= 16384 ? 1024 : (R >= 4096 ? 512 : 256);
       const int64_t* usplit = nullptr;
       if (P > 1) {
@@ -1633,9 +1668,13 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
       if (!wide) {
         fp.prof = c->buf<unsigned long long>("fit_prof", 16);
         RPK_CUDA(cudaMemsetAsync(fp.prof, 0, 16 * sizeof(unsigned long long), st));
+        geo_P = P;
+        geo_R = R;
+        geo_code = use_code;
+        geo_smem = smem;
+        geo_static = static_smem;
       }
 #endif
-      auto kern = wide ? k_fit_rows<false> : k_fit_rows<true>;
       RPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       int occ = 0;
       RPK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, nt, smem));
@@ -1684,6 +1723,12 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
               h[8] ? (double)tot / h[8] : 0.0);
       for (int k = 0; k < 6; ++k)
         fprintf(stderr, "  %-18s %5.1f%%  %8.0f cycles/row\n", nm[k], 100.0 * h[k] / (tot ? tot : 1), h[8] ? (double)h[k] / h[8] : 0.0);
+      unsigned long long ev[8];
+      RPK_CUDA(cudaMemcpyFromSymbol(ev, g_fit_ev, sizeof(ev)));
+      fprintf(stderr, "[fit paths] guess_ok=%llu guess_rejected=%llu queue_overflow=%llu band=%llu index_radix=%llu deferred=%llu "
+              "merged=%llu P=%d R=%d code=%d smem=%zu static=%zu\n",
+              ev[SEL_EV_GUESS_OK], ev[SEL_EV_GUESS_REJECTED], ev[SEL_EV_QUEUE_OVERFLOW], ev[SEL_EV_BAND], ev[SEL_EV_INDEX_RADIX],
+              ev[FIT_EV_DEFERRED], ev[FIT_EV_MERGED], geo_P, geo_R, geo_code, geo_smem, geo_static);
     }
 #endif
     c->mark("fit: row kernels");

@@ -37,6 +37,11 @@ typedef unsigned long long u64;
 #define SEL_MARK(k) do {} while (0)
 #define SEL_MARK_BEGIN() do {} while (0)
 #endif
+// Path counters (RPK_PHASE_PROF builds of fit.cu define it): called by thread 0 when block_select_topk takes a branch.
+enum SelEvent { SEL_EV_GUESS_OK, SEL_EV_GUESS_REJECTED, SEL_EV_QUEUE_OVERFLOW, SEL_EV_BAND, SEL_EV_INDEX_RADIX, SEL_EV_COUNT };
+#ifndef SEL_EVENT
+#define SEL_EVENT(src, ev) do {} while (0)
+#endif
 
 struct __align__(16) Entry {
   u64 key;
@@ -315,7 +320,10 @@ __device__ int compact_above(Src& src, u64 thr, Entry* list, int cap, SelShared*
       return sh->count;
     }
     // the queue overflowed: nothing was taken yet, visit directly
-    if (threadIdx.x == 0) sh->count = 0;
+    if (threadIdx.x == 0) {
+      sh->count = 0;
+      SEL_EVENT(src, SEL_EV_QUEUE_OVERFLOW);
+    }
     __syncthreads();
   }
   src.for_each([&](int slot, u64 k) {
@@ -385,6 +393,7 @@ __device__ int block_select_topk(Src& src, int K, Entry* list, int cap, int dire
       if (tid == 0) sh->count2 = 0;
       const int got = compact_above(src, thr, list, cap, sh, edge, &sh->count2, hist, 1 << BITS);
       if (sh->count2 >= K && got <= cap) m = got;
+      if (tid == 0) SEL_EVENT(src, m >= 0 ? SEL_EV_GUESS_OK : SEL_EV_GUESS_REJECTED);
       __syncthreads();
       SEL_MARK(3);
     }
@@ -404,6 +413,7 @@ __device__ int block_select_topk(Src& src, int K, Entry* list, int cap, int dire
       }
       if (m > cap) {
         // ---- C: a band of (near-)equal keys is too large.  Pin tau = the K-th largest akey.
+        if (tid == 0) SEL_EVENT(src, SEL_EV_BAND);
         __syncthreads();
         refine_keys<BITS>(src, K, -1, lo, hi, g, n_in, hist, sh);
         const u64 tau = sh->lo;
@@ -504,6 +514,7 @@ __device__ int block_select_topk(Src& src, int K, Entry* list, int cap, int dire
           if (take_eq) break;  // the class fitted as a whole; the final sort trims it
           // ---- exact tie class larger than the list: take the (need - gt) smallest indices by a radix
           //      refinement on the index
+          if (tid == 0) SEL_EVENT(src, SEL_EV_INDEX_RADIX);
           const int need_idx = need - gt;
           u64 ilo = 0, ihi = (u64)SENTINEL_IDX;
           int ig = 0, iin = eq;
