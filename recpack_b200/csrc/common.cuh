@@ -43,7 +43,7 @@ enum {
   DBG_MULTI_PASS = 4,  // fit / predict: at least two item-range passes
   DBG_SPLIT_ROWS = 8,  // fit: cut the heaviest rows into pieces even when they are small
   DBG_EXACT_SCORES = 16,  // predict: exact sums for every list even when only the lists are asked for
-  DBG_MANY_PASS = 32,     // predict (top-N): at least four item ranges
+  DBG_MANY_PASS = 32,     // predict: at least four item ranges
 };
 
 }  // namespace rpk
@@ -157,7 +157,7 @@ struct rpk_ctx {
   int64_t filter_I = -1;  // item filter of the predict calls (buffer p_item_ok), -1 = none
   bool pack_flag_pending = false;  // a stream-ordered rpk_model_pack_rows_v left its validation flag unchecked
 
-  // ---- per-pass candidate counts of the last rpk_predict_csr_count
+  // ---- user count of the last rpk_predict_csr_count (rpk_predict_csr_fill must follow it on the same input)
   int64_t pc_U = 0;
 
   template <class T>

@@ -13,9 +13,9 @@
 // atomics land, so the top-N lists are deterministic.  Two kernels:
 //   k_predict_a32  top-N: 32-bit approximate sums with one native shared-memory atomic (ATOMS.ADD) per
 //                  entry pick the few items that can be in the top N, a second sweep adds their exact q;
-//   k_predict      full CSR output, and the exact path for users k_predict_a32 hands over: the sum is kept
-//                  in two 32-bit limbs (q & 0xFFFFF, q >> 20), 64-bit compare-and-swap accumulators when a
-//                  limb could overflow.
+//   k_predict      full CSR output, and the exact path for users k_predict_a32 hands over: one CTA per user runs
+//                  its item ranges in order, the sum is kept in two 32-bit limbs (q & 0xFFFFF, q >> 20), 64-bit
+//                  accumulators when a limb could overflow.
 #include <stdlib.h>
 
 #include <type_traits>
@@ -580,7 +580,8 @@ void run_model_load_csr(rpk_ctx* c, int64_t I, int64_t nnz, const int64_t* indpt
 // ------------------------------------------------------------------------------------------
 // Scoring kernel
 // ------------------------------------------------------------------------------------------
-// Candidate sources: the dense accumulator range, or the list of slots touched by this user.
+// Candidate source of the two-limb kernel: slots [0, ns) are the accumulators of the item range, slots
+// [ns, ns + nc) the user's running list carried from the earlier ranges (exact keys).
 struct ScoreSrc {
   __device__ __forceinline__ bool has_queue() const { return false; }
   template <class F>
@@ -588,13 +589,13 @@ struct ScoreSrc {
   const unsigned* lo;
   const unsigned* hi;
   const u64* wide;     // non-null: 64-bit accumulators
-  const int* touched;  // non-null: slot list (sparse mode)
-  int r0, ns;
+  const Entry* carry;  // the running list
+  int r0, ns, nc;
   u64 floor_;
   __device__ __forceinline__ u64 score_at(int j) const {
     return wide ? wide[j] : (((u64)hi[j] << LIMB_BITS) + (u64)lo[j]);
   }
-  __device__ __forceinline__ int nslots() const { return ns; }
+  __device__ __forceinline__ int nslots() const { return ns + nc; }
   __device__ __forceinline__ u64 margin() const { return 0ull; }
   __device__ __forceinline__ void set_floor(u64 thr) { floor_ = thr; }
   // Selection key: the score rounded toward zero to float, as a bit pattern.  The map is monotone
@@ -603,7 +604,7 @@ struct ScoreSrc {
   __device__ __forceinline__ static u64 key_of(u64 score) { return (u64)__float_as_uint(__ull2float_rz(score)); }
   __device__ __forceinline__ void stats(SelShared* sh) const {
     if (threadIdx.x == 0) {
-      sh->count = ns;  // upper bound of the candidate count (slots can be empty or masked)
+      sh->count = ns + nc;  // upper bound of the candidate count (slots can be empty or masked)
       sh->kmin = (u64)__float_as_uint(1.0f);
       sh->kmax = (u64)__float_as_uint(9007199254740992.0f);
     }
@@ -612,12 +613,15 @@ struct ScoreSrc {
   template <class F>
   __device__ __forceinline__ void visit(F f, int stride) const {
     for (int slot = threadIdx.x * stride; slot < ns; slot += blockDim.x * stride) {
-      const int j = touched ? touched[slot] : slot;
-      const u64 sc = score_at(j);
+      const u64 sc = score_at(slot);
       if (sc != 0) {
         const u64 k = key_of(sc);
         if (k >= floor_) f(slot, k);
       }
+    }
+    for (int t = threadIdx.x * stride; t < nc; t += blockDim.x * stride) {
+      const u64 k = key_of(carry[t].key);
+      if (k >= floor_) f(ns + t, k);
     }
   }
   template <class F>
@@ -625,9 +629,12 @@ struct ScoreSrc {
   template <class F>
   __device__ __forceinline__ void for_each_sampled(F f) const { visit(f, SEL_SAMPLE); }
   __device__ __forceinline__ void entry(int slot, Entry& e) const {
-    const int j = touched ? touched[slot] : slot;
-    e.key = score_at(j);
-    e.idx = r0 + j;
+    if (slot >= ns) {
+      e = carry[slot - ns];
+      return;
+    }
+    e.key = score_at(slot);
+    e.idx = r0 + slot;
     e.aux = 0;
   }
   __device__ __forceinline__ int cmp3(const Entry& a, const Entry& b) const {
@@ -648,18 +655,17 @@ struct PredParams {
   const int4* work_tab;  // {user, history length, row start lo, hi} in processing order
   const int* n_work;     // non-null: number of work_tab records (device side), replaces U
   int U, P, R, I, N, mask, mode, force_wide;
-  int cap, direct_cap, tcap;
+  int cap, direct_cap;
   int* queue;
-  int* part_idx;
-  u64* part_sq;
-  int* part_len;
-  int64_t* pass_cnt;
-  const int64_t* out_indptr;
+  int* out_idx;          // top-N: [U x N] lists, [U x N] scores or null, [U] lengths
+  double* out_val;
+  int* out_len;
+  int64_t* out_row_nnz;  // count: [U] non-empty scores of every user
+  const int64_t* out_indptr;  // fill: the CSR the count sized
   int* out_indices;
   double* out_values;
   const ModelScale* scale;   // scores are reported as sum * scale->inv
   const unsigned char* item_ok;  // non-null: item filter, 1 = may be recommended
-  unsigned long long* prof;  // RPK_PHASE_PROF builds: cycles of thread 0 per phase
 };
 
 #ifdef RPK_PHASE_PROF
@@ -675,10 +681,10 @@ struct PredParams {
 #define PROF_MARK(k) do {} while (0)
 #endif
 
-// Invariant: the accumulators of a CTA are all zero between work items.  A light user touches few of
-// the R slots of a range, so its slots are recorded on first touch (the low limb of a touched slot can
-// never be zero again: every q is odd) and only those are ranked and cleared; heavy users, and the
-// full-CSR modes, sweep the whole range instead.
+// One work item is a user: its P item ranges run one after the other on the same accumulators.  Invariant: the
+// accumulators of a CTA are all zero between ranges.  Top-N: the user's running list (at most N entries, exact
+// keys) is kept behind the accumulators and offered to the next range's selection as extra candidates, so that
+// the selection of the last range gives the user's final list.
 __global__ void __launch_bounds__(1024, 1) k_predict(PredParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
   Entry* list = reinterpret_cast<Entry*>(smem);
@@ -687,54 +693,43 @@ __global__ void __launch_bounds__(1024, 1) k_predict(PredParams p) {
   u64* acc64 = reinterpret_cast<u64*>(smem + sel_smem_bytes(p.cap));
   unsigned* acc_lo = reinterpret_cast<unsigned*>(acc64);
   unsigned* acc_hi = acc_lo + p.R;
-  int* touched = reinterpret_cast<int*>(acc64 + p.R);
+  Entry* carry = reinterpret_cast<Entry*>(acc64 + p.R);
   __shared__ int s_work;
-  __shared__ int s_next;      // work item fetched ahead (its user row is warmed in L2 on the way)
+  __shared__ int s_next;      // work item fetched ahead (its record is warmed in L2 on the way)
   __shared__ u64 s_bound;
   __shared__ int s_cnt;
-  __shared__ int s_ntouched;
 
   const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
-  const int total = (p.n_work ? *p.n_work : p.U) * p.P;
+  const int total = p.n_work ? *p.n_work : p.U;
   if (total == 0) return;
   for (int s = tid; s < p.R; s += nt) acc64[s] = 0ull;
   if (tid == 0) s_next = atomicAdd(p.queue, 1);
-#ifdef RPK_PHASE_PROF
-  long long t_prev = clock64();
-#endif
   for (;;) {
-    PROF_MARK(7);
     if (tid == 0) {
       s_work = s_next;
       const int nx = atomicAdd(p.queue, 1);
       s_next = nx;
-      if (nx < total) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.work_tab + nx / p.P) : "memory");
+      if (nx < total) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.work_tab + nx) : "memory");
       s_bound = 0;
       s_cnt = 0;
-      s_ntouched = 0;
     }
     __syncthreads();
     const int w = s_work;
     __syncthreads();
     if (w >= total) break;
-    const int4 rec = p.work_tab[w / p.P];
+    const int4 rec = p.work_tab[w];
     const int u = rec.x;
-    const int pass = w % p.P;
-    const int r0 = pass * p.R;
-    const int ns = min(p.R, p.I - r0);
     const int64_t xb = ((int64_t)(unsigned)rec.z) | ((int64_t)rec.w << 32);
     const int d = rec.y;
-    const int64_t slot_out = (int64_t)u * p.P + pass;
-    PROF_MARK(0);
     if (d == 0) {  // user without history: empty prediction row (algorithms/base.py:123-127)
       if (p.mode == PRED_TOPN) {
         for (int t = tid; t < p.N; t += nt) {
-          p.part_idx[slot_out * p.N + t] = -1;
-          p.part_sq[slot_out * p.N + t] = 0;
+          p.out_idx[(int64_t)u * p.N + t] = -1;
+          if (p.out_val) p.out_val[(int64_t)u * p.N + t] = 0.0;
         }
-        if (tid == 0) p.part_len[slot_out] = 0;
+        if (tid == 0) p.out_len[u] = 0;
       } else if (p.mode == PRED_COUNT) {
-        if (tid == 0) p.pass_cnt[slot_out] = 0;
+        if (tid == 0) p.out_row_nnz[u] = 0;
       }
       continue;
     }
@@ -749,204 +744,163 @@ __global__ void __launch_bounds__(1024, 1) k_predict(PredParams p) {
       __syncthreads();
       wide = s_bound >= (((u64)1) << 32);
     }
-    PROF_MARK(1);
-    // sparse mode: track first touches (needs the limb accumulators and a single chunk)
-    const bool track = !wide && d <= LIMB_CHUNK && p.mode == PRED_TOPN && p.tcap > 0;
-    // ---- accumulate: history rows are dealt to the warps in chunks (<= 32 rows, one per lane, so that the
-    //      segment bounds are fetched in parallel); rows are added in groups of LIMB_CHUNK so that the low
-    //      limb (20 bits per term) cannot overflow 32 bits between normalisations
-    // the loop is instantiated for the three accumulator modes so that the hot path carries no mode tests
-    auto accumulate = [&](auto wide_c, auto track_c) {
-      constexpr bool WIDE = decltype(wide_c)::value;
-      constexpr bool TRACK = decltype(track_c)::value;
-      for (int c0 = 0; c0 < d; c0 += LIMB_CHUNK) {
-        const int c1 = min(d, c0 + LIMB_CHUNK);
-        int chunk = (c1 - c0 + nwarps - 1) / nwarps;
-        chunk = chunk < 1 ? 1 : (chunk > 32 ? 32 : chunk);
-        for (int base = c0 + warp * chunk; base < c1; base += nwarps * chunk) {
-          const int nvalid = min(chunk, c1 - base);
-          int64_t beg = 0;
-          int len = 0;
-          if (lane < nvalid) {
-            const int i = p.indices[xb + base + lane];
-            const int* sg = p.m_seg + (int64_t)i * (p.P + 1) + pass;
-            const int s0 = sg[0];
-            beg = p.m_ptr[i] + s0;
-            len = sg[1] - s0;
+    int nc = 0;       // top-N: entries of the running list
+    int running = 0;  // fill: entries written for this user so far
+    for (int pass = 0; pass < p.P; ++pass) {
+      const int r0 = pass * p.R;
+      const int ns = min(p.R, p.I - r0);
+      // ---- accumulate: history rows are dealt to the warps in chunks (<= 32 rows, one per lane, so that the
+      //      segment bounds are fetched in parallel); rows are added in groups of LIMB_CHUNK so that the low
+      //      limb (20 bits per term) cannot overflow 32 bits between normalisations
+      // the loop is instantiated for both accumulator modes so that the hot path carries no mode tests
+      auto accumulate = [&](auto wide_c) {
+        constexpr bool WIDE = decltype(wide_c)::value;
+        for (int c0 = 0; c0 < d; c0 += LIMB_CHUNK) {
+          const int c1 = min(d, c0 + LIMB_CHUNK);
+          int chunk = (c1 - c0 + nwarps - 1) / nwarps;
+          chunk = chunk < 1 ? 1 : (chunk > 32 ? 32 : chunk);
+          for (int base = c0 + warp * chunk; base < c1; base += nwarps * chunk) {
+            const int nvalid = min(chunk, c1 - base);
+            int64_t beg = 0;
+            int len = 0;
+            if (lane < nvalid) {
+              const int i = p.indices[xb + base + lane];
+              const int* sg = p.m_seg + (int64_t)i * (p.P + 1) + pass;
+              const int s0 = sg[0];
+              beg = p.m_ptr[i] + s0;
+              len = sg[1] - s0;
+            }
+            auto add_entry = [&](u64 ent) {
+              if (ent != 0ull) {
+                const int j = (int)(ent >> 40) - r0;
+                const u64 q = ent & Q_MASK40;
+                if (WIDE) {
+                  atomicAdd(&acc64[j], q);
+                } else {
+                  atomicAdd(&acc_lo[j], (unsigned)q & LIMB_MASK);
+                  atomicAdd(&acc_hi[j], (unsigned)(q >> LIMB_BITS));
+                }
+              }
+            };
+            // rows are taken four at a time: the first 96 entries of each (a row segment rarely has more) are
+            // loaded up front -- 12 independent loads in flight per lane -- and only then added
+            for (int l0 = 0; l0 < nvalid; l0 += 4) {
+              u64 ent[4][3];
+              int64_t bq[4];
+              int nq[4];
+#pragma unroll
+              for (int q = 0; q < 4; ++q) {
+                const int l = l0 + q;  // lanes >= nvalid hold len = 0
+                bq[q] = __shfl_sync(0xffffffffu, beg, l & 31);
+                nq[q] = l < nvalid ? __shfl_sync(0xffffffffu, len, l & 31) : 0;
+#pragma unroll
+                for (int it = 0; it < 3; ++it) {
+                  const int e = it * 32 + lane;
+                  ent[q][it] = e < nq[q] ? p.m_ent[bq[q] + e] : 0ull;
+                }
+              }
+#pragma unroll
+              for (int q = 0; q < 4; ++q) {
+#pragma unroll
+                for (int it = 0; it < 3; ++it)
+                  if (it * 32 < nq[q]) add_entry(ent[q][it]);
+                for (int e0 = 96; e0 < nq[q]; e0 += 32) {
+                  const int e = e0 + lane;
+                  add_entry(e < nq[q] ? p.m_ent[bq[q] + e] : 0ull);
+                }
+              }
+            }
           }
-          // add one entry to the accumulators; in sparse mode record the slot on its first touch
-          auto add_entry = [&](u64 ent) {
-            bool first = false;
-            int j = 0;
-            if (ent != 0ull) {
-              j = (int)(ent >> 40) - r0;
-              const u64 q = ent & Q_MASK40;
-              if (WIDE) {
-                atomicAdd(&acc64[j], q);
-              } else {
-                // a zero low limb would leave the slot looking untouched (a second first touch: the slot twice in
-                // the touched list), so it is added as 2^20 with one less in the high limb -- the same sum, and
-                // LIMB_CHUNK terms of at most 2^20 still fit the low limb
-                unsigned lo = (unsigned)q & LIMB_MASK, hi = (unsigned)(q >> LIMB_BITS);
-                if (lo == 0u) {
-                  lo = 1u << LIMB_BITS;
-                  --hi;
-                }
-                const unsigned old = atomicAdd(&acc_lo[j], lo);
-                atomicAdd(&acc_hi[j], hi);
-                first = old == 0u;
-              }
+          __syncthreads();
+          if (!WIDE && c1 < d) {  // carry the low limb into the high limb before the next chunk
+            for (int s = tid; s < ns; s += nt) {
+              unsigned l = acc_lo[s];
+              acc_hi[s] += l >> LIMB_BITS;
+              acc_lo[s] = l & LIMB_MASK;
             }
-            if (TRACK) {
-              const unsigned m = __ballot_sync(0xffffffffu, first);
-              if (m) {
-                const int leader = __ffs(m) - 1;
-                int pos = 0;
-                if (lane == leader) pos = atomicAdd(&s_ntouched, __popc(m));
-                pos = __shfl_sync(0xffffffffu, pos, leader);
-                if (first) {
-                  const int my = pos + __popc(m & ((1u << lane) - 1u));
-                  if (my < p.tcap) touched[my] = j;
-                }
-              }
-            }
-          };
-          // rows are taken four at a time: the first 96 entries of each (a row segment rarely has more) are
-          // loaded up front -- 12 independent loads in flight per lane -- and only then added
-          for (int l0 = 0; l0 < nvalid; l0 += 4) {
-            u64 ent[4][3];
-            int64_t bq[4];
-            int nq[4];
-  #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const int l = l0 + q;  // lanes >= nvalid hold len = 0
-              bq[q] = __shfl_sync(0xffffffffu, beg, l & 31);
-              nq[q] = l < nvalid ? __shfl_sync(0xffffffffu, len, l & 31) : 0;
-  #pragma unroll
-              for (int it = 0; it < 3; ++it) {
-                const int e = it * 32 + lane;
-                ent[q][it] = e < nq[q] ? p.m_ent[bq[q] + e] : 0ull;
-              }
-            }
-  #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-  #pragma unroll
-              for (int it = 0; it < 3; ++it)
-                if (it * 32 < nq[q]) add_entry(ent[q][it]);
-              for (int e0 = 96; e0 < nq[q]; e0 += 32) {
-                const int e = e0 + lane;
-                add_entry(e < nq[q] ? p.m_ent[bq[q] + e] : 0ull);
-              }
+            __syncthreads();
+          }
+        }
+      };
+      if (wide) accumulate(std::true_type{});
+      else accumulate(std::false_type{});
+      if (p.mask) {  // pipelines/pipeline.py:174-175 -- before the truncation to N
+        for (int r = tid; r < d; r += nt) {
+          const int j = p.indices[xb + r] - r0;
+          if (j >= 0 && j < ns) {
+            if (wide) acc64[j] = 0ull;
+            else {
+              acc_lo[j] = 0u;
+              acc_hi[j] = 0u;
             }
           }
         }
         __syncthreads();
-        if (!WIDE && c1 < d) {  // carry the low limb into the high limb before the next chunk
-          for (int s = tid; s < ns; s += nt) {
-            unsigned l = acc_lo[s];
-            acc_hi[s] += l >> LIMB_BITS;
-            acc_lo[s] = l & LIMB_MASK;
+      }
+      if (p.item_ok) {  // postprocessing/filters.py:58-101: filtered items are never recommended
+        for (int s = tid; s < ns; s += nt)
+          if (!p.item_ok[r0 + s]) {
+            if (wide) acc64[s] = 0ull;
+            else {
+              acc_lo[s] = 0u;
+              acc_hi[s] = 0u;
+            }
           }
+        __syncthreads();
+      }
+      ScoreSrc src{acc_lo, acc_hi, wide ? acc64 : nullptr, carry, r0, ns, nc, 0ull};
+      if (p.mode == PRED_TOPN) {
+        // top N of this range and the earlier ones: the carried keys are exact sums and key_of is monotone, so
+        // margin() = 0 holds for them too, and ties still go to the lower index
+        const int m = block_select_topk(src, p.N, list, p.cap, p.direct_cap, hist, sh);
+        if (pass + 1 == p.P) {
+          const double inv_scale = p.scale->inv;
+          for (int t = tid; t < p.N; t += nt) {
+            p.out_idx[(int64_t)u * p.N + t] = t < m ? list[t].idx : -1;
+            if (p.out_val) p.out_val[(int64_t)u * p.N + t] = t < m ? (double)list[t].key * inv_scale : 0.0;
+          }
+          if (tid == 0) p.out_len[u] = m;
+        } else {
+          for (int t = tid; t < m; t += nt) carry[t] = list[t];
+          nc = m;
+        }
+      } else if (p.mode == PRED_COUNT) {
+        int cnt = 0;
+        for (int s = tid; s < ns; s += nt) cnt += src.score_at(s) != 0;
+        cnt = __reduce_add_sync(0xffffffffu, cnt);
+        if (lane == 0 && cnt) atomicAdd(&s_cnt, cnt);
+      } else {
+        const int64_t out = p.out_indptr[u];
+        const double inv_scale = p.scale->inv;
+        for (int base = 0; base < ns; base += nt) {
+          const int s = base + tid;
+          const u64 sc = s < ns ? src.score_at(s) : 0ull;
+          const unsigned bal = __ballot_sync(0xffffffffu, sc != 0);
+          if (lane == 0) sh->warp_tot[warp] = __popc(bal);
+          __syncthreads();
+          int off = 0, tot = 0;
+          for (int q = 0; q < nwarps; ++q) {
+            int v = sh->warp_tot[q];
+            if (q < warp) off += v;
+            tot += v;
+          }
+          if (sc != 0) {
+            const int pos = running + off + __popc(bal & ((1u << lane) - 1u));
+            p.out_indices[out + pos] = r0 + s;
+            p.out_values[out + pos] = (double)sc * inv_scale;
+          }
+          running += tot;
           __syncthreads();
         }
       }
-    };
-    if (wide) accumulate(std::true_type{}, std::false_type{});
-    else if (track) accumulate(std::false_type{}, std::true_type{});
-    else accumulate(std::false_type{}, std::false_type{});
-    const int n_touched = s_ntouched;
-    const bool sparse = track && n_touched <= p.tcap;
-    PROF_MARK(2);
-#ifdef RPK_PHASE_PROF
-    if (tid == 0) {
-      atomicAdd(p.prof + 8, 1ull);
-      atomicAdd(p.prof + 9, (unsigned long long)sparse);
-      atomicAdd(p.prof + 10, (unsigned long long)n_touched);
-    }
-#endif
-    if (p.mask) {  // pipelines/pipeline.py:174-175 -- before the truncation to N
-      for (int r = tid; r < d; r += nt) {
-        const int j = p.indices[xb + r] - r0;
-        if (j >= 0 && j < ns) {
-          if (wide) acc64[j] = 0ull;
-          else {
-            acc_lo[j] = 0u;
-            acc_hi[j] = 0u;
-          }
-        }
-      }
       __syncthreads();
-    }
-    if (p.item_ok) {  // postprocessing/filters.py:58-101: filtered items are never recommended
-      for (int s = tid; s < ns; s += nt)
-        if (!p.item_ok[r0 + s]) {
-          if (wide) acc64[s] = 0ull;
-          else {
-            acc_lo[s] = 0u;
-            acc_hi[s] = 0u;
-          }
-        }
-      __syncthreads();
-    }
-    ScoreSrc src{acc_lo, acc_hi, wide ? acc64 : nullptr, sparse ? touched : nullptr, r0, sparse ? n_touched : ns, 0ull};
-    PROF_MARK(3);
-    if (p.mode == PRED_TOPN) {
-      const int m = block_select_topk(src, p.N, list, p.cap, p.direct_cap, hist, sh);
-      PROF_MARK(4);
-      for (int t = tid; t < p.N; t += nt) {
-        p.part_idx[slot_out * p.N + t] = t < m ? list[t].idx : -1;
-        p.part_sq[slot_out * p.N + t] = t < m ? list[t].key : 0ull;
-      }
-      if (tid == 0) p.part_len[slot_out] = m;
-    } else if (p.mode == PRED_COUNT) {
-      int cnt = 0;
-      for (int s = tid; s < ns; s += nt) cnt += src.score_at(s) != 0;
-      cnt = __reduce_add_sync(0xffffffffu, cnt);
-      if (lane == 0 && cnt) atomicAdd(&s_cnt, cnt);
-      __syncthreads();
-      if (tid == 0) p.pass_cnt[slot_out] = s_cnt;
-    } else {
-      int64_t out = p.out_indptr[u];
-      const double inv_scale = p.scale->inv;
-      for (int q = 0; q < pass; ++q) out += p.pass_cnt[(int64_t)u * p.P + q];
-      int running = 0;
-      for (int base = 0; base < ns; base += nt) {
-        const int s = base + tid;
-        const u64 sc = s < ns ? src.score_at(s) : 0ull;
-        const unsigned bal = __ballot_sync(0xffffffffu, sc != 0);
-        if (lane == 0) sh->warp_tot[warp] = __popc(bal);
-        __syncthreads();
-        int off = 0, tot = 0;
-        for (int q = 0; q < nwarps; ++q) {
-          int v = sh->warp_tot[q];
-          if (q < warp) off += v;
-          tot += v;
-        }
-        if (sc != 0) {
-          const int pos = running + off + __popc(bal & ((1u << lane) - 1u));
-          p.out_indices[out + pos] = r0 + s;
-          p.out_values[out + pos] = (double)sc * inv_scale;
-        }
-        running += tot;
-        __syncthreads();
-      }
-    }
-    __syncthreads();
-    PROF_MARK(5);
-    // ---- restore the all-zero invariant
-    if (sparse) {
-      for (int t = tid; t < n_touched; t += nt) {
-        const int j = touched[t];
-        acc_lo[j] = 0u;
-        acc_hi[j] = 0u;
-      }
-    } else {
+      // ---- restore the all-zero invariant
       for (int s = tid; s < ns; s += nt) acc64[s] = 0ull;
       if (ns < p.R)
         for (int s = tid; s < ns; s += nt) acc_hi[s] = 0u;
+      __syncthreads();
     }
-    __syncthreads();
-    PROF_MARK(6);
+    if (p.mode == PRED_COUNT && tid == 0) p.out_row_nnz[u] = s_cnt;
   }
 }
 
@@ -996,8 +950,7 @@ struct Pred32Params {
   int* out_len;          // [U]
   const ModelScale* scale;
   const unsigned char* item_ok;  // non-null: item filter (1 = may be recommended), padded to a multiple of 4 items
-  int* ovf_flag;         // per user: 1 = handed to the two-limb kernel
-  int* ovf_count;        // number of such users
+  int* ovf_count;        // number of users handed to the two-limb kernel
   int4* ovf_tab;         // their work records
   unsigned long long* prof;
 };
@@ -1524,7 +1477,7 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
           continue;
         }
         // survivors do not fit: the exact kernel takes the whole user
-        if (tid == 0 && atomicExch(&p.ovf_flag[u], 1) == 0) p.ovf_tab[atomicAdd(p.ovf_count, 1)] = s_rec[cur];
+        if (tid == 0) p.ovf_tab[atomicAdd(p.ovf_count, 1)] = s_rec[cur];
         break;
       }
       own = false;
@@ -1642,49 +1595,6 @@ __global__ void __launch_bounds__(A32_NT, 2) k_predict_a32(Pred32Params p) {
   }
 }
 
-// One warp per user: merge the P per-range lists of the two-limb kernel (each best-first, exact keys) into the final
-// top-N.  only non-null: only the users flagged there are processed (the ones the 32-bit kernel handed over).
-__global__ void k_predict_finalize(const int* __restrict__ part_idx, const u64* __restrict__ part_sq,
-                                   const int* __restrict__ part_len, int64_t U, int P, int N, int* __restrict__ out_idx,
-                                   double* __restrict__ out_val, int* __restrict__ out_len, const int* __restrict__ only,
-                                   const ModelScale* __restrict__ scale) {
-  const int lane = threadIdx.x & 31;
-  int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  const double inv = scale->inv;
-  for (int64_t u = warp; u < U; u += nwarps) {
-    if (only && !only[u]) continue;
-    const int PN = P * N;
-    const int* pi = part_idx + u * PN;
-    const u64* ps = part_sq + u * PN;
-    const int* pl = part_len + u * P;
-    int tot = 0;
-    for (int q = 0; q < P; ++q) tot += pl[q];
-    const int m = min(N, tot);
-    for (int e = lane; e < PN; e += 32) {
-      const int je = pi[e];
-      if (je < 0) continue;
-      const u64 se = ps[e];
-      int rank = 0;
-      for (int f = 0; f < PN; ++f) {
-        const int jf = pi[f];
-        if (jf < 0) continue;
-        const u64 sf = ps[f];
-        rank += (sf > se) || (sf == se && jf < je);
-      }
-      if (rank < N) {
-        out_idx[u * N + rank] = je;
-        if (out_val) out_val[u * N + rank] = (double)se * inv;
-      }
-    }
-    for (int t = m + lane; t < N; t += 32) {
-      out_idx[u * N + t] = -1;
-      if (out_val) out_val[u * N + t] = 0.0;
-    }
-    if (lane == 0) out_len[u] = m;
-  }
-}
-
 // Work table in processing order: one 16-byte record per user {user, history length, row start}, so that a
 // CTA needs a single load (prefetched one item ahead) to start on a user.
 __global__ void k_build_work_tab(const int* __restrict__ order, const int64_t* __restrict__ indptr, int64_t U,
@@ -1702,15 +1612,6 @@ __global__ void k_row_lengths(const int64_t* __restrict__ indptr, int64_t U, u64
   if (u < U) work[u] = (u64)(indptr[u + 1] - indptr[u]);
 }
 
-__global__ void k_sum_passes(const int64_t* __restrict__ pass_cnt, int64_t U, int P, int64_t* __restrict__ row_nnz) {
-  int64_t u = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (u < U) {
-    int64_t s = 0;
-    for (int q = 0; q < P; ++q) s += pass_cnt[u * P + q];
-    row_nnz[u] = s;
-  }
-}
-
 // ------------------------------------------------------------------------------------------
 // Host driver
 // ------------------------------------------------------------------------------------------
@@ -1721,7 +1622,7 @@ static int next_pow2(int v) {
 }
 
 struct PredGeom {
-  int cap, direct_cap, P, R, nt, tcap;
+  int cap, direct_cap, P, R, nt;
   size_t fixed, smem;
 };
 
@@ -1730,33 +1631,28 @@ static PredGeom predict_geometry(rpk_ctx* c, int N) {
   const bool tiny = c->flags & DBG_TINY_LIST;
   g.cap = std::max(tiny ? 64 : 256, next_pow2(2 * std::max(N, 1)));
   g.direct_cap = tiny ? std::max(N, 1) : std::min(g.cap, std::max(64, 2 * N));
-  g.fixed = sel_smem_bytes(g.cap);
+  // the user's running list (top-N), carried from range to range behind the accumulators
+  g.fixed = sel_smem_bytes(g.cap) + (size_t)N * sizeof(Entry);
   RPK_REQUIRE((size_t)c->smem_max > g.fixed + 1024 + 8192, "N too large for shared memory");
   const size_t avail = (size_t)c->smem_max - g.fixed - 1024;
   const int64_t I = c->m_I;
-  // 8 B of accumulator per item of a range + a list of touched slots (4 B each, up to 8192 of them)
+  // 8 B of accumulator per item of a range
   int P = 1;
-  int64_t R = 0, T = 0;
+  int64_t R = 0;
   for (;; ++P) {
     R = ((I + P - 1) / P + 3) & ~(int64_t)3;
     if (R < 4) R = 4;
-    T = std::min<int64_t>(R, tiny ? 48 : 8192);
-    if ((size_t)(R * 8 + T * 4) <= avail) break;
+    if ((size_t)R * 8 <= avail) break;
   }
-  if ((c->flags & DBG_MULTI_PASS) && P < 2 && I >= 8) {
-    P = 2;
+  const int p_min = (c->flags & DBG_MANY_PASS) ? 4 : ((c->flags & DBG_MULTI_PASS) ? 2 : 1);
+  if (P < p_min && I >= 4 * p_min) {
+    P = p_min;
     R = ((I + P - 1) / P + 3) & ~(int64_t)3;
-    T = std::min<int64_t>(R, tiny ? 48 : 8192);
   }
   g.P = P;
   g.R = (int)R;
-  g.tcap = (int)T;
-  g.smem = g.fixed + (size_t)R * sizeof(u64) + (size_t)T * sizeof(int);
+  g.smem = g.fixed + (size_t)R * sizeof(u64);
   g.nt = g.R >= 8192 ? 1024 : (g.R >= 2048 ? 512 : 256);
-  if (const char* e = getenv("RPK_PRED_NT")) {  // tuning hook
-    int v = atoi(e);
-    if (v >= 64 && v <= 1024 && v % 32 == 0) g.nt = v;
-  }
   return g;
 }
 
@@ -1886,13 +1782,7 @@ static void launch_predict_kernel(rpk_ctx* c, PredParams& pp, const PredGeom& g,
   int occ = 0;
   RPK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_predict, g.nt, g.smem));
   RPK_REQUIRE(occ >= 1, "predict kernel does not fit on an SM");
-  const int64_t total = U * g.P;
-  const int grid = (int)std::min<int64_t>(total, (int64_t)c->sm_count * occ);
-  pp.prof = nullptr;
-#ifdef RPK_PHASE_PROF
-  pp.prof = c->buf<unsigned long long>("p_prof", 16);
-  RPK_CUDA(cudaMemsetAsync(pp.prof, 0, 16 * sizeof(unsigned long long), c->stream));
-#endif
+  const int grid = (int)std::min<int64_t>(U, (int64_t)c->sm_count * occ);
   k_predict<<<grid, g.nt, g.smem, c->stream>>>(pp);
   RPK_LAUNCH_CHECK(c);
 }
@@ -1929,11 +1819,10 @@ static void fill_common(rpk_ctx* c, PredParams& pp, const PredGeom& g, int64_t U
   pp.force_wide = (c->flags & DBG_WIDE_ACC) ? 1 : 0;
   pp.cap = g.cap;
   pp.direct_cap = g.direct_cap;
-  pp.tcap = g.tcap;
-  pp.part_idx = nullptr;
-  pp.part_sq = nullptr;
-  pp.part_len = nullptr;
-  pp.pass_cnt = nullptr;
+  pp.out_idx = nullptr;
+  pp.out_val = nullptr;
+  pp.out_len = nullptr;
+  pp.out_row_nnz = nullptr;
   pp.out_indptr = nullptr;
   pp.out_indices = nullptr;
   pp.out_values = nullptr;
@@ -1993,23 +1882,18 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
   if (U > 0) {
     c->mark("predict: begin");
     PredGeom g = predict_geometry(c, N);
-    RPK_REQUIRE(U * (int64_t)g.P < ((int64_t)1 << 31), "too many (user, item range) work items in one call; split the batch");
     ensure_segments(c, g);
     PredParams pp;
     fill_common(c, pp, g, U, indptr, indices, N, mask_history, PRED_TOPN);
-    pp.part_idx = c->buf<int>("p_part_idx", (size_t)U * g.P * N);
-    pp.part_sq = c->buf<u64>("p_part_sq", (size_t)U * g.P * N);
-    pp.part_len = c->buf<int>("p_part_len", (size_t)U * g.P);
+    pp.out_idx = o_idx.dev;
+    pp.out_val = o_val.dev;
+    pp.out_len = o_len.dev;
     const ModelScale* scale = c->get<ModelScale>("m_scale");
-    const int fgrid = (int)std::min<int64_t>((U * 32 + 255) / 256, (int64_t)c->sm_count * 16);
     // the block table of the 32-bit kernel indexes 4-entry blocks with 32 bits
     const Pred32Geom g2 = predict32_geometry(c, N);
     const bool blocks_fit = (c->m_nnz + 3 * c->m_I * g2.P) / 4 < (int64_t)0x7fffffff;
     if ((c->flags & DBG_WIDE_ACC) || !blocks_fit) {  // debug flag / giant models: every user through the two-limb kernel
       launch_predict(c, pp, g, U, indptr);
-      k_predict_finalize<<<fgrid, 256, 0, st>>>(pp.part_idx, pp.part_sq, pp.part_len, U, g.P, N, o_idx.dev, o_val.dev,
-                                                o_len.dev, nullptr, scale);
-      RPK_LAUNCH_CHECK(c);
     } else {
       ensure_blocks(c, g2.P, g2.R);
       Pred32Params qp;
@@ -2030,12 +1914,10 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
       qp.out_val = o_val.dev;
       qp.out_len = o_len.dev;
       qp.scale = scale;
-      // per-user flags: [0, U) handed to the two-limb kernel, [U] their count
-      int* flags = c->buf<int>("p_ovf_flag", (size_t)U + 1);
-      qp.ovf_flag = flags;
-      qp.ovf_count = flags + U;
+      // users handed to the two-limb kernel (each at most once: the handoff leaves the user's range loop)
+      qp.ovf_count = c->buf<int>("p_ovf_count", 1);
       qp.ovf_tab = c->buf<int4>("p_ovf_tab", (size_t)U);
-      RPK_CUDA(cudaMemsetAsync(flags, 0, sizeof(int) * ((size_t)U + 1), st));
+      RPK_CUDA(cudaMemsetAsync(qp.ovf_count, 0, sizeof(int), st));
       const PredWork w = prepare_work(c, U, indptr);
       qp.work_tab = w.tab;
       qp.queue = w.queue + 1;
@@ -2054,7 +1936,8 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
       k_predict_a32<<<grid, g2.nt, g2.smem, st>>>(qp);
       RPK_LAUNCH_CHECK(c);
       c->mark("predict: scoring kernel");
-      // users whose survivors overflowed the list: exact two-limb kernel (normally none; the kernel then exits)
+      // users whose survivors overflowed the list: exact two-limb kernel, which writes their final lists (normally
+      // none; the kernel then exits)
       pp.work_tab = qp.ovf_tab;
       pp.n_work = qp.ovf_count;
       pp.queue = w.queue;
@@ -2084,10 +1967,6 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
                 (double)h[12] / us, (double)h[13] / us, (double)h[14] / us, (double)h[3] / us);
       }
 #endif
-      // the two-limb kernel's lists of the handed-over users
-      k_predict_finalize<<<fgrid, 256, 0, st>>>(pp.part_idx, pp.part_sq, pp.part_len, U, g.P, N, o_idx.dev, o_val.dev, o_len.dev,
-                                                qp.ovf_flag, scale);
-      RPK_LAUNCH_CHECK(c);
     }
   }
   c->mark("predict: final lists");
@@ -2101,7 +1980,6 @@ void run_predict_csr_count(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* in
                            int mask_history, int64_t* out_row_nnz_u) {
   check_predict_args(c, U, nnz);
   RPK_REQUIRE(out_row_nnz_u, "out_row_nnz must not be null");
-  cudaStream_t st = c->stream;
   const int64_t* indptr = stage_in(c, indptr_u, (size_t)U + 1, "p_indptr");
   const int32_t* indices = stage_in(c, indices_u, (size_t)nnz, "p_indices");
   Out<int64_t> o;
@@ -2111,10 +1989,8 @@ void run_predict_csr_count(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* in
     ensure_segments(c, g);
     PredParams pp;
     fill_common(c, pp, g, U, indptr, indices, 1, mask_history, PRED_COUNT);
-    pp.pass_cnt = c->buf<int64_t>("p_pass_cnt", (size_t)U * g.P);
+    pp.out_row_nnz = o.dev;
     launch_predict(c, pp, g, U, indptr);
-    k_sum_passes<<<ceil_div(U, 256), 256, 0, st>>>(pp.pass_cnt, U, g.P, o.dev);
-    RPK_LAUNCH_CHECK(c);
     c->pc_U = U;
   }
   o.finish(c);
@@ -2146,7 +2022,6 @@ void run_predict_csr_fill(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* ind
   ensure_segments(c, g);
   PredParams pp;
   fill_common(c, pp, g, U, indptr, indices, 1, mask_history, PRED_FILL);
-  pp.pass_cnt = c->get<int64_t>("p_pass_cnt");
   pp.out_indptr = out_indptr;
   pp.out_indices = o_i.dev;
   pp.out_values = o_v.dev;

@@ -333,7 +333,7 @@ def test_predict_lists_only_near_ties_take_the_exact_pass(engine, flags):
     assert np.array_equal(full["idx"], want["idx"]) and np.array_equal(full["val"], want["val"])
 
 
-@pytest.mark.parametrize("flags", [0, 1, 4])
+@pytest.mark.parametrize("flags", [0, 1, 4, 32, 33])  # 32: four item ranges (the last holds 24 of the 120 items)
 def test_predict_full_csr_matches_oracle_and_reference(engine, flags):
     from recpack_b200.matrix import binary_structure
 

@@ -3,8 +3,8 @@
 The kernel runs the item ranges of a user one after the other on approximate 32-bit sums and leaves them only where it
 cannot prove the order.  Each case below builds a model and users that force one such branch:
 
-  handoff              more survivors than the list holds: the user goes to the two-limb kernel (k_predict +
-                       k_predict_finalize, flagged users only)
+  handoff              more survivors than the list holds: the user goes to the two-limb kernel (k_predict, which
+                       writes the final lists of the handed-over users only)
   carried retry        the bound carried from the earlier ranges lets more than cap - N items of a later range through:
                        that range is swept again with its own bound
   exact restart        an approximate entry of an earlier range is too close to a later range's exact one: the user is

@@ -1,6 +1,7 @@
 """Top-N scoring over several item ranges per user: the 32-bit kernel runs the ranges of a user one after the other,
 carries the survivor bound of the earlier ranges into the later ones and merges every range's survivors into one
-running list.  Each case below puts the deciding entries in a different place across the ranges; the lists (and the
+running list; the two-limb kernel (DBG_WIDE_ACC) offers its running list to the next range's selection as extra
+candidates.  Each case below puts the deciding entries in a different place across the ranges; the lists (and the
 scores, when asked for) must be the oracle's, bit for bit."""
 import numpy as np
 import pytest
@@ -10,7 +11,7 @@ from oracle import recpack_oracle as orc
 
 pytestmark = pytest.mark.gpu
 
-DBG_TINY_LIST, DBG_MULTI_PASS, DBG_MANY_PASS = 2, 4, 32  # two ranges / four ranges (at 64 items: 16 each)
+DBG_WIDE_ACC, DBG_TINY_LIST, DBG_MULTI_PASS, DBG_MANY_PASS = 1, 2, 4, 32  # two ranges / four ranges (at 64 items: 16 each)
 I = 64
 
 
@@ -85,7 +86,8 @@ def _random_rows(rng, U, lo=1, hi=12):
     return rows
 
 
-FLAGS = [DBG_MULTI_PASS, DBG_MANY_PASS, DBG_MANY_PASS | DBG_TINY_LIST]
+FLAGS = [DBG_MULTI_PASS, DBG_MANY_PASS, DBG_MANY_PASS | DBG_TINY_LIST,
+         DBG_WIDE_ACC | DBG_MULTI_PASS, DBG_WIDE_ACC | DBG_MANY_PASS, DBG_WIDE_ACC | DBG_MANY_PASS | DBG_TINY_LIST]
 
 
 @pytest.mark.parametrize("flags", FLAGS)
