@@ -172,6 +172,14 @@ RPK_EXPORT int64_t rpk_fit_token(const rpk_ctx* ctx);
 RPK_EXPORT int rpk_model_load_last_fit(rpk_ctx* ctx, int64_t token);
 RPK_EXPORT int rpk_model_load_csr(rpk_ctx* ctx, int64_t I, int64_t nnz,
                        const int64_t* indptr, const int32_t* indices, const double* values);
+/* A model of any sign (finite values, ascending unique columns per row), scored in float64 instead of fixed point:
+ * rpk_predict_topn / _csr_count / _csr_fill then return scipy's X @ S bit for bit -- every score is the left fold of
+ * s_ij over the user's history rows in their stored order, sums of exactly 0.0 are not stored, and the lists hold the
+ * N largest stored scores (score desc, item index asc), negative ones included when fewer than N positive ones exist.
+ * The history mask and the item filter apply as for the other models.  The rpk_model_load_* calls above keep
+ * rejecting negative values. */
+RPK_EXPORT int rpk_model_load_signed_csr(rpk_ctx* ctx, int64_t I, int64_t nnz,
+                              const int64_t* indptr, const int32_t* indices, const double* values);
 
 /*
  * Score U users: score_uj = sum over history items i of S_ij; optionally drop the user's own
@@ -181,6 +189,8 @@ RPK_EXPORT int rpk_model_load_csr(rpk_ctx* ctx, int64_t I, int64_t nnz,
  * The lists are the same with and without out_val.  Without it the kernel stops at 32-bit approximate sums
  * wherever those already prove the order (gaps larger than the error bound) and computes exact sums only for the
  * remaining lists.
+ * A model loaded with rpk_model_load_signed_csr is scored in float64 (scipy's X @ S, see there): out_val then holds the
+ * exact float64 sums, and a sum of exactly 0.0 is not listed.
  */
 RPK_EXPORT int rpk_predict_topn(rpk_ctx* ctx, int64_t U, int64_t nnz,
                      const int64_t* indptr, const int32_t* indices,

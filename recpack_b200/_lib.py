@@ -37,6 +37,7 @@ _SIGNATURES = {
     "rpk_fit_token": (C.c_int64, [C.c_void_p]),
     "rpk_model_load_last_fit": (C.c_int, [C.c_void_p, C.c_int64]),
     "rpk_model_load_csr": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _i64p, _i32p, _f64p]),
+    "rpk_model_load_signed_csr": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _i64p, _i32p, _f64p]),
     "rpk_predict_topn": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _i64p, _i32p, C.c_int, C.c_int, _i32p, _f64p, _i32p]),
     "rpk_predict_item_filter": (C.c_int, [C.c_void_p, _vp, C.c_int64]),
     "rpk_predict_csr_count": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _i64p, _i32p, C.c_int, _i64p]),

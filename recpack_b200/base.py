@@ -44,8 +44,13 @@ class GpuSimilarityMixin:
     With both unset ``predict`` returns every non-zero score like the reference.  Scores are exact sums
     of the similarities in fixed point relative to the largest similarity of the model
     (``q = rint(v * 2^e)`` with ``2^e * vmax`` in ``[2^39, 2^40)``, see DESIGN.md 2): they agree with the
-    reference's float64 sums to ``d_u * vmax * 2^-40`` and do not depend on summation order.  Similarity values
-    must be finite and non-negative (a signed, dense model such as EASE's has its own scorer: ``recpack_b200.EASE``)."""
+    reference's float64 sums to ``d_u * vmax * 2^-40`` and do not depend on summation order.
+
+    A model with at least one negative value (Pearson neighbours, embedding cosines, any signed weights) is scored
+    in float64 instead: ``predict`` is then scipy's ``X @ similarity_matrix_`` bit for bit (each score the left fold
+    over the user's history items in ascending order; sums of exactly 0.0 are not stored), and ``predict_topK``
+    keeps the N largest stored scores, negative ones included when fewer than N positive ones exist (DESIGN.md 2).
+    Similarity values must be finite."""
 
     predict_topK = None
     remove_history = False
@@ -146,9 +151,10 @@ class GpuSimilarityMixin:
                 if S.nnz and not np.all(S.data):
                     S = S.copy()
                     S.eliminate_zeros()
-                engine.model_load_csr(S.shape[0], np.ascontiguousarray(S.indptr, dtype=np.int64),
-                                      np.ascontiguousarray(S.indices, dtype=np.int32),
-                                      np.ascontiguousarray(S.data, dtype=np.float64))
+                # a model with a negative value is scored in float64 (X @ S bit for bit), any other in fixed point
+                load = engine.model_load_signed_csr if S.nnz and np.any(S.data < 0) else engine.model_load_csr
+                load(S.shape[0], np.ascontiguousarray(S.indptr, dtype=np.int64), np.ascontiguousarray(S.indices, dtype=np.int32),
+                     np.ascontiguousarray(S.data, dtype=np.float64))
             engine._model_key = key
             engine._model_owner = self  # keeps id(self) unique while it is the resident model
 
@@ -222,8 +228,9 @@ class GpuSimilarityMixin:
 
 
 class ItemSimilarityMatrixAlgorithm(GpuSimilarityMixin, _SimilarityBase):
-    """recpack/algorithms/base.py:220-279 with ``_predict`` on the GPU: any algorithm that sets a sparse,
-    non-negative ``similarity_matrix_`` in ``_fit`` scores through rpk_predict_*."""
+    """recpack/algorithms/base.py:220-279 with ``_predict`` on the GPU: any algorithm that sets a sparse
+    ``similarity_matrix_`` in ``_fit`` scores through rpk_predict_* -- in fixed point when it is non-negative, in
+    float64 (scipy's ``X @ S`` bit for bit) when it has a negative value."""
 
 
 class TopKItemSimilarityMatrixAlgorithm(GpuSimilarityMixin, _TopKBase):

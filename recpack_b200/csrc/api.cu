@@ -197,6 +197,13 @@ int rpk_model_load_csr(rpk_ctx* ctx, int64_t I, int64_t nnz, const int64_t* indp
   RPK_API_END(ctx)
 }
 
+int rpk_model_load_signed_csr(rpk_ctx* ctx, int64_t I, int64_t nnz, const int64_t* indptr, const int32_t* indices,
+                              const double* values) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_model_load_signed_csr(ctx, I, nnz, indptr, indices, values);
+  RPK_API_END(ctx)
+}
+
 int rpk_predict_topn(rpk_ctx* ctx, int64_t U, int64_t nnz, const int64_t* indptr, const int32_t* indices, int N,
                      int mask_history, int32_t* out_idx, double* out_val, int32_t* out_len) {
   RPK_API_BEGIN(ctx)

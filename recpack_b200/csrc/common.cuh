@@ -154,6 +154,7 @@ struct rpk_ctx {
   bool m_pad = false;  // padded block layout of the model is current
   int m_max_len = 0;  // longest model row
   int m_exp = 39;     // scale of the loaded model: q = rint(v * 2^m_exp)
+  bool m_signed = false;  // the model came from rpk_model_load_signed_csr (float64 scoring, k_predict_signed)
   int64_t filter_I = -1;  // item filter of the predict calls (buffer p_item_ok), -1 = none
   bool pack_flag_pending = false;  // a stream-ordered rpk_model_pack_rows_v left its validation flag unchecked
 

@@ -233,7 +233,9 @@ struct RealParams {
   int cap, direct_cap;
   int diag;       // 1: column i of row i is an explicit zero that competes in the selection (fit: setdiag)
   int mask_list;  // 1: the columns named by the list itself are removed (history removal in scoring)
+  const unsigned char* item_ok;  // non-null: item filter of the scoring (1 = may be recommended)
   int mode;       // 0: top-K lists; 1: count the stored entries per row; 2: write CSR rows (ascending columns)
+  const int* nrows_dev;  // non-null: device-side number of rows of `order` (replaces nrows)
   int* queue;
   int* scr_idx;  // [grid x (I + 1)]
   double* scr_val;
@@ -257,6 +259,7 @@ __global__ void __launch_bounds__(1024, 1) k_real_rows(RealParams p) {
   const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
   int* scr_idx = p.scr_idx + (int64_t)blockIdx.x * (p.I + 1);
   double* scr_val = p.scr_val + (int64_t)blockIdx.x * (p.I + 1);
+  const int nrows = p.nrows_dev ? *p.nrows_dev : p.nrows;
   for (;;) {
     __syncthreads();
     if (tid == 0) {
@@ -265,7 +268,7 @@ __global__ void __launch_bounds__(1024, 1) k_real_rows(RealParams p) {
       s_diag = -1;
     }
     __syncthreads();
-    if (s_row >= p.nrows) break;
+    if (s_row >= nrows) break;
     const int i = p.order[s_row];
     const int64_t ub = p.cscptr[i];
     const int nu = (int)(p.cscptr[i + 1] - ub);
@@ -322,6 +325,11 @@ __global__ void __launch_bounds__(1024, 1) k_real_rows(RealParams p) {
           const int j = p.csc_users[ub + k];
           if (j >= r0 && j < r1) acc[j - r0] = 0.0;
         }
+        __syncthreads();
+      }
+      if (p.item_ok) {  // postprocessing/filters.py:58-101, before the truncation
+        for (int t = tid; t < r1 - r0; t += nt)
+          if (!p.item_ok[r0 + t]) acc[t] = 0.0;
         __syncthreads();
       }
       if (p.mode == 0) {
@@ -592,7 +600,9 @@ void run_fit_real(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64_t* 
     rp.col_scale = col_scale;
     rp.diag = 1;
     rp.mask_list = 0;
+    rp.item_ok = nullptr;
     rp.mode = 0;
+    rp.nrows_dev = nullptr;
     rp.out_row_nnz = nullptr;
     rp.out_indptr = nullptr;
     rp.csr_indices = nullptr;
@@ -622,6 +632,92 @@ void run_fit_real(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64_t* 
   finish_call(c);
 }
 
+// Rows of C = A @ B through k_real_rows, every operand in device memory (a_val null: every left value is 1.0, a binary
+// history).  order null: all rows of A, heaviest first; else the rows order[0 .. *n_order) (n_order: device-side count,
+// at most `rows`).  item_ok (non-null) removes the filtered columns before the truncation to N.
+void spgemm_rows_device(rpk_ctx* c, int64_t rows, const int64_t* a_ptr, const int32_t* a_idx, const double* a_val, int64_t I,
+                        const int64_t* b_ptr, const int32_t* b_idx, const double* b_val, const int* order, const int* n_order, int N,
+                        int mask_history, const unsigned char* item_ok, int mode, int32_t* out_idx, double* out_val,
+                        int32_t* out_len, int64_t* out_row_nnz, const int64_t* out_indptr, int32_t* csr_indices,
+                        double* csr_values) {
+  if (rows <= 0) return;
+  cudaStream_t st = c->stream;
+  int* queue = c->buf<int>("sg_queue", 4);
+  RPK_CUDA(cudaMemsetAsync(queue, 0, sizeof(int) * 4, st));
+  if (!order) {
+    u64* work = c->buf<u64>("sg_work", (size_t)rows);
+    int* ord = c->buf<int>("sg_order", (size_t)rows);
+    int* bcnt = c->buf<int>("sg_bcnt", 65 * 2 + 2);
+    int* boff = bcnt + 65;
+    RPK_CUDA(cudaMemsetAsync(bcnt, 0, sizeof(int) * (65 * 2 + 2), st));
+    k_spgemm_work<<<(int)std::min<int64_t>((rows * 32 + 255) / 256, (int64_t)c->sm_count * 16), 256, 0, st>>>(a_ptr, a_idx, b_ptr, rows,
+                                                                                                        work);
+    RPK_LAUNCH_CHECK(c);
+    k_bucket_count<<<ceil_div(rows, 256), 256, 0, st>>>(work, 0, rows, bcnt);
+    RPK_LAUNCH_CHECK(c);
+    k_bucket_offsets<<<1, 32, 0, st>>>(bcnt, boff);
+    RPK_LAUNCH_CHECK(c);
+    k_bucket_scatter<<<ceil_div(rows, 256), 256, 0, st>>>(work, 0, rows, boff, ord);
+    RPK_LAUNCH_CHECK(c);
+    order = ord;
+  }
+  const bool tiny = c->flags & DBG_TINY_LIST;
+  const int cap = std::max(tiny ? 64 : 1024, next_pow2(2 * N));
+  const int direct_cap = tiny ? N : cap;
+  const size_t fixed = sel_smem_bytes(cap);
+  RPK_REQUIRE((size_t)c->smem_max > fixed + 4096 + 2048, "N too large for shared memory");
+  const size_t avail = (size_t)c->smem_max - fixed - 2048;
+  int64_t Rmax = (int64_t)(avail / sizeof(double)) & ~(int64_t)7;
+  int P = (int)((std::max<int64_t>(I, 1) + Rmax - 1) / Rmax);
+  if (P < 1) P = 1;
+  if ((c->flags & DBG_MULTI_PASS) && P < 2 && I >= 16) P = 2;
+  const int R = (int)(((std::max<int64_t>(I, 1) + P - 1) / P + 7) & ~(int64_t)7);
+  const size_t smem = fixed + (size_t)R * sizeof(double);
+  const int nt = R >= 8192 ? 1024 : (R >= 1024 ? 256 : 64);
+  RPK_CUDA(cudaFuncSetAttribute(k_real_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(rows, (int64_t)c->sm_count));
+  RealParams rp;
+  rp.indptr = b_ptr;
+  rp.indices = b_idx;
+  rp.left = nullptr;
+  rp.right = b_val;
+  rp.cscptr = a_ptr;
+  rp.csc_users = a_idx;
+  rp.csc_off = nullptr;
+  rp.left_entry = a_val;
+  // a few handed-over rows search their slices instead of paying for the table of all rows of B
+  rp.split = n_order ? nullptr : build_split(c, b_ptr, b_idx, I, I, P, R, nt, &rp.split_w);
+  if (n_order) rp.split_w = 0;
+  rp.row_scale = nullptr;
+  rp.col_scale = nullptr;
+  rp.order = order;
+  rp.nrows = (int)rows;
+  rp.nrows_dev = n_order;
+  rp.P = P;
+  rp.R = R;
+  rp.I = (int)I;
+  rp.K = N;
+  rp.item_begin = 0;
+  rp.cap = cap;
+  rp.direct_cap = direct_cap;
+  rp.diag = 0;
+  rp.mask_list = mask_history ? 1 : 0;
+  rp.item_ok = item_ok;
+  rp.mode = mode;
+  rp.queue = queue;
+  rp.scr_idx = c->buf<int>("fr_scr_idx", mode == 0 ? (size_t)grid * (size_t)(I + 1) : 16);
+  rp.scr_val = c->buf<double>("fr_scr_val", mode == 0 ? (size_t)grid * (size_t)(I + 1) : 16);
+  rp.out_idx = out_idx;
+  rp.out_val = out_val;
+  rp.out_len = out_len;
+  rp.out_row_nnz = reinterpret_cast<long long*>(out_row_nnz);
+  rp.out_indptr = out_indptr;
+  rp.csr_indices = csr_indices;
+  rp.csr_values = csr_values;
+  k_real_rows<<<grid, nt, smem, st>>>(rp);
+  RPK_LAUNCH_CHECK(c);
+}
+
 // C = A @ B for a real-valued CSR A [rows x I] and a CSR B [I x I] with ascending columns (the similarity model), float64
 // in scipy's csr_matmat order (bit-identical sums): per-row top-N lists (mode 0), stored entries per row (mode 1) or the
 // CSR rows themselves (mode 2, out_indptr from the counts).  Replaces `X_decayed @ similarity_matrix_` of
@@ -646,7 +742,6 @@ void run_spgemm(rpk_ctx* c, int64_t rows, int64_t a_nnz, const int64_t* a_indptr
     RPK_REQUIRE(out_indptr_u && (out_nnz == 0 || (csr_indices_u && csr_values_u)), "CSR outputs must not be null");
     N = 1;
   }
-  cudaStream_t st = c->stream;
   const int64_t* a_ptr = stage_in(c, a_indptr_u, (size_t)rows + 1, "sg_a_ptr");
   const int32_t* a_idx = stage_in(c, a_indices_u, (size_t)a_nnz, "sg_a_idx");
   const double* a_val = stage_in(c, a_values_u, (size_t)a_nnz, "sg_a_val");
@@ -668,75 +763,8 @@ void run_spgemm(rpk_ctx* c, int64_t rows, int64_t a_nnz, const int64_t* a_indptr
     o_cv.init(c, csr_values_u, (size_t)out_nnz, "sg_out_cv");
   }
   c->mark("spgemm: begin");
-  if (rows > 0) {
-    u64* work = c->buf<u64>("sg_work", (size_t)rows);
-    int* order = c->buf<int>("sg_order", (size_t)rows);
-    int* bcnt = c->buf<int>("sg_bcnt", 65 * 2 + 2);
-    int* boff = bcnt + 65;
-    int* queue = c->buf<int>("sg_queue", 4);
-    RPK_CUDA(cudaMemsetAsync(bcnt, 0, sizeof(int) * (65 * 2 + 2), st));
-    RPK_CUDA(cudaMemsetAsync(queue, 0, sizeof(int) * 4, st));
-    k_spgemm_work<<<(int)std::min<int64_t>((rows * 32 + 255) / 256, (int64_t)c->sm_count * 16), 256, 0, st>>>(a_ptr, a_idx, b_ptr, rows,
-                                                                                                        work);
-    RPK_LAUNCH_CHECK(c);
-    k_bucket_count<<<ceil_div(rows, 256), 256, 0, st>>>(work, 0, rows, bcnt);
-    RPK_LAUNCH_CHECK(c);
-    k_bucket_offsets<<<1, 32, 0, st>>>(bcnt, boff);
-    RPK_LAUNCH_CHECK(c);
-    k_bucket_scatter<<<ceil_div(rows, 256), 256, 0, st>>>(work, 0, rows, boff, order);
-    RPK_LAUNCH_CHECK(c);
-    const bool tiny = c->flags & DBG_TINY_LIST;
-    const int cap = std::max(tiny ? 64 : 1024, next_pow2(2 * N));
-    const int direct_cap = tiny ? N : cap;
-    const size_t fixed = sel_smem_bytes(cap);
-    RPK_REQUIRE((size_t)c->smem_max > fixed + 4096 + 2048, "N too large for shared memory");
-    const size_t avail = (size_t)c->smem_max - fixed - 2048;
-    int64_t Rmax = (int64_t)(avail / sizeof(double)) & ~(int64_t)7;
-    int P = (int)((std::max<int64_t>(I, 1) + Rmax - 1) / Rmax);
-    if (P < 1) P = 1;
-    if ((c->flags & DBG_MULTI_PASS) && P < 2 && I >= 16) P = 2;
-    const int R = (int)(((std::max<int64_t>(I, 1) + P - 1) / P + 7) & ~(int64_t)7);
-    const size_t smem = fixed + (size_t)R * sizeof(double);
-    const int nt = R >= 8192 ? 1024 : (R >= 1024 ? 256 : 64);
-    RPK_CUDA(cudaFuncSetAttribute(k_real_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(rows, (int64_t)c->sm_count));
-    RealParams rp;
-    rp.indptr = b_ptr;
-    rp.indices = b_idx;
-    rp.left = nullptr;
-    rp.right = b_val;
-    rp.cscptr = a_ptr;
-    rp.csc_users = a_idx;
-    rp.csc_off = nullptr;
-    rp.left_entry = a_val;
-    rp.split = build_split(c, b_ptr, b_idx, I, I, P, R, nt, &rp.split_w);
-    rp.row_scale = nullptr;
-    rp.col_scale = nullptr;
-    rp.order = order;
-    rp.nrows = (int)rows;
-    rp.P = P;
-    rp.R = R;
-    rp.I = (int)I;
-    rp.K = N;
-    rp.item_begin = 0;
-    rp.cap = cap;
-    rp.direct_cap = direct_cap;
-    rp.diag = 0;
-    rp.mask_list = mask_history ? 1 : 0;
-    rp.mode = mode;
-    rp.queue = queue;
-    rp.scr_idx = c->buf<int>("fr_scr_idx", mode == 0 ? (size_t)grid * (size_t)(I + 1) : 16);
-    rp.scr_val = c->buf<double>("fr_scr_val", mode == 0 ? (size_t)grid * (size_t)(I + 1) : 16);
-    rp.out_idx = o_idx.dev;
-    rp.out_val = o_val.dev;
-    rp.out_len = o_len.dev;
-    rp.out_row_nnz = reinterpret_cast<long long*>(o_cnt.dev);
-    rp.out_indptr = o_ptr;
-    rp.csr_indices = o_ci.dev;
-    rp.csr_values = o_cv.dev;
-    k_real_rows<<<grid, nt, smem, st>>>(rp);
-    RPK_LAUNCH_CHECK(c);
-  }
+  spgemm_rows_device(c, rows, a_ptr, a_idx, a_val, I, b_ptr, b_idx, b_val, nullptr, nullptr, N, mask_history, nullptr, mode, o_idx.dev,
+                     o_val.dev, o_len.dev, o_cnt.dev, o_ptr, o_ci.dev, o_cv.dev);
   c->mark("spgemm: rows");
   o_idx.finish(c);
   o_val.finish(c);

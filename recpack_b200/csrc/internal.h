@@ -48,6 +48,13 @@ void run_spgemm(rpk_ctx* c, int64_t rows, int64_t a_nnz, const int64_t* a_indptr
                 int64_t I, int64_t b_nnz, const int64_t* b_indptr, const int32_t* b_indices, const double* b_values, int N,
                 int mask_history, int mode, int32_t* out_idx, double* out_val, int32_t* out_len, int64_t* out_row_nnz,
                 const int64_t* out_indptr, int64_t out_nnz, int32_t* csr_indices, double* csr_values);
+void spgemm_rows_device(rpk_ctx* c, int64_t rows, const int64_t* a_ptr, const int32_t* a_idx, const double* a_val, int64_t I,
+                        const int64_t* b_ptr, const int32_t* b_idx, const double* b_val, const int* order, const int* n_order, int N,
+                        int mask_history, const unsigned char* item_ok, int mode, int32_t* out_idx, double* out_val,
+                        int32_t* out_len, int64_t* out_row_nnz, const int64_t* out_indptr, int32_t* csr_indices,
+                        double* csr_values);
+void run_model_load_signed_csr(rpk_ctx* c, int64_t I, int64_t nnz, const int64_t* indptr, const int32_t* indices,
+                               const double* values);
 void run_split_fraction(rpk_ctx* c, int64_t n_users, const int64_t* uids, const int64_t* seg, const int64_t* rows,
                         int64_t n_rows, double in_frac, uint64_t seed, uint8_t* out_in_mask);
 void run_gram_dense_f64(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64_t* indptr, const int32_t* indices, double* out_G);

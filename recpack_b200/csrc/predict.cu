@@ -16,7 +16,10 @@
 //   k_predict      full CSR output, and the exact path for users k_predict_a32 hands over: one CTA per user runs
 //                  its item ranges in order, the sum is kept in two 32-bit limbs (q & 0xFFFFF, q >> 20), 64-bit
 //                  accumulators when a limb could overflow.
+#include <limits.h>
+#include <math.h>
 #include <stdlib.h>
+#include <string.h>
 
 #include <type_traits>
 
@@ -285,6 +288,7 @@ static void model_common_begin(rpk_ctx* c, int64_t I) {
   c->m_P = 0;  // segment tables must be rebuilt
   c->m_P2 = 0;
   c->m_pad = false;
+  c->m_signed = false;
   int* flag = c->buf<int>("m_flag", 1);
   RPK_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), c->stream));
   RPK_CUDA(cudaMemsetAsync(c->buf<u64>("m_vmax", 1), 0, sizeof(u64), c->stream));
@@ -1866,6 +1870,9 @@ static void check_predict_args(rpk_ctx* c, int64_t U, int64_t nnz) {
   RPK_REQUIRE(c->bufs.count("m_scale") != 0, "no similarity model loaded (call rpk_model_load_* first)");
 }
 
+static void predict_signed_topn(rpk_ctx* c, int64_t U, const int64_t* indptr, const int32_t* indices, int N, int mask_history,
+                                int32_t* out_idx, double* out_val, int32_t* out_len);
+
 void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_u, const int32_t* indices_u, int N,
                       int mask_history, int32_t* out_idx_u, double* out_val_u, int32_t* out_len_u) {
   check_predict_args(c, U, nnz);
@@ -1879,7 +1886,11 @@ void run_predict_topn(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr_
   o_idx.init(c, out_idx_u, (size_t)U * N, "p_out_idx");
   o_val.init(c, out_val_u, (size_t)U * N, "p_out_val");
   o_len.init(c, out_len_u, (size_t)U, "p_out_len");
-  if (U > 0) {
+  if (U > 0 && c->m_signed) {
+    // exact float64 scores are computed for every list either way; without out_val they go to a scratch buffer
+    double* val = o_val.dev ? o_val.dev : c->buf<double>("ps_val", (size_t)U * N);
+    predict_signed_topn(c, U, indptr, indices, N, mask_history, o_idx.dev, val, o_len.dev);
+  } else if (U > 0) {
     c->mark("predict: begin");
     PredGeom g = predict_geometry(c, N);
     ensure_segments(c, g);
@@ -1984,7 +1995,12 @@ void run_predict_csr_count(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* in
   const int32_t* indices = stage_in(c, indices_u, (size_t)nnz, "p_indices");
   Out<int64_t> o;
   o.init(c, out_row_nnz_u, (size_t)U, "p_row_nnz");
-  if (U > 0) {
+  if (U > 0 && c->m_signed) {
+    spgemm_rows_device(c, U, indptr, indices, nullptr, c->m_I, c->get<int64_t>("m_ptr"), c->get<int>("ms_idx"),
+                       c->get<double>("ms_val"), nullptr, nullptr, 1, mask_history, item_filter_ptr(c), PRED_COUNT, nullptr,
+                       nullptr, nullptr, o.dev, nullptr, nullptr, nullptr);
+    c->pc_U = U;
+  } else if (U > 0) {
     PredGeom g = predict_geometry(c, 1);
     ensure_segments(c, g);
     PredParams pp;
@@ -2018,6 +2034,15 @@ void run_predict_csr_fill(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* ind
   Out<double> o_v;
   o_i.init(c, out_indices_u, (size_t)total, "p_csr_idx");
   o_v.init(c, out_values_u, (size_t)total, "p_csr_val");
+  if (c->m_signed) {
+    spgemm_rows_device(c, U, indptr, indices, nullptr, c->m_I, c->get<int64_t>("m_ptr"), c->get<int>("ms_idx"),
+                       c->get<double>("ms_val"), nullptr, nullptr, 1, mask_history, item_filter_ptr(c), PRED_FILL, nullptr,
+                       nullptr, nullptr, nullptr, out_indptr, o_i.dev, o_v.dev);
+    o_i.finish(c);
+    o_v.finish(c);
+    finish_call(c);
+    return;
+  }
   PredGeom g = predict_geometry(c, 1);
   ensure_segments(c, g);
   PredParams pp;
@@ -2029,6 +2054,535 @@ void run_predict_csr_fill(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* ind
   o_i.finish(c);
   o_v.finish(c);
   finish_call(c);
+}
+
+
+// ------------------------------------------------------------------------------------------
+// Signed models: float64 scores, bit-identical to scipy's X @ S
+// ------------------------------------------------------------------------------------------
+// A model with negative values is scored in float64: score_uj is the left fold of s_ij over the user's history rows in
+// their stored (ascending) order, exactly scipy's csr_matmat, and a sum of exactly 0.0 is not stored.  k_predict_signed
+// screens with signed fixed-point sums and folds in float64 only the items that can reach the list:
+//   model    every entry is kept as (q << 24) | column, q = rint(v * 2^e) signed (|q| <= 2^38, e from max |v|), next to
+//            its float64 value and column; rowmax = ceil(max |q| / 2^20) per row.
+//   screen   the accumulator of item j is x = (sum of t_ij) * 2^c + (rows that touched j), t_ij = floor(q_ij / 2^sft),
+//            c = bits of d (the history length), so x != 0 exactly when j was touched and a = x >> c is the signed sum.
+//            sft is the smallest shift with (sum of rowmax * 2^20 >> sft + d) * 2^c + d < 2^31: no int32 overflow.
+//            With unit = 2^(sft - e), each term satisfies v / unit in [t - 1/2, t + 3/2) (floor plus rint), and the
+//            float64 fold differs from the real sum by at most gamma_{d-1} * sum |v| < unit (d < 2048), so the
+//            float64 score lies in unit * [a - W, a + W], W = 2d + 2.
+//   bound    L = the larger of (a_N - W) * unit, a_N the N-th largest of the per-thread maxima of a (N distinct items
+//            reach it), and the N-th exact score carried from the earlier item ranges.  Survivors: the touched items
+//            with (a + W) * unit >= L; every other item of the range scores strictly below L.
+//   exact    the survivors' scores are folded in float64 in history order (their s_ij gathered into shared memory a
+//            chunk of rows at a time), exact zeros dropped, merged with the carried list, ordered by (score desc,
+//            column asc).  The list is proven when no touched item was screened out, or when its N-th score >= L.
+//   fallback the user goes to the float64 row kernel (k_real_rows) when the survivors do not fit the list, when the
+//            list is not proven (exact zeros left fewer than N scores >= L), and for histories of >= 2048 rows.
+constexpr int SG_NT = 512;
+constexpr int SG_EXACT_D = 2048;
+#ifdef RPK_PHASE_PROF
+constexpr int SG_LONG_SEG = 1024;  // counted: model row segments longer than this
+#endif
+
+__global__ void k_signed_vmax(const double* __restrict__ val, int64_t n, u64* __restrict__ vmax_bits, int* __restrict__ flag) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  u64 best = 0;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
+    const double v = fabs(val[t]);
+    if (!(v <= 1.7976931348623157e308)) atomicOr(flag, 1);  // NaN or infinite
+    else best = max(best, (u64)__double_as_longlong(v));
+  }
+  best = warp_max_u64(best);
+  if ((threadIdx.x & 31) == 0 && best) atomicMax(vmax_bits, best);
+}
+
+// One warp per row of a CSR with ascending unique columns.
+__global__ void k_model_from_signed_csr(const int64_t* __restrict__ indptr, const int* __restrict__ indices,
+                                        const double* __restrict__ values, int64_t I, int e, u64* __restrict__ ent,
+                                        unsigned* __restrict__ rowmax, int* __restrict__ flag) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < I; i += nwarps) {
+    const int64_t b = indptr[i], en = indptr[i + 1];
+    u64 qmax = 0;
+    for (int64_t k = b + lane; k < en; k += 32) {
+      const int j = indices[k];
+      if (j < 0 || j >= I) atomicOr(flag, 1);
+      if (k > b && indices[k - 1] >= j) atomicOr(flag, 2);
+      const long long q = __double2ll_rn(scalbn(values[k], e));  // |q| <= 2^38
+      qmax = max(qmax, (u64)(q < 0 ? -q : q));
+      ent[k] = ((u64)q << 24) | (u64)(unsigned)(j & 0xffffff);
+    }
+    qmax = warp_max_u64(qmax);
+    if (lane == 0) rowmax[i] = (unsigned)((qmax + 0xfffffull) >> 20);
+  }
+}
+
+void run_model_load_signed_csr(rpk_ctx* c, int64_t I, int64_t nnz, const int64_t* indptr_u, const int32_t* indices_u,
+                               const double* values_u) {
+  model_common_begin(c, I);
+  RPK_REQUIRE(nnz >= 0, "negative nnz");
+  cudaStream_t st = c->stream;
+  const int64_t* indptr = stage_in(c, indptr_u, (size_t)I + 1, "m_in_ptr");
+  const int32_t* indices = stage_in(c, indices_u, (size_t)nnz, "m_in_idx");
+  const double* values = stage_in(c, values_u, (size_t)nnz, "m_in_val");
+  int64_t* m_ptr = c->buf<int64_t>("m_ptr", (size_t)I + 1);
+  int32_t* m_idx = c->buf<int32_t>("ms_idx", (size_t)nnz);
+  double* m_val = c->buf<double>("ms_val", (size_t)nnz);
+  RPK_CUDA(cudaMemcpyAsync(m_ptr, indptr, sizeof(int64_t) * ((size_t)I + 1), cudaMemcpyDeviceToDevice, st));
+  RPK_CUDA(cudaMemcpyAsync(m_idx, indices, sizeof(int32_t) * (size_t)nnz, cudaMemcpyDeviceToDevice, st));
+  RPK_CUDA(cudaMemcpyAsync(m_val, values, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToDevice, st));
+  u64* vmax = c->get<u64>("m_vmax");
+  int* flag = c->get<int>("m_flag");
+  if (nnz > 0) {
+    k_signed_vmax<<<(int)std::min<int64_t>(ceil_div(nnz, 256), (int64_t)c->sm_count * 16), 256, 0, st>>>(values, nnz, vmax, flag);
+    RPK_LAUNCH_CHECK(c);
+  }
+  u64 vb = 0;
+  int64_t ends[2] = {0, 0};
+  RPK_CUDA(cudaMemcpyAsync(&vb, vmax, sizeof(u64), cudaMemcpyDeviceToHost, st));
+  RPK_CUDA(cudaMemcpyAsync(&ends[0], m_ptr, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  RPK_CUDA(cudaMemcpyAsync(&ends[1], m_ptr + I, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  RPK_CUDA(cudaStreamSynchronize(st));
+  if (!(ends[0] == 0 && ends[1] == nnz)) {
+    c->m_I = 0;
+    throw Error("similarity model: indptr does not match nnz");
+  }
+  double vm = 0.0;
+  memcpy(&vm, &vb, sizeof(vm));
+  const int e = vm > 0.0 ? 37 - ilogb(vm) : 37;  // max |v| * 2^e in [2^37, 2^38)
+  u64* ent = c->buf<u64>("ms_ent", (size_t)nnz);
+  unsigned* rowmax = c->buf<unsigned>("ms_rowmax", (size_t)I);
+  if (I > 0) {
+    const int grid = (int)std::min<int64_t>((I * 32 + 255) / 256, (int64_t)c->sm_count * 16);
+    k_model_from_signed_csr<<<grid, 256, 0, st>>>(indptr, indices, values, I, e, ent, rowmax, flag);
+    RPK_LAUNCH_CHECK(c);
+  }
+  int h = 0;
+  RPK_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+  RPK_CUDA(cudaStreamSynchronize(st));
+  if (h & 1) {
+    c->m_I = 0;
+    throw Error("similarity model: values must be finite, columns in [0, I)");
+  }
+  if (h & 2) {
+    c->m_I = 0;
+    throw Error("similarity model: column indices must be unique and ascending within a row");
+  }
+  ModelScale hs;
+  hs.e = e;
+  hs.inv = ldexp(1.0, -e);
+  hs.pad = 0;
+  RPK_CUDA(cudaMemcpyAsync(c->get<ModelScale>("m_scale"), &hs, sizeof(hs), cudaMemcpyHostToDevice, st));
+  RPK_CUDA(cudaStreamSynchronize(st));
+  c->m_exp = e;
+  c->m_nnz = nnz;
+  c->m_max_len = 0;
+  c->m_signed = true;
+  c->mark("model: signed CSR loaded (sync)");
+}
+
+// seg[i * (P + 1) + p] = offset inside row i of the first entry with column >= p * R
+__global__ void k_signed_seg(const int64_t* __restrict__ m_ptr, const int* __restrict__ m_idx, int64_t I, int P, int R,
+                             int* __restrict__ seg) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= I * (P + 1)) return;
+  const int64_t i = t / (P + 1);
+  const int p = (int)(t % (P + 1));
+  const int64_t b = m_ptr[i];
+  int lo = 0, hi = (int)(m_ptr[i + 1] - b);
+  const int64_t target = (int64_t)p * R;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (m_idx[b + mid] < target) lo = mid + 1;
+    else hi = mid;
+  }
+  seg[t] = lo;
+}
+
+struct SignedParams {
+  const int* indices;    // histories (CSR columns of the users)
+  const int4* work_tab;  // {user, history length, row start lo, hi} in processing order
+  const int64_t* m_ptr;
+  const int* seg;        // [I x (P + 1)] offset of every item range inside every model row
+  const u64* ent;        // (q << 24) | column
+  const double* val;     // float64 values of the entries
+  const unsigned* rowmax;
+  int U, P, R, N, mask, cap, gbuf, e;
+  int* queue;
+  int* out_idx;
+  double* out_val;
+  int* out_len;
+  const unsigned char* item_ok;  // non-null: item filter (1 = may be recommended)
+  int* ovf_count;                // users handed to the float64 row kernel ...
+  int* ovf_users;                // ... and their ids
+  unsigned long long* prof;      // instrumented build: path counters
+};
+
+__host__ __device__ __forceinline__ size_t sg_fixed_bytes(int cap, int gbuf) {
+  return (size_t)(cap + SEL_RANK_MAX) * sizeof(Entry) + (size_t)cap * sizeof(double) + (size_t)gbuf * sizeof(double) +
+         (size_t)SG_NT * (sizeof(int64_t) + sizeof(int));
+}
+
+__device__ __forceinline__ u64 sg_key(double v) {  // orders like v (v is never NaN)
+  const u64 b = (u64)__double_as_longlong(v);
+  return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double sg_value(u64 k) {
+  const u64 b = (k >> 63) ? (k & 0x7fffffffffffffffull) : ~k;
+  return __longlong_as_double((long long)b);
+}
+
+#ifdef RPK_PHASE_PROF
+#define SG_COUNT(k, v) \
+  do {                 \
+    if (tid == 0) atomicAdd(p.prof + (k), (unsigned long long)(v)); \
+  } while (0)
+#else
+#define SG_COUNT(k, v) do {} while (0)
+#endif
+enum { SGC_USERS, SGC_RANGES, SGC_SURVIVORS, SGC_OVERLAP, SGC_OVERFLOW, SGC_ZEROS, SGC_HEAVY, SGC_LONG, SGC_N };
+
+// One CTA per user (heaviest first from a shared counter); the user's item ranges run in order on the same
+// accumulators, which are all zero between ranges.
+__global__ void __launch_bounds__(SG_NT) k_predict_signed(SignedParams p) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  Entry* list = reinterpret_cast<Entry*>(smem);  // the user's running list, then this range's survivors behind it
+  Entry* list2 = list + p.cap;                   // SEL_RANK_MAX entries
+  double* fsum = reinterpret_cast<double*>(list2 + SEL_RANK_MAX);  // float64 folds of the survivors
+  double* gbuf = fsum + p.cap;                   // gathered s_ij: [rows of a chunk x survivors]
+  int64_t* tab_b = reinterpret_cast<int64_t*>(gbuf + p.gbuf);  // staged rows: first entry of the range's segment ...
+  int* tab_n = reinterpret_cast<int*>(tab_b + SG_NT);          // ... and its length
+  int* acc = tab_n + SG_NT;
+  __shared__ int s_w, s_cnt, s_out, s_keep;
+  __shared__ unsigned long long s_b20;
+  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
+  const int N = p.N, P = p.P;
+  for (int t = tid; t < p.R; t += nt) acc[t] = 0;
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) {
+      s_w = atomicAdd(p.queue, 1);
+      s_b20 = 0ull;
+    }
+    __syncthreads();
+    const int w = s_w;
+    if (w >= p.U) break;
+    const int4 rec = p.work_tab[w];
+    const int u = rec.x, d = rec.y;
+    const int64_t xb = ((int64_t)(unsigned)rec.z) | ((int64_t)rec.w << 32);
+    SG_COUNT(SGC_USERS, 1);
+    if (d == 0) {  // user without history: empty prediction row
+      for (int t = tid; t < N; t += nt) {
+        p.out_idx[(int64_t)u * N + t] = -1;
+        p.out_val[(int64_t)u * N + t] = 0.0;
+      }
+      if (tid == 0) p.out_len[u] = 0;
+      continue;
+    }
+    if (d >= SG_EXACT_D) {  // the margin 2d + 2 would let too much through: float64 row kernel
+      if (tid == 0) p.ovf_users[atomicAdd(p.ovf_count, 1)] = u;
+      SG_COUNT(SGC_HEAVY, 1);
+      continue;
+    }
+    // ---- shift of the fixed-point sums from the bound of the user's rows
+    {
+      u64 b = 0;
+      for (int r = tid; r < d; r += nt) b += p.rowmax[p.indices[xb + r]];
+      b = __reduce_add_sync(0xffffffffu, (unsigned)b);  // d < 2048 rows of at most 2^18 + 1 each: fits 32 bits
+      if (lane == 0 && b) atomicAdd(&s_b20, b);
+    }
+    __syncthreads();
+    const u64 B = s_b20 << 20;
+    const int cb = 32 - __clz(d);  // count field: d < 2^cb
+    int sft = 0;
+    while ((((B >> sft) + (u64)d) << cb) + (u64)d > 0x7fffffffull) ++sft;
+    const int sh = 24 + sft;
+    const long long W = 2ll * d + 2;
+    const int uexp = sft - p.e;  // unit = 2^uexp
+    int r = 0;                   // entries of the running list (best first, exact)
+    bool handed = false;
+    for (int pass = 0; pass < P && !handed; ++pass) {
+      const int r0 = pass * p.R;
+      // ---- screen: one shared-memory reduction per model entry
+      for (int c0 = 0; c0 < d; c0 += SG_NT) {
+        const int n = min(SG_NT, d - c0);
+        __syncthreads();
+        if (tid < n) {
+          const int i = p.indices[xb + c0 + tid];
+          const int* sg = p.seg + (int64_t)i * (P + 1) + pass;
+          const int s0 = sg[0], s1 = sg[1];
+          tab_b[tid] = p.m_ptr[i] + s0;
+          tab_n[tid] = s1 - s0;
+#ifdef RPK_PHASE_PROF
+          if (s1 - s0 > SG_LONG_SEG) atomicAdd(p.prof + SGC_LONG, 1ull);
+#endif
+        }
+        __syncthreads();
+        for (int rr = warp; rr < n; rr += nwarps) {
+          const u64* row = p.ent + tab_b[rr];
+          const int len = tab_n[rr];
+          for (int k = lane; k < len; k += 32) {
+            const u64 e = __ldg(row + k);
+            const unsigned add = ((unsigned)(int)((long long)e >> sh) << cb) + 1u;
+            asm volatile("red.shared.add.u32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(acc + ((int)(e & 0xffffff) - r0))),
+                         "r"(add)
+                         : "memory");
+          }
+        }
+      }
+      __syncthreads();
+      const int ns = p.R;  // slots of this range (those beyond the last item are never touched)
+      if (p.mask) {  // pipelines/pipeline.py:174-175, before the truncation to N
+        for (int rr = tid; rr < d; rr += nt) {
+          const int j = p.indices[xb + rr] - r0;
+          if (j >= 0 && j < ns) acc[j] = 0;
+        }
+      }
+      if (p.item_ok) {  // postprocessing/filters.py:58-101
+        for (int t = tid; t < ns; t += nt)
+          if (acc[t] && !p.item_ok[r0 + t]) acc[t] = 0;
+      }
+      __syncthreads();
+      // ---- bound: the N-th largest of the per-thread maxima of a (bit by bit, one block count per bit)
+      unsigned mykey = 0u;  // 0: no touched slot; else a ^ 2^31 (orders like a)
+      for (int t = tid; t < ns; t += nt) {
+        const int x = acc[t];
+        if (x) mykey = max(mykey, (unsigned)(x >> cb) ^ 0x80000000u);
+      }
+      if (tid == 0) {
+        s_cnt = 0;
+        s_out = 0;
+        s_keep = 0;
+      }
+      long long thr = LLONG_MIN;  // survivors: a >= thr
+      double L = -INFINITY;       // the N-th stored score is at least L (when the list is proven)
+      if (__syncthreads_count(mykey != 0u) >= N) {
+        unsigned pre = 0u;
+        for (int bit = 31; bit >= 0; --bit) {
+          const unsigned cand = pre | (1u << bit);
+          if (__syncthreads_count(mykey >= cand) >= N) pre = cand;
+        }
+        const long long aN = (long long)(int)(pre ^ 0x80000000u);
+        thr = aN - 2 * W;
+        L = scalbn((double)(aN - W), uexp);
+      }
+      if (r >= N) {  // the carried N-th exact score
+        const double EN = sg_value(list[N - 1].key);
+        const double up = ceil(scalbn(EN, -uexp));
+        const long long tc = up > 4.0e18 ? LLONG_MAX / 2 : (up < -4.0e18 ? LLONG_MIN / 2 : (long long)up - W);
+        thr = max(thr, tc);
+        L = fmax(L, EN);
+      }
+      // ---- survivors behind the running list; every touched slot is cleared
+      const int room = p.cap - r;
+      for (int t = tid; t < ns; t += nt) {
+        const int x = acc[t];
+        if (!x) continue;
+        acc[t] = 0;
+        if ((long long)(x >> cb) >= thr) {
+          const int pos = atomicAdd(&s_cnt, 1);
+          if (pos < room) {
+            Entry en;
+            en.key = 0ull;
+            en.idx = r0 + t;
+            en.aux = 0;
+            list[r + pos] = en;
+          }
+        } else {
+          s_out = 1;
+        }
+      }
+      __syncthreads();
+      const int m = s_cnt;
+      const bool screened_out = s_out != 0;
+      SG_COUNT(SGC_RANGES, 1);
+      SG_COUNT(SGC_SURVIVORS, m);
+      if (m > N) SG_COUNT(SGC_OVERLAP, 1);
+      if (m > room) {  // the survivors do not fit the list
+        if (tid == 0) p.ovf_users[atomicAdd(p.ovf_count, 1)] = u;
+        SG_COUNT(SGC_OVERFLOW, 1);
+        handed = true;
+        break;
+      }
+      // ---- exact pass: float64 left folds of the survivors, rows in history order
+      if (m > 0) {
+        Entry* sv = list + r;
+        for (int t = tid; t < m; t += nt) {
+          acc[sv[t].idx - r0] = t + 1;
+          fsum[t] = 0.0;
+        }
+        const int dc = min(SG_NT, max(1, p.gbuf / m));  // rows per gathered chunk
+        int tc0 = 0, tn = min(SG_NT, d);                // rows staged in the table (the last screen chunk)
+        if (d > SG_NT) tc0 = ((d - 1) / SG_NT) * SG_NT, tn = d - tc0;
+        for (int g0 = 0; g0 < d; g0 += dc) {
+          const int gn = min(dc, d - g0);
+          __syncthreads();  // the previous chunk is folded
+          if (g0 < tc0 || g0 + gn > tc0 + tn) {
+            tc0 = g0;
+            tn = min(SG_NT, d - g0);
+            if (tid < tn) {
+              const int i = p.indices[xb + tc0 + tid];
+              const int* sg = p.seg + (int64_t)i * (P + 1) + pass;
+              tab_b[tid] = p.m_ptr[i] + sg[0];
+              tab_n[tid] = sg[1] - sg[0];
+            }
+          }
+          for (int t = tid; t < gn * m; t += nt) gbuf[t] = 0.0;
+          __syncthreads();
+          for (int rr = warp; rr < gn; rr += nwarps) {
+            const int64_t b = tab_b[g0 - tc0 + rr];
+            const int len = tab_n[g0 - tc0 + rr];
+            for (int k = lane; k < len; k += 32) {
+              const int sidx = acc[(int)(__ldg(p.ent + b + k) & 0xffffff) - r0];
+              if (sidx) gbuf[rr * m + sidx - 1] = __ldg(p.val + b + k);
+            }
+          }
+          __syncthreads();
+          for (int t = tid; t < m; t += nt) {
+            double f = fsum[t];
+            for (int k = 0; k < gn; ++k) f = __dadd_rn(f, gbuf[k * m + t]);  // + 0.0 where row k has no entry j
+            fsum[t] = f;
+          }
+        }
+        __syncthreads();
+        // stored survivors (non-zero folds) -> gbuf as entries, then back behind the running list
+        Entry* tmp = reinterpret_cast<Entry*>(gbuf);
+        for (int t = tid; t < m; t += nt) {
+          Entry en = sv[t];
+          acc[en.idx - r0] = 0;
+          const double v = fsum[t];
+          if (v != 0.0) {
+            en.key = sg_key(v);
+            tmp[atomicAdd(&s_keep, 1)] = en;
+          }
+        }
+        __syncthreads();
+        const int kept = s_keep;
+        for (int t = tid; t < kept; t += nt) sv[t] = tmp[t];
+        __syncthreads();
+        const int tot = r + kept;
+        Entry* s = tot > 1 ? a32_order(list, list2, tot) : list;
+        const int keep = min(tot, N);
+        if (s != list) {
+          for (int t = tid; t < keep; t += nt) list[t] = s[t];
+          __syncthreads();
+        }
+        r = keep;
+      }
+      // the list is proven when nothing was screened out, or when its N-th score reaches L
+      if (screened_out && (r < N || sg_value(list[N - 1].key) < L)) {
+        if (tid == 0) p.ovf_users[atomicAdd(p.ovf_count, 1)] = u;
+        SG_COUNT(SGC_ZEROS, 1);
+        handed = true;
+        break;
+      }
+      __syncthreads();
+    }
+    if (handed) continue;
+    for (int t = tid; t < N; t += nt) {
+      p.out_idx[(int64_t)u * N + t] = t < r ? list[t].idx : -1;
+      p.out_val[(int64_t)u * N + t] = t < r ? sg_value(list[t].key) : 0.0;
+    }
+    if (tid == 0) p.out_len[u] = r;
+  }
+}
+
+static void predict_signed_topn(rpk_ctx* c, int64_t U, const int64_t* indptr, const int32_t* indices, int N, int mask_history,
+                                int32_t* out_idx, double* out_val, int32_t* out_len) {
+  cudaStream_t st = c->stream;
+  const int64_t I = c->m_I;
+  const bool tiny = c->flags & DBG_TINY_LIST;
+  const int cap = std::max(tiny ? 64 : 256, next_pow2(2 * N));
+  const int gbuf = std::max(2048, 2 * cap);  // also holds cap entries (16 B) while the survivors are compacted
+  const size_t fixed = sg_fixed_bytes(cap, gbuf);
+  // two CTAs per SM when the accumulators of the item ranges still fit, else one
+  auto ranges = [&](int ctas, int64_t& R) -> int {
+    const size_t per_cta = std::min<size_t>((size_t)c->smem_max, (size_t)c->smem_per_sm / ctas - 1024);
+    if (per_cta < fixed + 4096) return 0;
+    const int64_t Rmax = (int64_t)((per_cta - fixed) / sizeof(int)) & ~(int64_t)3;
+    const int P = (int)std::max<int64_t>(1, (I + Rmax - 1) / Rmax);
+    R = ((I + P - 1) / P + 3) & ~(int64_t)3;
+    return P;
+  };
+  int64_t R1 = 0, R2 = 0;
+  const int P1 = ranges(1, R1), P2 = ranges(2, R2);
+  RPK_REQUIRE(P1 > 0, "N too large for shared memory");
+  const bool two = P2 > 0 && (P2 <= 3 || P2 <= P1 + 1);
+  int P = two ? P2 : P1;
+  int64_t R = std::max<int64_t>(4, two ? R2 : R1);
+  const int p_min = (c->flags & DBG_MANY_PASS) ? 4 : ((c->flags & DBG_MULTI_PASS) ? 2 : 1);
+  if (P < p_min && I >= 4 * p_min) {
+    P = p_min;
+    R = ((I + P - 1) / P + 3) & ~(int64_t)3;
+  }
+  const size_t smem = fixed + (size_t)R * sizeof(int);
+  if (c->m_P != P || c->m_R != (int)R) {
+    int* seg = c->buf<int>("ms_seg", (size_t)I * (P + 1));
+    if (I > 0) {
+      k_signed_seg<<<ceil_div(I * (P + 1), 256), 256, 0, st>>>(c->get<int64_t>("m_ptr"), c->get<int>("ms_idx"), I, P, (int)R, seg);
+      RPK_LAUNCH_CHECK(c);
+    }
+    c->m_P = P;
+    c->m_R = (int)R;
+  }
+  SignedParams sp;
+  sp.indices = indices;
+  sp.m_ptr = c->get<int64_t>("m_ptr");
+  sp.seg = c->get<int>("ms_seg");
+  sp.ent = c->get<u64>("ms_ent");
+  sp.val = c->get<double>("ms_val");
+  sp.rowmax = c->get<unsigned>("ms_rowmax");
+  sp.U = (int)U;
+  sp.P = P;
+  sp.R = (int)R;
+  sp.N = N;
+  sp.mask = mask_history;
+  sp.cap = cap;
+  sp.gbuf = gbuf;
+  sp.e = c->m_exp;
+  sp.out_idx = out_idx;
+  sp.out_val = out_val;
+  sp.out_len = out_len;
+  sp.item_ok = item_filter_ptr(c);
+  sp.ovf_count = c->buf<int>("ps_ovf_count", 1);
+  sp.ovf_users = c->buf<int>("ps_ovf_users", (size_t)U);
+  RPK_CUDA(cudaMemsetAsync(sp.ovf_count, 0, sizeof(int), st));
+  const PredWork w = prepare_work(c, U, indptr);
+  sp.work_tab = w.tab;
+  sp.queue = w.queue + 1;
+  sp.prof = nullptr;
+#ifdef RPK_PHASE_PROF
+  sp.prof = c->buf<unsigned long long>("ps_prof", SGC_N);
+  RPK_CUDA(cudaMemsetAsync(sp.prof, 0, SGC_N * sizeof(unsigned long long), st));
+#endif
+  RPK_CUDA(cudaFuncSetAttribute(k_predict_signed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 0;
+  RPK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_predict_signed, SG_NT, smem));
+  RPK_REQUIRE(occ >= 1, "predict kernel does not fit on an SM");
+  const int grid = (int)std::min<int64_t>(U, (int64_t)c->sm_count * occ);
+  c->mark("predict signed: work table");
+  c->ev_record(4);
+  k_predict_signed<<<grid, SG_NT, smem, st>>>(sp);
+  RPK_LAUNCH_CHECK(c);
+  // the users handed over: float64 rows of X @ S with unit left values (normally few; the kernel then exits)
+  spgemm_rows_device(c, U, indptr, indices, nullptr, I, sp.m_ptr, c->get<int>("ms_idx"), sp.val, sp.ovf_users, sp.ovf_count, N,
+                     mask_history, sp.item_ok, 0, out_idx, out_val, out_len, nullptr, nullptr, nullptr, nullptr);
+  c->ev_record(5);
+  c->ev_valid[2] = true;
+  c->mark("predict signed: scoring");
+#ifdef RPK_PHASE_PROF
+  {
+    unsigned long long h[SGC_N];
+    RPK_CUDA(cudaMemcpyAsync(h, sp.prof, sizeof(h), cudaMemcpyDeviceToHost, st));
+    RPK_CUDA(cudaStreamSynchronize(st));
+    fprintf(stderr, "[predict signed paths] grid=%d P=%d R=%lld smem=%zu occ=%d users=%llu ranges=%llu survivors=%llu "
+            "overlap ranges=%llu overflow users=%llu zero users=%llu heavy users=%llu long segments=%llu\n",
+            grid, P, (long long)R, smem, occ, h[SGC_USERS], h[SGC_RANGES], h[SGC_SURVIVORS], h[SGC_OVERLAP], h[SGC_OVERFLOW],
+            h[SGC_ZEROS], h[SGC_HEAVY], h[SGC_LONG]);
+  }
+#endif
 }
 
 }  // namespace rpk

@@ -309,6 +309,11 @@ class Engine:
         self._check(self._lib.rpk_model_load_csr(self._h, int(I), int(indices.shape[0]), _addr(indptr, np.int64),
                                                  _addr(indices, np.int32), _addr(values, np.float64)))
 
+    def model_load_signed_csr(self, I, indptr, indices, values):
+        """A model of any sign, scored in float64: predictions are scipy's ``X @ S`` bit for bit."""
+        self._check(self._lib.rpk_model_load_signed_csr(self._h, int(I), int(indices.shape[0]), _addr(indptr, np.int64),
+                                                        _addr(indices, np.int32), _addr(values, np.float64)))
+
     # -- predict --------------------------------------------------------------------------
     def predict_topn(self, U, indptr, indices, N, mask_history=True, want_val=True, out=None):
         if out is None:

@@ -125,6 +125,7 @@ def real_top_k(X: csr_matrix, K: int, similarity: str = "cosine") -> csr_matrix:
 def pearson_top_k(X: csr_matrix, K: int) -> csr_matrix:
     """``get_top_K_values(compute_pearson_similarity(X), K)`` (nearest_neighbour.py:87-111, util.py:80-96) without the
     item x item matrix: ratings are centred per item over the positive entries, the cosine Gram of the centred matrix and
-    the per-row selection run on the GPU (rpk_fit_topk_real).  Similarities can be negative, so the result is a similarity
-    matrix for the TARSItemKNN family (scored by rpk_spgemm_*), not a model for the fixed-point scorer of ``ItemKNN.predict``."""
+    the per-row selection run on the GPU (rpk_fit_topk_real).  Similarities can be negative: set as the
+    ``similarity_matrix_`` of an ``ItemSimilarityMatrixAlgorithm`` the result is scored in float64 (scipy's ``X @ S``
+    bit for bit), and the TARSItemKNN family scores it through rpk_spgemm_*."""
     return real_top_k(X, K, "pearson")
