@@ -292,6 +292,14 @@ RPK_EXPORT int rpk_gram_dense_u16(rpk_ctx* ctx, int64_t I, int64_t Kd, const uin
  *                           I - P @ diag(1 / diag(P)) followed by B @ diag(w), w_j = 1 / n_j^alpha (NULL: no scaling).
  *                           P and out_B are DEVICE matrices [I x I] float64 and may be the same buffer.  The inverse
  *                           itself is a library call on the caller's side (cuSOLVER potrf + potri).
+ *   rpk_ease_prune          EASE._prune (ease.py:97-109): the min(keep, nnz(B)) entries of the DEVICE matrix B [I x I]
+ *                           with the largest |B_ij| as a canonical CSR (ascending columns, values bit for bit).  The
+ *                           entries are the values != 0.0; every NaN ranks above +inf; +x and -x tie; ties at the cut
+ *                           go to the entries first in row-major order.  out_indptr int64[I + 1], out_indices int32
+ *                           and out_values float64 sized keep, out_nnz int64[1] receives the count; outputs may be host
+ *                           or device memory.  keep = 0 keeps nothing (the reference's "K = 0 keeps all" is the
+ *                           caller's: pass keep = I * I).  Workspace: 16 bytes per entry of the top-digit bin that
+ *                           holds the cut.
  *   rpk_predict_dense_topn  scores = X @ B for a dense float64 model B (device, [I x I] row-major): every score is
  *   rpk_predict_dense_full  the sum over the user's history in ascending item order, one float64 addition per term
  *                           (scipy's csr @ dense order).  _topn keeps the N best non-zero scores per user (score
@@ -301,6 +309,8 @@ RPK_EXPORT int rpk_gram_dense_u16(rpk_ctx* ctx, int64_t I, int64_t Kd, const uin
 RPK_EXPORT int rpk_gram_dense_f64(rpk_ctx* ctx, int64_t U, int64_t I, int64_t nnz, const int64_t* indptr,
                        const int32_t* indices, double* out_G);
 RPK_EXPORT int rpk_ease_from_inverse(rpk_ctx* ctx, int64_t I, const double* P, const double* w, double* out_B);
+RPK_EXPORT int rpk_ease_prune(rpk_ctx* ctx, int64_t I, const double* B, int64_t keep, int64_t* out_indptr,
+                   int32_t* out_indices, double* out_values, int64_t* out_nnz);
 RPK_EXPORT int rpk_predict_dense_topn(rpk_ctx* ctx, int64_t U, int64_t nnz, const int64_t* indptr, const int32_t* indices,
                            int64_t I, const double* B, int N, int mask_history,
                            int32_t* out_idx, double* out_val, int32_t* out_len);

@@ -46,6 +46,7 @@ _SIGNATURES = {
     "rpk_coverage_topn": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int64, _i32p, _i32p, _i64p, _i64p, _vp]),
     "rpk_gram_dense_f64": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, _i64p, _i32p, _f64p]),
     "rpk_ease_from_inverse": (C.c_int, [C.c_void_p, C.c_int64, _f64p, _f64p, _f64p]),
+    "rpk_ease_prune": (C.c_int, [C.c_void_p, C.c_int64, _f64p, C.c_int64, _i64p, _i32p, _f64p, _i64p]),
     "rpk_predict_dense_topn": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _i64p, _i32p, C.c_int64, _f64p, C.c_int, C.c_int,
                                          _i32p, _f64p, _i32p]),
     "rpk_predict_dense_full": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, _i64p, _i32p, C.c_int64, _f64p, C.c_int, _f64p]),

@@ -142,15 +142,7 @@ class GpuSimilarityMixin:
             if dev is not None and dev["device"] == engine.device:
                 engine.model_load_topk(dev["I"], dev["idx"].shape[1], dev["idx"], dev["val"], dev["len"])
             else:
-                S = self.similarity_matrix_
-                if not isinstance(S, csr_matrix):
-                    S = csr_matrix(S)
-                if not S.has_canonical_format:
-                    S = S.copy()
-                    S.sum_duplicates()
-                if S.nnz and not np.all(S.data):
-                    S = S.copy()
-                    S.eliminate_zeros()
+                S = canonical_csr(self.similarity_matrix_)
                 # a model with a negative value is scored in float64 (X @ S bit for bit), any other in fixed point
                 load = engine.model_load_signed_csr if S.nnz and np.any(S.data < 0) else engine.model_load_csr
                 load(S.shape[0], np.ascontiguousarray(S.indptr, dtype=np.int64), np.ascontiguousarray(S.indices, dtype=np.int32),
@@ -171,26 +163,8 @@ class GpuSimilarityMixin:
         I = self._n_items()
         if X.shape[1] != I:
             raise ValueError("matmul: dimension mismatch with signature (n?,k),(k,m?)->(n?,m?)")
-        U = X.shape[0]
-        from .postprocessing import combined_mask
-
-        with engine.model_lock:  # load + score as one step: the engine holds one model at a time
-            self._ensure_device_model(engine)
-            engine.predict_item_filter(combined_mask(self._postfilters, I))
-            if self.predict_topK is None:
-                X, indptr, indices = binary_structure(X)
-                o_ptr, o_idx, o_val = engine.predict_csr(U, indptr, indices, mask_history=bool(self.remove_history))
-                return csr_matrix((o_val, o_idx, o_ptr), shape=(U, I))
-            N = int(self.predict_topK)
-            X, _, _, ptr_d, idx_d = device_structure(X, engine.device)
-            top = engine.predict_topn(U, ptr_d, idx_d, N, mask_history=bool(self.remove_history))
-            engine.sync()
-        idx, val, ln = to_host(top["idx"], top["val"], top["len"])
-        M = lists_to_csr(idx, val, ln, I, attach=True)
-        # the metrics read the lists where they are, as long as the matrix still is what predict returned
-        M._rpk_topn_dev = (top["idx"], top["len"], engine.device)
-        M._rpk_topn_sig = matrix_signature(M)
-        return M
+        return predict_with_model(engine, self._ensure_device_model, X, I, self.predict_topK, self.remove_history,
+                                  self._postfilters)
 
     # -- the reference's checks, without Python sets over nonzero() -------------------------------------
     def _transform_fit_input(self, X):
@@ -235,6 +209,44 @@ class ItemSimilarityMatrixAlgorithm(GpuSimilarityMixin, _SimilarityBase):
 
 class TopKItemSimilarityMatrixAlgorithm(GpuSimilarityMixin, _TopKBase):
     """recpack/algorithms/base.py:282-304."""
+
+
+def canonical_csr(S) -> csr_matrix:
+    """S as a CSR with sorted, unique column indices and no stored zeros (copied only when it is not one already)."""
+    if not isinstance(S, csr_matrix):
+        S = csr_matrix(S)
+    if not S.has_canonical_format:
+        S = S.copy()
+        S.sum_duplicates()
+    if S.nnz and not np.all(S.data):
+        S = S.copy()
+        S.eliminate_zeros()
+    return S
+
+
+def predict_with_model(engine, ensure_model, X: csr_matrix, I: int, predict_topK, remove_history, postfilters=()) -> csr_matrix:
+    """Scores X with the model that ``ensure_model(engine)`` makes resident: the full CSR of the scores when
+    ``predict_topK`` is None, else the top-N lists as a CSR that carries them (host and device) for the metrics."""
+    from .postprocessing import combined_mask
+
+    U = X.shape[0]
+    with engine.model_lock:  # load + score as one step: the engine holds one model at a time
+        ensure_model(engine)
+        engine.predict_item_filter(combined_mask(postfilters, I))
+        if predict_topK is None:
+            X, indptr, indices = binary_structure(X)
+            o_ptr, o_idx, o_val = engine.predict_csr(U, indptr, indices, mask_history=bool(remove_history))
+            return csr_matrix((o_val, o_idx, o_ptr), shape=(U, I))
+        N = int(predict_topK)
+        X, _, _, ptr_d, idx_d = device_structure(X, engine.device)
+        top = engine.predict_topn(U, ptr_d, idx_d, N, mask_history=bool(remove_history))
+        engine.sync()
+    idx, val, ln = to_host(top["idx"], top["val"], top["len"])
+    M = lists_to_csr(idx, val, ln, I, attach=True)
+    # the metrics read the lists where they are, as long as the matrix still is what predict returned
+    M._rpk_topn_dev = (top["idx"], top["len"], engine.device)
+    M._rpk_topn_sig = matrix_signature(M)
+    return M
 
 
 def matrix_signature(M: csr_matrix):

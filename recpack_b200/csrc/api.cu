@@ -267,6 +267,13 @@ int rpk_ease_from_inverse(rpk_ctx* ctx, int64_t I, const double* P, const double
   RPK_API_END(ctx)
 }
 
+int rpk_ease_prune(rpk_ctx* ctx, int64_t I, const double* B, int64_t keep, int64_t* out_indptr, int32_t* out_indices,
+                   double* out_values, int64_t* out_nnz) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_ease_prune(ctx, I, B, keep, out_indptr, out_indices, out_values, out_nnz);
+  RPK_API_END(ctx)
+}
+
 int rpk_predict_dense_topn(rpk_ctx* ctx, int64_t U, int64_t nnz, const int64_t* indptr, const int32_t* indices, int64_t I,
                            const double* B, int N, int mask_history, int32_t* out_idx, double* out_val, int32_t* out_len) {
   RPK_API_BEGIN(ctx)

@@ -5,12 +5,17 @@
 //   P = inv(XTX + l2 * I)                              ease.py:80    -> the caller (cuSOLVER potrf / potri through torch)
 //   B = I - P @ diag(1 / diag(P)); diag(B) = 0         ease.py:83-84 -> rpk_ease_from_inverse: B_ij = -P_ij / P_jj, B_ii = 0
 //   B = B @ diag(1 / n_j^alpha)                        ease.py:86-88 -> the same kernel, column scale w_j
+//   prune to the K largest |B_ij|                      ease.py:97-109 -> rpk_ease_prune: exact top-K by magnitude, canonical CSR
 //   scores = X @ B                                     base.py:248   -> rpk_predict_dense_*: sum over the history in
 //                                                                       ascending item order, float64, one add per term --
 //                                                                       scipy's csr_matvecs order, so equal inputs give
 //                                                                       bit-identical scores
+#include <algorithm>
+#include <vector>
+
 #include "common.cuh"
 #include "internal.h"
+#include "prims.cuh"
 #include "select.cuh"
 
 namespace rpk {
@@ -92,6 +97,293 @@ void run_ease_from_inverse(rpk_ctx* c, int64_t I, const double* P_u, const doubl
   k_ease_finish<<<ceil_div(I * I, 256), 256, 0, c->stream>>>(P_u, dg, w, I, B_u);
   RPK_LAUNCH_CHECK(c);
   finish_call(c);
+}
+
+// ------------------------------------------------------------------------------------------
+// Pruning (EASE._prune, ease.py:97-109): the K largest-magnitude entries of a dense device B as a canonical CSR.
+// Key of an entry: the bit pattern of |v| (sign cleared), every NaN mapped to one key above +inf; key 0 (+-0.0) is not
+// an entry.  The K-th largest key T is found by a radix select: a histogram of the top 15 key bits over B, the
+// entries of the boundary bin collected as candidates, four more digits over the candidates.  Kept: key > T, and the
+// first K - #(key > T) entries with key == T in row-major order.  B is read three times: histogram, collect, fill.
+// ------------------------------------------------------------------------------------------
+static constexpr u64 PRUNE_NAN_KEY = 0x7ff0000000000001ull;  // +inf is 0x7ff0000000000000
+static constexpr int PRUNE_BINS = 1 << 15;                  // top digit: key bits 62..48 (bit 63 is always 0)
+static constexpr int PRUNE_TOP_SHIFT = 48;
+
+__device__ __forceinline__ u64 prune_key(double v) {
+  const u64 k = (u64)__double_as_longlong(v) & 0x7fffffffffffffffull;
+  return k < PRUNE_NAN_KEY ? k : PRUNE_NAN_KEY;
+}
+
+__device__ __forceinline__ void prune_hist_flush(const unsigned* sh, int nbins, u64* __restrict__ hist) {
+  __syncthreads();
+  for (int b = threadIdx.x; b < nbins; b += blockDim.x)
+    if (sh[b]) atomicAdd(hist + b, (u64)sh[b]);
+}
+
+// hist[key >> 48] over the non-zero entries of B [n = I*I] (one shared-memory histogram per CTA).
+__global__ void __launch_bounds__(1024) k_prune_hist(const double* __restrict__ B, int64_t n, u64* __restrict__ hist) {
+  extern __shared__ unsigned sh_hist[];
+  for (int b = threadIdx.x; b < PRUNE_BINS; b += blockDim.x) sh_hist[b] = 0;
+  __syncthreads();
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+#pragma unroll 4
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
+    const u64 k = prune_key(__ldg(B + t));
+    if (k) atomicAdd(sh_hist + (k >> PRUNE_TOP_SHIFT), 1u);
+  }
+  prune_hist_flush(sh_hist, PRUNE_BINS, hist);
+}
+
+// One CTA per row: row_gt[i] = #(key >> 48 > bin); the entries of the bin are appended to the candidates
+// (key, flat position), in no particular order.
+__global__ void __launch_bounds__(256) k_prune_collect(const double* __restrict__ B, int64_t I, u64 bin, u64* __restrict__ cand_key,
+                                                       int64_t* __restrict__ cand_pos, unsigned long long* __restrict__ n_cand,
+                                                       int* __restrict__ row_gt) {
+  __shared__ int wsum[8];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int64_t i = blockIdx.x; i < I; i += gridDim.x) {
+    const double* row = B + i * I;
+    int gt = 0;
+    for (int64_t j0 = 0; j0 < I; j0 += blockDim.x) {
+      const int64_t j = j0 + threadIdx.x;
+      const u64 k = j < I ? prune_key(__ldg(row + j)) : 0ull;
+      gt += (k >> PRUNE_TOP_SHIFT) > bin;
+      const bool in_bin = k != 0ull && (k >> PRUNE_TOP_SHIFT) == bin;
+      const unsigned m = __ballot_sync(0xffffffffu, in_bin);
+      if (m) {
+        unsigned long long base = 0;
+        if (lane == 0) base = atomicAdd(n_cand, (unsigned long long)__popc(m));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (in_bin) {
+          const unsigned long long at = base + __popc(m & ((1u << lane) - 1u));
+          cand_key[at] = k;
+          cand_pos[at] = i * I + j;
+        }
+      }
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) gt += __shfl_xor_sync(0xffffffffu, gt, o);
+    if (lane == 0) wsum[warp] = gt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      int s = 0;
+      for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += wsum[w];
+      row_gt[i] = s;
+    }
+    __syncthreads();
+  }
+}
+
+// hist[(key >> shift) & (2^width - 1)] over the candidates whose key agrees with `prefix` above bit shift + width.
+__global__ void __launch_bounds__(1024) k_prune_cand_hist(const u64* __restrict__ cand_key, int64_t n, u64 prefix, int shift,
+                                                          int width, u64* __restrict__ hist) {
+  extern __shared__ unsigned sh_hist[];
+  const int nbins = 1 << width;
+  for (int b = threadIdx.x; b < nbins; b += blockDim.x) sh_hist[b] = 0;
+  __syncthreads();
+  const int hi = shift + width;
+  const u64 want = prefix >> hi;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
+    const u64 k = cand_key[t];
+    if ((k >> hi) == want) atomicAdd(sh_hist + (int)((k >> shift) & (u64)(nbins - 1)), 1u);
+  }
+  prune_hist_flush(sh_hist, nbins, hist);
+}
+
+// Candidates above the threshold T add to their row's count, those equal to T to the row's tie count.
+__global__ void k_prune_row_counts(const u64* __restrict__ cand_key, const int64_t* __restrict__ cand_pos, int64_t n, int64_t I,
+                                   u64 T, int* __restrict__ row_gt, int* __restrict__ row_eq) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
+    const u64 k = cand_key[t];
+    if (k > T) atomicAdd(row_gt + cand_pos[t] / I, 1);
+    else if (k == T) atomicAdd(row_eq + cand_pos[t] / I, 1);
+  }
+}
+
+// Row i takes the leftmost of the ties that the rows before it left over: min(row_eq, max(0, ties - eq_before)).
+__global__ void k_prune_take(const int* __restrict__ row_gt, const int* __restrict__ row_eq, const int64_t* __restrict__ eq_before,
+                             int64_t I, int64_t ties, int* __restrict__ row_take, int* __restrict__ row_keep) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= I) return;
+  const int64_t left = ties - eq_before[i];
+  const int take = left <= 0 ? 0 : (int)min(left, (int64_t)row_eq[i]);
+  row_take[i] = take;
+  row_keep[i] = row_gt[i] + take;
+}
+
+// One CTA per row: the kept entries in ascending column order at out_indptr[i] (ordered block-wide compaction).
+__global__ void __launch_bounds__(256) k_prune_fill(const double* __restrict__ B, int64_t I, u64 T, const int* __restrict__ row_take,
+                                                    const int64_t* __restrict__ indptr, int32_t* __restrict__ out_idx,
+                                                    double* __restrict__ out_val) {
+  __shared__ int wt[8], wk[8];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const unsigned below = (1u << lane) - 1u;
+  for (int64_t i = blockIdx.x; i < I; i += gridDim.x) {
+    const double* row = B + i * I;
+    const int take = row_take[i];
+    int64_t at = indptr[i];
+    int ties_seen = 0;
+    for (int64_t j0 = 0; j0 < I; j0 += blockDim.x) {
+      const int64_t j = j0 + threadIdx.x;
+      const double v = j < I ? __ldg(row + j) : 0.0;
+      const u64 k = prune_key(v);
+      const bool tie = k == T;
+      const unsigned mt = __ballot_sync(0xffffffffu, tie);
+      if (lane == 0) wt[warp] = __popc(mt);
+      __syncthreads();
+      int tie_rank = ties_seen + __popc(mt & below), tie_tile = 0;
+      for (int w = 0; w < nw; ++w) {
+        tie_rank += w < warp ? wt[w] : 0;
+        tie_tile += wt[w];
+      }
+      const bool keep = k > T || (tie && tie_rank < take);
+      const unsigned mk = __ballot_sync(0xffffffffu, keep);
+      if (lane == 0) wk[warp] = __popc(mk);
+      __syncthreads();
+      int pos = __popc(mk & below), kept_tile = 0;
+      for (int w = 0; w < nw; ++w) {
+        pos += w < warp ? wk[w] : 0;
+        kept_tile += wk[w];
+      }
+      if (keep) {
+        out_idx[at + pos] = (int32_t)j;
+        out_val[at + pos] = v;
+      }
+      at += kept_tile;
+      ties_seen += tie_tile;
+      __syncthreads();
+    }
+  }
+}
+
+// Stream-ordered workspace sized per call (it can be as large as B), returned to the pool on every exit path.
+template <class T>
+struct StreamBuf {
+  T* p = nullptr;
+  cudaStream_t st;
+  StreamBuf(cudaStream_t s, size_t count) : st(s) { RPK_CUDA(cudaMallocAsync((void**)&p, sizeof(T) * count, st)); }
+  void release() {
+    if (p) RPK_CUDA(cudaFreeAsync(p, st));
+    p = nullptr;
+  }
+  ~StreamBuf() {
+    if (p) cudaFreeAsync(p, st);  // an exception is already on its way: nothing to report here
+  }
+  StreamBuf(const StreamBuf&) = delete;
+  StreamBuf& operator=(const StreamBuf&) = delete;
+};
+
+// Index of the bin that holds the need-th largest entry (counting from the top); need becomes its rank inside the bin.
+static int prune_pick(const std::vector<u64>& h, u64& need) {
+  for (int b = (int)h.size() - 1; b >= 0; --b) {
+    if (h[b] >= need) return b;
+    need -= h[b];
+  }
+  throw Error("internal: prune selection ran out of entries");
+}
+
+void run_ease_prune(rpk_ctx* c, int64_t I, const double* B, int64_t keep, int64_t* out_indptr_u, int32_t* out_indices_u,
+                    double* out_values_u, int64_t* out_nnz_u) {
+  RPK_REQUIRE(I >= 1 && keep >= 0 && B && out_indptr_u && out_nnz_u, "bad arguments");
+  RPK_REQUIRE(I < ((int64_t)1 << 31), "item count must be below 2^31");
+  RPK_REQUIRE(is_device_ptr(B), "rpk_ease_prune works on a device matrix B");
+  cudaStream_t st = c->stream;
+  const int64_t n = I * I;
+  u64* hist = c->buf<u64>("prune_hist", PRUNE_BINS);
+  std::vector<u64> h(PRUNE_BINS);
+  const size_t hist_smem = sizeof(unsigned) * PRUNE_BINS;
+  RPK_CUDA(cudaFuncSetAttribute(k_prune_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_smem));
+  RPK_CUDA(cudaFuncSetAttribute(k_prune_cand_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_smem));
+  auto read_hist = [&](int nbins) {
+    h.assign(nbins, 0);
+    RPK_CUDA(cudaMemcpyAsync(h.data(), hist, sizeof(u64) * nbins, cudaMemcpyDeviceToHost, st));
+    RPK_CUDA(cudaStreamSynchronize(st));
+  };
+  c->mark("prune_hist");
+  RPK_CUDA(cudaMemsetAsync(hist, 0, sizeof(u64) * PRUNE_BINS, st));
+  k_prune_hist<<<c->sm_count, 1024, hist_smem, st>>>(B, n, hist);
+  RPK_LAUNCH_CHECK(c);
+  read_hist(PRUNE_BINS);
+  u64 nnz = 0;
+  for (u64 x : h) nnz += x;
+  const int64_t K = std::min<int64_t>(keep, (int64_t)nnz);
+
+  Out<int64_t> o_ptr, o_nnz;
+  Out<int32_t> o_idx;
+  Out<double> o_val;
+  o_ptr.init(c, out_indptr_u, (size_t)I + 1, "prune_out_ptr");
+  o_nnz.init(c, out_nnz_u, 1, "prune_out_nnz");
+  if (K > 0) {
+    RPK_REQUIRE(out_indices_u && out_values_u, "out_indices / out_values must not be null");
+    o_idx.init(c, out_indices_u, (size_t)K, "prune_out_idx");
+    o_val.init(c, out_values_u, (size_t)K, "prune_out_val");
+  }
+  RPK_CUDA(cudaMemcpyAsync(o_nnz.dev, &K, sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  if (K == 0) {
+    RPK_CUDA(cudaMemsetAsync(o_ptr.dev, 0, sizeof(int64_t) * ((size_t)I + 1), st));
+  } else {
+    // the boundary bin of the top digit: its entries become the candidates
+    u64 need = (u64)K;
+    const int b1 = prune_pick(h, need);
+    const int64_t n_cand = (int64_t)h[b1];
+    StreamBuf<u64> cand_key_buf(st, (size_t)n_cand);
+    StreamBuf<int64_t> cand_pos_buf(st, (size_t)n_cand);
+    u64* cand_key = cand_key_buf.p;
+    int64_t* cand_pos = cand_pos_buf.p;
+    unsigned long long* n_cand_dev = c->buf<unsigned long long>("prune_ncand", 1);
+    int* row_gt = c->buf<int>("prune_row_gt", (size_t)I);
+    int* row_eq = c->buf<int>("prune_row_eq", (size_t)I);
+    int* row_take = c->buf<int>("prune_row_take", (size_t)I);
+    int* row_keep = c->buf<int>("prune_row_keep", (size_t)I);
+    int64_t* eq_before = c->buf<int64_t>("prune_eq_before", (size_t)I + 1);
+    RPK_CUDA(cudaMemsetAsync(n_cand_dev, 0, sizeof(unsigned long long), st));
+    RPK_CUDA(cudaMemsetAsync(row_eq, 0, sizeof(int) * (size_t)I, st));
+    const int row_grid = (int)std::min<int64_t>(I, (int64_t)c->sm_count * 8);
+    c->mark("prune_collect");
+    k_prune_collect<<<row_grid, 256, 0, st>>>(B, I, (u64)b1, cand_key, cand_pos, n_cand_dev, row_gt);
+    RPK_LAUNCH_CHECK(c);
+    // the remaining 48 key bits, digit by digit over the candidates
+    c->mark("prune_select");
+    u64 T = (u64)b1 << PRUNE_TOP_SHIFT;
+    const int digits[4][2] = {{33, 15}, {18, 15}, {3, 15}, {0, 3}};
+    const int cgrid = (int)std::min<int64_t>(ceil_div(n_cand, 1024), c->sm_count);
+    for (auto& dg : digits) {
+      const int nbins = 1 << dg[1];
+      RPK_CUDA(cudaMemsetAsync(hist, 0, sizeof(u64) * nbins, st));
+      k_prune_cand_hist<<<cgrid, 1024, sizeof(unsigned) * nbins, st>>>(cand_key, n_cand, T, dg[0], dg[1], hist);
+      RPK_LAUNCH_CHECK(c);
+      read_hist(nbins);
+      T |= (u64)prune_pick(h, need) << dg[0];
+    }
+    // T is the K-th largest key; `need` of its ties are kept
+    c->mark("prune_counts");
+    k_prune_row_counts<<<(int)std::min<int64_t>(ceil_div(n_cand, 256), (int64_t)c->sm_count * 16), 256, 0, st>>>(
+        cand_key, cand_pos, n_cand, I, T, row_gt, row_eq);
+    RPK_LAUNCH_CHECK(c);
+    cand_key_buf.release();
+    cand_pos_buf.release();
+    scan_i32_i64(c, row_eq, eq_before, I);
+    k_prune_take<<<ceil_div(I, 256), 256, 0, st>>>(row_gt, row_eq, eq_before, I, (int64_t)need, row_take, row_keep);
+    RPK_LAUNCH_CHECK(c);
+    scan_i32_i64(c, row_keep, o_ptr.dev, I);
+    int64_t total = -1;
+    RPK_CUDA(cudaMemcpyAsync(&total, o_ptr.dev + I, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    RPK_CUDA(cudaStreamSynchronize(st));
+    RPK_REQUIRE(total == K, "internal: pruned row counts do not add up to K");
+    c->mark("prune_fill");
+    k_prune_fill<<<row_grid, 256, 0, st>>>(B, I, T, row_take, o_ptr.dev, o_idx.dev, o_val.dev);
+    RPK_LAUNCH_CHECK(c);
+    c->mark("prune_end");
+  }
+  o_ptr.finish(c);
+  o_nnz.finish(c);
+  o_idx.finish(c);
+  o_val.finish(c);
+  RPK_CUDA(cudaStreamSynchronize(st));  // the host value behind the out_nnz copy lives on this frame
+  c->host_out_pending = false;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -59,6 +59,8 @@ void run_split_fraction(rpk_ctx* c, int64_t n_users, const int64_t* uids, const 
                         int64_t n_rows, double in_frac, uint64_t seed, uint8_t* out_in_mask);
 void run_gram_dense_f64(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64_t* indptr, const int32_t* indices, double* out_G);
 void run_ease_from_inverse(rpk_ctx* c, int64_t I, const double* P, const double* w, double* B);
+void run_ease_prune(rpk_ctx* c, int64_t I, const double* B, int64_t keep, int64_t* out_indptr, int32_t* out_indices,
+                    double* out_values, int64_t* out_nnz);
 void run_predict_dense(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr, const int32_t* indices, int64_t I, const double* B,
                        int N, int mask_history, int32_t* out_idx, double* out_val, int32_t* out_len, double* out_full);
 void run_gram_dense_u16(rpk_ctx* c, int64_t I, int64_t Kd, const unsigned char* A, unsigned short* G);

@@ -10,6 +10,15 @@ scaling from rpk_ease_from_inverse.  The model stays on the device as a dense fl
 history in ascending item order -- the order of scipy's ``csr @ dense`` -- so equal models give bit-identical scores;
 ``predict_topK`` / ``remove_history`` as for ItemKNN.
 
+``density`` (``_prune``, ease.py:97-109): after the closed form the model is pruned on the device to its
+``K = min(int(density * I*I), nnz)`` largest-magnitude entries (rpk_ease_prune; ``K = 0`` keeps every entry, as the
+reference's ``argpartition(..., -0)[0:-0]`` does) and the dense model is dropped.  Ties at the cut go to the entries
+first in row-major order.  The pruned model is scored like every signed similarity model, in float64 and bit for bit
+scipy's ``X @ S`` (rpk_model_load_signed_csr); its values must be finite there.  The loaded model is keyed by
+(estimator, version) like ``GpuSimilarityMixin``'s: after editing ``similarity_matrix_`` in place, call
+``invalidate_device_model()``.  A negative ``density`` raises ``ValueError`` (the reference computes a negative K and
+zeroes the |K| smallest entries instead, or fails in ``argpartition`` when |K| >= nnz).
+
 The reference inverts with LAPACK's LU (``np.linalg.inv``); Cholesky on the GPU agrees with it to rounding
 (~1e-12 relative on B), not bit for bit -- the tolerance of the tests."""
 from __future__ import annotations
@@ -21,7 +30,7 @@ from scipy.sparse import csr_matrix
 from sklearn.utils.validation import check_is_fitted
 
 from . import _ref
-from .base import lists_to_csr, matrix_signature
+from .base import canonical_csr, lists_to_csr, matrix_signature, predict_with_model
 from .engine import get_engine
 from .matrix import binary_structure, device_structure, to_csr_matrix, to_host
 
@@ -62,8 +71,8 @@ class EASE(_EaseBase):
     def _fit(self, X: csr_matrix) -> None:
         import torch
 
-        if self.density:
-            raise NotImplementedError("EASE(density=...) (pruning of B, ease.py:97-109) is not implemented on the B200 path")
+        if self.density and self.density < 0:
+            raise ValueError("density must be non-negative")
         engine = get_engine()
         X, indptr, indices, ptr_d, idx_d = device_structure(X, engine.device)
         U, I = X.shape
@@ -83,8 +92,16 @@ class EASE(_EaseBase):
         B = engine.ease_from_inverse(P, w)  # in place
         engine.sync()
         d = self.__dict__
-        d["_B_dev"] = B
         d["_similarity_host"] = None
+        d["_model_version"] = d.get("_model_version", 0) + 1
+        if self.density:
+            S = engine.ease_prune(B, prune_keep(self.density, I))
+            del B, P
+            d["_B_dev"] = None
+            d["_S_dev"] = S
+        else:
+            d["_B_dev"] = B
+            d["_S_dev"] = None
 
     # -- similarity_matrix_: the dense model as the reference stores it, built on demand -------------------
     @property
@@ -92,10 +109,14 @@ class EASE(_EaseBase):
         d = self.__dict__
         S = d.get("_similarity_host")
         if S is None:
-            B = d.get("_B_dev")
-            if B is None:
+            B, S_dev = d.get("_B_dev"), d.get("_S_dev")
+            if B is not None:
+                S = csr_matrix(B.cpu().numpy())
+            elif S_dev is not None:
+                I = int(S_dev[0].shape[0]) - 1
+                S = csr_matrix(tuple(t.cpu().numpy() for t in S_dev[::-1]), shape=(I, I))
+            else:
                 raise AttributeError(f"{type(self).__name__} object has no attribute 'similarity_matrix_'")
-            S = csr_matrix(B.cpu().numpy())
             d["_similarity_host"] = S
         return S
 
@@ -104,25 +125,33 @@ class EASE(_EaseBase):
         d = self.__dict__
         d["_similarity_host"] = S
         d["_B_dev"] = None
+        d["_S_dev"] = None
+        d["_model_version"] = d.get("_model_version", 0) + 1
 
     def __sklearn_is_fitted__(self):
         d = self.__dict__
-        return d.get("_similarity_host") is not None or d.get("_B_dev") is not None
+        return any(d.get(k) is not None for k in ("_similarity_host", "_B_dev", "_S_dev"))
 
     def __getstate__(self):
-        if self.__dict__.get("_B_dev") is not None:
-            self.similarity_matrix_
+        d = self.__dict__
+        if d.get("_B_dev") is not None or d.get("_S_dev") is not None:
+            self.similarity_matrix_  # pickles carry the host matrix, never device memory
         state = dict(super().__getstate__())
         state["_B_dev"] = None
+        state["_S_dev"] = None
         return state
 
     def _check_fit_complete(self):
         import warnings
 
+        import torch
+
         check_is_fitted(self)
-        B = self.__dict__.get("_B_dev")
+        B, S_dev = self.__dict__.get("_B_dev"), self.__dict__.get("_S_dev")
         if B is not None:
             missing = int((B != 0).sum(dim=1).eq(0).sum().item())
+        elif S_dev is not None:
+            missing = int(torch.diff(S_dev[0]).eq(0).sum().item())
         else:
             S = csr_matrix(self.similarity_matrix_)
             missing = int(S.shape[0] - np.count_nonzero(np.asarray((S != 0).sum(axis=1)).ravel()))
@@ -152,8 +181,50 @@ class EASE(_EaseBase):
             d["_B_dev"] = B
         return B
 
+    def _ensure_sparse_model(self, engine):
+        """Loads the pruned model as a signed model (float64 scoring) unless it is the engine's resident one; the key
+        (estimator, version) is that of ``GpuSimilarityMixin._ensure_device_model``."""
+        d = self.__dict__
+        key = (id(self), d.get("_model_version", 0))
+        with engine.model_lock:
+            if engine._model_key == key:
+                return
+            engine._model_key = None  # a failed load leaves no model behind
+            S_dev = d.get("_S_dev")
+            if S_dev is not None and S_dev[0].device.index == engine.device:
+                ptr, idx, val = S_dev
+            else:
+                S = canonical_csr(self.similarity_matrix_)
+                ptr, idx, val = (np.ascontiguousarray(S.indptr, dtype=np.int64), np.ascontiguousarray(S.indices, dtype=np.int32),
+                                 np.ascontiguousarray(S.data, dtype=np.float64))
+            engine.model_load_signed_csr(int(ptr.shape[0]) - 1, ptr, idx, val)
+            engine._model_key = key
+            engine._model_owner = self
+
+    def invalidate_device_model(self):
+        """Call after editing ``similarity_matrix_`` in place: the next predict takes the model from the host matrix
+        again instead of the device copy that the fit (or an earlier predict) left behind."""
+        d = self.__dict__
+        if d.get("_similarity_host") is not None:
+            d["_S_dev"] = None
+            d["_B_dev"] = None
+        d["_model_version"] = d.get("_model_version", 0) + 1
+
+    def _n_items(self):
+        d = self.__dict__
+        if d.get("_S_dev") is not None:
+            return int(d["_S_dev"][0].shape[0]) - 1
+        if d.get("_B_dev") is not None:
+            return int(d["_B_dev"].shape[0])
+        return self.similarity_matrix_.shape[0]
+
     def _predict(self, X: csr_matrix) -> csr_matrix:
         engine = get_engine()
+        if self.density:  # a pruned model: float64 sparse scoring, the route of every signed similarity model
+            I = self._n_items()
+            if X.shape[1] != I:
+                raise ValueError("matmul: dimension mismatch with signature (n?,k),(k,m?)->(n?,m?)")
+            return predict_with_model(engine, self._ensure_sparse_model, X, I, self.predict_topK, self.remove_history)
         B = self._device_model(engine)
         I = int(B.shape[0])
         if X.shape[1] != I:
@@ -172,3 +243,11 @@ class EASE(_EaseBase):
         M._rpk_topn_dev = (top["idx"], top["len"], engine.device)
         M._rpk_topn_sig = matrix_signature(M)
         return M
+
+
+def prune_keep(density, I: int) -> int:
+    """How many entries ``_prune`` keeps of an I x I model, before the cap at its nnz: ``int(density * (I*I))`` as one
+    float64 product of the exact integer I*I (ease.py:105); 0 there means every entry stays (``argpartition(a, -0)[0:-0]``
+    is empty), so I*I is returned instead."""
+    K = int(float(density) * (int(I) * int(I)))
+    return K if K > 0 else int(I) * int(I)

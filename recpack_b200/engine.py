@@ -234,6 +234,25 @@ class Engine:
                                                     _addr(out, np.float64)))
         return out
 
+    def ease_prune(self, B, keep):
+        """rpk_ease_prune: the min(keep, nnz(B)) largest-magnitude entries of the device matrix B [I, I] as a canonical
+        CSR of device tensors (indptr int64, indices int32, values float64), trimmed to the kept count."""
+        import torch
+
+        I = int(B.shape[0])
+        keep = int(keep)
+        cap = max(1, min(keep, I * I))
+        indptr = torch.empty(I + 1, dtype=torch.int64, device=B.device)
+        indices = torch.empty(cap, dtype=torch.int32, device=B.device)
+        values = torch.empty(cap, dtype=torch.float64, device=B.device)
+        nnz = np.zeros(1, dtype=np.int64)
+        self._check(self._lib.rpk_ease_prune(self._h, I, _addr(B, np.float64), keep, _addr(indptr, np.int64),
+                                             _addr(indices, np.int32), _addr(values, np.float64), _addr(nnz)))
+        n = int(nnz[0])
+        if n < cap:  # let the unused part of the output go
+            indices, values = indices[:n].clone(), values[:n].clone()
+        return indptr, indices, values
+
     def predict_dense_topn(self, U, indptr, indices, B, N, mask_history=True, want_val=True):
         out = {
             "idx": _empty_like_kind(indices, (U, N), np.int32),
