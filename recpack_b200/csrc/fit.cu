@@ -718,7 +718,7 @@ struct FitParams {
   const int* csc_users;
   const unsigned* pref;   // per-item exclusive prefix of history lengths (CSC order)
   const u64* work;        // per-item total of history lengths
-  const unsigned short* g16;  // dense-leg counts [I x ldg] (null: none)
+  const unsigned short* g16;  // dense-leg counts [I x ldg] (null: none); uint8 counts in the G8 kernel
   int64_t ldg;
   const int* pre;         // per item: slot of its pre-accumulated counters in `hbuf`, -1 = none (null: none at all)
   unsigned* hbuf;         // [slots x hstride] packed 16-bit counters summed over the pieces of a split row
@@ -912,7 +912,9 @@ __global__ void __launch_bounds__(1024) k_heavy_plan(const int* __restrict__ ord
   }
 }
 
-template <bool PACK16>
+// G8: the dense-leg counts are uint8 (at most 255 dense users); a separate instantiation, so that the uint16 kernel
+// keeps its code
+template <bool PACK16, bool G8>
 __global__ void __launch_bounds__(1024, 1) k_fit_rows(FitParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
   Entry* list = reinterpret_cast<Entry*>(smem);
@@ -1006,7 +1008,44 @@ __global__ void __launch_bounds__(1024, 1) k_fit_rows(FitParams p) {
       continue;
     }
     const int nwords = PACK16 ? (ns + 1) >> 1 : ns;
-    if (p.g16) {
+    if (G8 && p.g16) {
+      // start from the 8-bit counts of the dense leg: 8 counts (8 B, r0 is a multiple of 8) become 4 packed 16-bit
+      // counter words; counts of columns >= ns (the next row, or padding) are masked off
+      const unsigned char* g8 = reinterpret_cast<const unsigned char*>(p.g16);
+      const uint2* gv = reinterpret_cast<const uint2*>(g8 + (int64_t)i * p.ldg + r0);
+      const int nvec = (ns + 7) >> 3;
+      if (PACK16) {
+        // the row comes from HBM (59 KB at ML-25M shape): one bulk L2 prefetch puts all of it in flight at once, the
+        // loads below then mostly hit L2 (the strip has a spare row at its end, so the rounded-up range stays inside)
+        if (tid == 0) {
+          const uintptr_t b = reinterpret_cast<uintptr_t>(gv) & ~(uintptr_t)15;
+          const uintptr_t e = (reinterpret_cast<uintptr_t>(gv + nvec) + 15) & ~(uintptr_t)15;
+          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(b), "r"((unsigned)(e - b)) : "memory");
+        }
+        uint4* c4 = reinterpret_cast<uint4*>(cnt);
+        for (int s0 = tid; s0 < nvec; s0 += 2 * nt) {  // two loads in flight per thread
+          uint2 v[2];
+#pragma unroll
+          for (int q = 0; q < 2; ++q) v[q] = s0 + q * nt < nvec ? __ldcs(gv + s0 + q * nt) : make_uint2(0u, 0u);
+#pragma unroll
+          for (int q = 0; q < 2; ++q) {
+            const int s = s0 + q * nt;
+            if (s >= nvec) break;
+            const int left = ns - 8 * s;  // valid counts in this vector
+            if (left < 8) {
+              v[q].x = left >= 4 ? v[q].x : v[q].x & ((1u << (8 * left)) - 1u);
+              v[q].y = left <= 4 ? 0u : v[q].y & ((1u << (8 * (left - 4))) - 1u);
+            }
+            c4[s] = make_uint4(__byte_perm(v[q].x, 0u, 0x4140), __byte_perm(v[q].x, 0u, 0x4342),
+                               __byte_perm(v[q].y, 0u, 0x4140), __byte_perm(v[q].y, 0u, 0x4342));
+          }
+        }
+      } else {
+        const unsigned char* grow = g8 + (int64_t)i * p.ldg + r0;
+        for (int s = tid; s < nwords; s += nt) cnt[s] = grow[s];
+      }
+      for (int s = (PACK16 ? 4 * nvec : nwords) + tid; s < (PACK16 ? p.R >> 1 : p.R); s += nt) cnt[s] = 0u;
+    } else if (p.g16) {
       // start from the counts of the dense leg (tensor-core Gram over the densest users)
       const unsigned short* grow = p.g16 + (int64_t)i * p.ldg + r0;
       if (PACK16) {
@@ -1392,8 +1431,12 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
     // rates measured on B200 (profiles/r2_summary.md): the sparse kernel does 6-7e11 counter updates/s when the packed
     // counters of a row fit one pass, 1.8e11/s when the catalogue needs several item-range passes (I = 200,000: 3)
     const bool one_pass = (size_t)I * 2 + 49152 <= (size_t)c->smem_max;
-    const double dense_rate = 1.6e15, sparse_rate = one_pass ? 7e11 : 1.8e11, hbm = 5e12;
-    const double fixed = (double)rows_total * (double)rows_pad * 4.0 / hbm;
+    // The count strip costs its store: measured on B200 at ML-25M shape, Kd = 256 (profiles/r9_bench_before_after.txt),
+    // the Gram writes the 7.0 GB uint16 strip at 2.3 TB/s (16 B per lane from registers) and the 3.5 GB uint8 strip at
+    // 4.3 TB/s (TMA tensor stores).  Halving the bytes the row kernel reads back changed its time by 0.2 %, so the
+    // read-back is not charged.  uint8 needs at most 255 dense users: the model weighs that against its best choice
+    // at 16 bits.
+    const double dense_rate = 1.6e15, sparse_rate = one_pass ? 7e11 : 1.8e11, store_u16 = 2.3e12, store_u8 = 4.3e12;
     double best_gain = 0.0, saved = 0.0;
     int best_h = 0, best_tau = 0;
     int64_t taken = 0;
@@ -1404,7 +1447,9 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
       taken += cnt_d;
       saved += (double)cnt_d * (double)d * (double)d * share / sparse_rate;
       const double kd = (double)((taken + 127) / 128 * 128);
-      const double cost = 2.0 * kd * (double)rows_total * (double)rows_pad / dense_rate + fixed;
+      const double pairs = (double)rows_total * (double)rows_pad;
+      const double strip = taken <= 255 ? pairs / store_u8 : 2.0 * pairs / store_u16;
+      const double cost = 2.0 * kd * pairs / dense_rate + strip;
       const double gain = saved - cost;
       if (!dense_auto || gain > best_gain) {  // a fixed request takes as many users as allowed
         best_gain = gain;
@@ -1420,6 +1465,7 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
   c->mark("fit: item counts + split");
   const int* dense_slot = nullptr;
   const unsigned short* g16 = nullptr;
+  const unsigned char* g8 = nullptr;
   const int* n_sparse = n;  // per-item user counts on the sparse path
   c->last_dense_users = hmax;
   c->last_dense_kd = hmax > 0 ? (int)(((int64_t)hmax + 127) / 128 * 128) : 0;
@@ -1431,7 +1477,9 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
     unsigned char* A = c->buf<unsigned char>("fit_dense_A", (size_t)rows_pad * kd_pad);
     // only this shard's item rows of the dense Gram are needed (row block aligned down to the 128-row tile)
     const int64_t g_row0 = item_begin / 128 * 128;
-    unsigned short* G = c->buf<unsigned short>("fit_dense_G", (size_t)(item_end - g_row0 + 1) * rows_pad);
+    // at most 255 dense users: every count fits 8 bits, and the strip is written and read at half the bytes
+    const bool counts8 = hmax <= 255;
+    unsigned char* G = c->buf<unsigned char>("fit_dense_G", (size_t)(item_end - g_row0 + 1) * rows_pad * (counts8 ? 1 : 2));
     if (strip == 0) {
       const int thr_init[2] = {dense_tau, 0};
       RPK_CUDA(cudaMemcpyAsync(thr_cnt, thr_init, sizeof(thr_init), cudaMemcpyHostToDevice, st));
@@ -1445,11 +1493,17 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
       c->mark("fit: dense operand");
     }
     c->span_begin(0);
-    run_gram_dense_tc(c, A, rows_pad, kd_pad, g_row0, item_end, G, rows_pad);
+    if (counts8) {
+      run_gram_dense_tc(c, A, rows_pad, kd_pad, g_row0, item_end, G, rows_pad);
+      g8 = G - g_row0 * rows_pad;  // indexed by absolute item row in the fit kernel
+    } else {
+      unsigned short* G16 = reinterpret_cast<unsigned short*>(G);
+      run_gram_dense_tc(c, A, rows_pad, kd_pad, g_row0, item_end, G16, rows_pad);
+      g16 = G16 - g_row0 * rows_pad;
+    }
     c->span_end(0);
     c->mark("fit: tensor-core Gram");
     dense_slot = slot;
-    g16 = G - g_row0 * rows_pad;  // indexed by absolute item row in the fit kernel
     n_sparse = n_light;
   }
   scan_i32_i64(c, n_sparse, cscptr, I);
@@ -1557,7 +1611,8 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
     cudaStream_t main_st = st;
     for (int wide = 1; wide >= 0; --wide) {
       cudaStream_t st = wide ? c->side : main_st;  // shadows the outer stream inside this launch
-      auto kern = wide ? k_fit_rows<false> : k_fit_rows<true>;
+      auto kern = wide ? (g8 ? k_fit_rows<false, true> : k_fit_rows<false, false>)
+                       : (g8 ? k_fit_rows<true, true> : k_fit_rows<true, false>);
       // the kernel's static tables (popularity-code table, count floors, heavy columns) come out of the same
       // per-block limit as the dynamic shared memory
       cudaFuncAttributes fa;
@@ -1605,7 +1660,7 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
       fp.csc_users = csc_users;
       fp.pref = pref;
       fp.work = work;
-      fp.g16 = g16;
+      fp.g16 = g8 ? reinterpret_cast<const unsigned short*>(g8) : g16;
       fp.ldg = rows_pad;
       fp.sk = sk;
       fp.order = wide ? order_h : order_l;
@@ -1764,7 +1819,7 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
 }
 
 // The public fit: stages the inputs and outputs once and runs the row range in strips of at most `strip_rows` rows, so
-// that only one strip of the dense-leg count matrix (uint16, rows x I) exists at a time: the item x item matrix is
+// that only one strip of the dense-leg count matrix (uint16 or uint8, rows x I) exists at a time: the item x item matrix is
 // never materialised as a whole (an 80 GB object at I = 200,000) and the tensor-core leg stays on for large catalogues.
 void run_fit(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64_t* indptr_u, const int32_t* indices_u,
              int similarity, const double* item_pow_u, int K, int64_t item_begin, int64_t item_end, int32_t* out_idx_u,

@@ -66,5 +66,8 @@ void run_predict_dense(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr
 void run_gram_dense_u16(rpk_ctx* c, int64_t I, int64_t Kd, const unsigned char* A, unsigned short* G);
 void run_gram_dense_tc(rpk_ctx* c, const unsigned char* A, int64_t rows_pad, int64_t kd_pad, int64_t row_begin,
                        int64_t row_end, unsigned short* G, int64_t ldg);
+// the same with uint8 counts: every row of A holds at most 255 ones
+void run_gram_dense_tc(rpk_ctx* c, const unsigned char* A, int64_t rows_pad, int64_t kd_pad, int64_t row_begin,
+                       int64_t row_end, unsigned char* G, int64_t ldg);
 
 }  // namespace rpk
