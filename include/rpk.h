@@ -19,6 +19,8 @@
  *                       (metrics/dcg.py:21-128, metrics/recall.py:21-85)
  *   rpk_gram_dense_f64 / rpk_ease_from_inverse / rpk_predict_dense_*
  *                       EASE._fit and its dense X @ B predict (recpack/algorithms/ease.py:63-95)
+ *   rpk_embed_topk      the similarity_matrix_ of Prod2Vec (cosine_similarity of the item embeddings +
+ *                       get_top_K_values) and of any item-factor matrix
  *
  * Conventions
  *   - plain C types only; every call returns 0 on success, non-zero on failure, with a
@@ -44,7 +46,7 @@
 extern "C" {
 #endif
 
-#define RPK_ABI_VERSION 2
+#define RPK_ABI_VERSION 3
 
 #if defined(__GNUC__)
 #define RPK_EXPORT __attribute__((visibility("default")))
@@ -54,7 +56,7 @@ extern "C" {
 
 typedef struct rpk_ctx rpk_ctx;
 
-enum { RPK_SIM_COSINE = 0, RPK_SIM_CONDPROB = 1 };
+enum { RPK_SIM_COSINE = 0, RPK_SIM_CONDPROB = 1, RPK_SIM_DOT = 2 /* rpk_embed_topk only */ };
 enum { RPK_METRIC_NDCG = 0, RPK_METRIC_RECALL = 1, RPK_METRIC_DCG = 2, RPK_METRIC_CALIBRATED_RECALL = 3,
        RPK_METRIC_PRECISION = 4,        /* hits / K (recpack/metrics/precision.py:41-50) */
        RPK_METRIC_RECIPROCAL_RANK = 5,  /* 1 / rank of the first hit, 0 without one (metrics/reciprocal_rank.py:37-40) */
@@ -316,6 +318,26 @@ RPK_EXPORT int rpk_predict_dense_topn(rpk_ctx* ctx, int64_t U, int64_t nnz, cons
                            int32_t* out_idx, double* out_val, int32_t* out_len);
 RPK_EXPORT int rpk_predict_dense_full(rpk_ctx* ctx, int64_t U, int64_t nnz, const int64_t* indptr, const int32_t* indices,
                            int64_t I, const double* B, int mask_history, double* out_scores);
+
+/*
+ * Item neighbours of a dense embedding matrix E (float64 [I x D] row-major, finite; 1 <= D <= 1024, I < 2^24,
+ * 1 <= K <= 1024).  DESIGN.md 2, "Embedding neighbours":
+ *   RPK_SIM_DOT:    s_ij = left fold over d = 0 .. D-1 of fl(e_id * e_jd), starting from the first product, separate
+ *                   multiply and add (no FMA); every squared row norm must be below 2^1020
+ *   RPK_SIM_COSINE: the same fold over xhat_i = fl(e_i / n_i), n_i = fl(sqrt(fold of fl(e_id * e_id))); a zero row stays zero
+ * For every row i in [item_begin, item_end): over the columns j != i, the K largest stored values (an exact +-0.0 is not
+ * stored), ordered by (value desc, column asc); negative values are kept when fewer than K larger ones exist.  Outputs
+ * as rpk_fit_topk_real: out_idx int32 [rows x K] (-1 padded), out_val float64 (0 padded, may be NULL), out_len int32[rows].
+ * NaN / inf in E and arguments outside the limits fail the call.  Synchronises once (the check of E).
+ * The tensor cores (tf32) only screen candidates under the error bound of DESIGN.md 4.9; every value and every order
+ * decision is made in float64 on the definition, so the result does not depend on the screen.
+ *
+ * rpk_embed_screen_f32: the screen's approximate matrix, out_S float32 [I x I] (I <= 65536), in the units of s.  For
+ * verification of the bound only.
+ */
+RPK_EXPORT int rpk_embed_topk(rpk_ctx* ctx, int64_t I, int D, const double* E, int similarity, int K,
+                   int64_t item_begin, int64_t item_end, int32_t* out_idx, double* out_val, int32_t* out_len);
+RPK_EXPORT int rpk_embed_screen_f32(rpk_ctx* ctx, int64_t I, int D, const double* E, int similarity, float* out_S);
 
 /* Device time (CUDA events on the context's stream) of the dominant kernels of the last calls:
  * out_ms[0] = tensor-core Gram of the last fit, out_ms[1] = sparse fit kernels of the last fit,

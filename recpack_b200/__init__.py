@@ -8,6 +8,7 @@ from .base import Algorithm, ItemSimilarityMatrixAlgorithm, TopKItemSimilarityMa
 from .matrix import UnsupportedTypeError, to_csr_matrix  # noqa: F401
 from .metrics import NDCGK, DCGK, RecallK, CalibratedRecallK, PrecisionK, ReciprocalRankK, HitK, CoverageK  # noqa: F401
 from .ease import EASE  # noqa: F401
+from .embedding import embedding_top_k  # noqa: F401
 from .nearest_neighbour import ItemKNN, pearson_top_k, real_top_k  # noqa: F401
 from .postprocessing import ExcludeItems, SelectItems  # noqa: F401
 from .splitters import FractionInteractionSplitter  # noqa: F401

@@ -63,6 +63,9 @@ _SIGNATURES = {
     "rpk_split_fraction": (C.c_int, [C.c_void_p, C.c_int64, _i64p, _i64p, _i64p, C.c_int64, C.c_double, C.c_uint64, _vp]),
     "rpk_fit_strip_rows": (C.c_int, [C.c_void_p, C.c_int64]),
     "rpk_last_timings": (C.c_int, [C.c_void_p, _vp]),
+    "rpk_embed_topk": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _f64p, C.c_int, C.c_int, C.c_int64, C.c_int64, _i32p, _f64p,
+                                 _i32p]),
+    "rpk_embed_screen_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _f64p, C.c_int, _vp]),
     "rpk_metrics_topn": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _i32p, _i32p, _i64p, _i32p, C.c_int64, C.c_int,
                                    _i32p, _i32p, _f64p, _f64p, C.c_int, _f64p, _f64p, _i64p]),
 }
@@ -89,7 +92,7 @@ def load():
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args
-    if lib.rpk_abi_version() != 2:
+    if lib.rpk_abi_version() != 3:
         raise RpkError("librpk.so ABI version mismatch; rebuild it")
     _lib = lib
     return lib

@@ -295,6 +295,19 @@ int rpk_gram_dense_u16(rpk_ctx* ctx, int64_t I, int64_t Kd, const uint8_t* A, ui
   RPK_API_END(ctx)
 }
 
+int rpk_embed_topk(rpk_ctx* ctx, int64_t I, int D, const double* E, int similarity, int K, int64_t item_begin,
+                   int64_t item_end, int32_t* out_idx, double* out_val, int32_t* out_len) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_embed_topk(ctx, I, D, E, similarity, K, item_begin, item_end, out_idx, out_val, out_len);
+  RPK_API_END(ctx)
+}
+
+int rpk_embed_screen_f32(rpk_ctx* ctx, int64_t I, int D, const double* E, int similarity, float* out_S) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_embed_screen_f32(ctx, I, D, E, similarity, out_S);
+  RPK_API_END(ctx)
+}
+
 int rpk_last_timings(rpk_ctx* ctx, double* out_ms) {
   RPK_API_BEGIN(ctx)
   if (!out_ms) throw rpk::Error("out_ms must not be null");

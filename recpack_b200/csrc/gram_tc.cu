@@ -19,6 +19,7 @@
 
 #include "common.cuh"
 #include "internal.h"
+#include "tc.cuh"
 
 namespace rpk {
 
@@ -42,45 +43,6 @@ constexpr size_t tc_smem_bytes() {
          256 /*barriers*/;
 }
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-// smem box -> global through the tensor map (bulk async-group of the issuing thread)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(map),
-               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 // D[tmem] (+)= A[smem] * B[smem]^T, int8 x int8 -> int32
 __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -92,23 +54,6 @@ __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t desc_a, uint64
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// Arrive on an mbarrier once all previously issued tcgen05.mma of this thread have completed.
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// K-major operand tile in shared memory, 128 B rows, SWIZZLE_128B (what the TMA box writes): 8-row
-// groups are 1024 B apart (SBO), LBO is unused for swizzled K-major layouts (1), descriptor version 1.
-__device__ __forceinline__ uint64_t umma_desc_kmajor_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFFu) >> 4);  // start address, 16 B units, bits [0,14)
-  d |= (uint64_t)1 << 16;                         // leading byte offset (unused) bits [16,30)
-  d |= (uint64_t)(1024 >> 4) << 32;               // stride byte offset bits [32,46)
-  d |= (uint64_t)1 << 46;                         // descriptor version (Blackwell) bits [46,48)
-  d |= (uint64_t)2 << 61;                         // layout type SWIZZLE_128B bits [61,64)
-  return d;
-}
-
 // Instruction descriptor: dense, no saturation, D = S32, A = B = unsigned 8 bit, both K-major, N, M.
 __host__ __device__ constexpr uint32_t umma_idesc_i8(int M, int N) {
   return (2u << 4) | (0u << 7) | (0u << 10) | (0u << 15) | (0u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
@@ -303,22 +248,6 @@ k_gram_i8_tc(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
 // ------------------------------------------------------------------------------------------
 // Host side
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    RPK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-    RPK_REQUIRE(p != nullptr && q == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled is not available in this driver");
-    fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 // A: device, [rows_pad x kd_pad] uint8 row-major, rows_pad % 256 == 0, kd_pad % 128 == 0.
 // Computes rows [row_begin, row_end) of G = A A^T (row_begin % 128 == 0) against all columns.
 // G: device, [(row_end - row_begin) x ldg] OutT, ldg >= rows_pad.  OutT = uint8 needs at most 255 ones in every row

@@ -69,5 +69,8 @@ void run_gram_dense_tc(rpk_ctx* c, const unsigned char* A, int64_t rows_pad, int
 // the same with uint8 counts: every row of A holds at most 255 ones
 void run_gram_dense_tc(rpk_ctx* c, const unsigned char* A, int64_t rows_pad, int64_t kd_pad, int64_t row_begin,
                        int64_t row_end, unsigned char* G, int64_t ldg);
+void run_embed_topk(rpk_ctx* c, int64_t I, int D, const double* E, int similarity, int K, int64_t item_begin,
+                    int64_t item_end, int32_t* out_idx, double* out_val, int32_t* out_len);
+void run_embed_screen_f32(rpk_ctx* c, int64_t I, int D, const double* E, int similarity, float* out_S);
 
 }  // namespace rpk

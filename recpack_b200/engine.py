@@ -13,6 +13,7 @@ from . import _lib
 from ._lib import RpkError
 
 SIM_CODES = {"cosine": 0, "conditional_probability": 1}
+EMBED_SIM_CODES = {"cosine": 0, "dot": 2}
 METRIC_CODES = {"ndcg": 0, "recall": 1, "dcg": 2, "calibrated_recall": 3, "precision": 4, "reciprocal_rank": 5, "hits": 6}
 
 DBG_WIDE_ACC, DBG_TINY_LIST, DBG_MULTI_PASS, DBG_SPLIT_ROWS, DBG_EXACT_SCORES = 1, 2, 4, 8, 16
@@ -216,6 +217,30 @@ class Engine:
         I, Kd = A.shape
         out = _empty_like_kind(A, (I, I), np.uint16)
         self._check(self._lib.rpk_gram_dense_u16(self._h, int(I), int(Kd), _addr(A, np.uint8), _addr(out, np.uint16)))
+        return out
+
+    # -- item neighbours of a dense embedding matrix ---------------------------------------
+    def embed_topk(self, E, K, similarity="cosine", item_begin=0, item_end=None, want_val=True):
+        """rpk_embed_topk for a float64 [I, D] matrix (numpy or torch CUDA).  Returns dict(idx, val, len), rank order."""
+        I, D = (int(n) for n in E.shape)
+        item_end = I if item_end is None else int(item_end)
+        rows = max(item_end - int(item_begin), 0)
+        out = {
+            "idx": _empty_like_kind(E, (rows, K), np.int32),
+            "val": _empty_like_kind(E, (rows, K), np.float64) if want_val else None,
+            "len": _empty_like_kind(E, (rows,), np.int32),
+        }
+        self._check(self._lib.rpk_embed_topk(self._h, I, D, _addr(E, np.float64), EMBED_SIM_CODES[similarity], int(K),
+                                             int(item_begin), int(item_end), _addr(out["idx"], np.int32),
+                                             _addr(out["val"], np.float64, allow_none=True), _addr(out["len"], np.int32)))
+        return out
+
+    def embed_screen_f32(self, E, similarity="cosine"):
+        """rpk_embed_screen_f32: the screen's approximate [I, I] float32 matrix (verification entry)."""
+        I, D = (int(n) for n in E.shape)
+        out = _empty_like_kind(E, (I, I), np.float32)
+        self._check(self._lib.rpk_embed_screen_f32(self._h, I, D, _addr(E, np.float64), EMBED_SIM_CODES[similarity],
+                                                   _addr(out, np.float32)))
         return out
 
     # -- EASE: dense Gram, closed-form model, dense scoring ----------------------------------
