@@ -10,6 +10,8 @@
 //                                                                       ascending item order, float64, one add per term --
 //                                                                       scipy's csr_matvecs order, so equal inputs give
 //                                                                       bit-identical scores
+#include <stdio.h>
+
 #include <algorithm>
 #include <vector>
 
@@ -441,6 +443,7 @@ struct DenseParams {
   u64* part_key;    // ordered bit patterns of the scores
   int* part_len;
   double* full;     // non-null: write every score [U x I] instead of lists
+  int* nan_flag;    // lists: set when a score to rank is NaN (it has no place in the order)
 };
 
 // One CTA per (user, column range): the scores of the range are accumulated in shared memory, a thread owns its
@@ -478,6 +481,9 @@ __global__ void __launch_bounds__(1024, 1) k_predict_dense(DenseParams p) {
       __syncthreads();
       continue;
     }
+    bool nan = false;
+    for (int s = tid; s < ns; s += nt) nan |= isnan(acc[s]);
+    if (nan) atomicOr(p.nan_flag, 1);
     DenseScoreSrc src{acc, r0, ns};
     const int m = block_select_topk(src, p.N, list, p.cap, p.direct_cap, hist, sh);
     const int64_t slot_out = (int64_t)u * p.P + pass;
@@ -571,9 +577,11 @@ void run_predict_dense(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr
       R = ((I + P - 1) / P + 1) & ~(int64_t)1;
       if ((size_t)R * 8 <= avail) break;
     }
-    if ((c->flags & DBG_MULTI_PASS) && P < 2 && I >= 8) {
-      P = 2;
+    const int p_min = (c->flags & DBG_MANY_PASS) ? 4 : ((c->flags & DBG_MULTI_PASS) ? 2 : 1);
+    if (P < p_min && I >= 4 * p_min) {
+      P = p_min;
       R = ((I + P - 1) / P + 1) & ~(int64_t)1;
+      P = (int)((I + R - 1) / R);  // the even R can leave the last range empty at small I (I = 17: R = 6, three ranges)
     }
     p.indptr = indptr;
     p.indices = indices;
@@ -588,6 +596,8 @@ void run_predict_dense(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr
     p.part_idx = full ? nullptr : c->buf<int>("d_part_idx", (size_t)U * P * N);
     p.part_key = full ? nullptr : c->buf<u64>("d_part_key", (size_t)U * P * N);
     p.part_len = full ? nullptr : c->buf<int>("d_part_len", (size_t)U * P);
+    p.nan_flag = full ? nullptr : c->buf<int>("d_nan", 1);
+    if (!full) RPK_CUDA(cudaMemsetAsync(p.nan_flag, 0, sizeof(int), st));
     const size_t smem = fixed + (size_t)R * 8;
     RPK_CUDA(cudaFuncSetAttribute(k_predict_dense, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int nt = R >= 8192 ? 1024 : (R >= 2048 ? 512 : 256);
@@ -601,7 +611,16 @@ void run_predict_dense(rpk_ctx* c, int64_t U, int64_t nnz, const int64_t* indptr
       const int fgrid = (int)std::min<int64_t>((U * 32 + 255) / 256, (int64_t)c->sm_count * 16);
       k_dense_finalize<<<fgrid, 256, 0, st>>>(p.part_idx, p.part_key, p.part_len, U, P, N, o_idx.dev, o_val.dev, o_len.dev);
       RPK_LAUNCH_CHECK(c);
+      int nan = 0;
+      RPK_CUDA(cudaMemcpyAsync(&nan, p.nan_flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+      RPK_CUDA(cudaStreamSynchronize(st));
+      RPK_REQUIRE(!nan, "dense model: a score to rank is NaN (a NaN in the model, e.g. EASE(alpha != 0) with an item "
+                        "nobody interacted with); top-N is not defined, the full scores are");
     }
+#ifdef RPK_PHASE_PROF
+    fprintf(stderr, "[dense paths] P=%d R=%lld nt=%d smem=%zu users=%lld N=%d full=%d\n", P, (long long)R, nt, smem,
+            (long long)U, Nn, full ? 1 : 0);
+#endif
   }
   o_idx.finish(c);
   o_val.finish(c);

@@ -8,7 +8,9 @@ scaling from rpk_ease_from_inverse.  The model stays on the device as a dense fl
 
 ``_predict``: ``X @ B`` with the dense scorer (rpk_predict_dense_*): every score is the float64 sum over the user's
 history in ascending item order -- the order of scipy's ``csr @ dense`` -- so equal models give bit-identical scores;
-``predict_topK`` / ``remove_history`` as for ItemKNN.
+``predict_topK`` / ``remove_history`` as for ItemKNN.  A NaN in the model (``alpha != 0`` with an item nobody
+interacted with) stays NaN in the full scores, as in the reference; top-N raises ``RpkError`` when a score it would
+rank is NaN.
 
 ``density`` (``_prune``, ease.py:97-109): after the closed form the model is pruned on the device to its
 ``K = min(int(density * I*I), nnz)`` largest-magnitude entries (rpk_ease_prune; ``K = 0`` keeps every entry, as the

@@ -16,7 +16,7 @@ SIM_CODES = {"cosine": 0, "conditional_probability": 1}
 EMBED_SIM_CODES = {"cosine": 0, "dot": 2}
 METRIC_CODES = {"ndcg": 0, "recall": 1, "dcg": 2, "calibrated_recall": 3, "precision": 4, "reciprocal_rank": 5, "hits": 6}
 
-DBG_WIDE_ACC, DBG_TINY_LIST, DBG_MULTI_PASS, DBG_SPLIT_ROWS, DBG_EXACT_SCORES = 1, 2, 4, 8, 16
+DBG_WIDE_ACC, DBG_TINY_LIST, DBG_MULTI_PASS, DBG_SPLIT_ROWS, DBG_EXACT_SCORES, DBG_MANY_PASS = 1, 2, 4, 8, 16, 32
 
 
 def _is_torch(x):
