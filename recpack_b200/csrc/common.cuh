@@ -44,6 +44,7 @@ enum {
   DBG_SPLIT_ROWS = 8,  // fit: cut the heaviest rows into pieces even when they are small
   DBG_EXACT_SCORES = 16,  // predict: exact sums for every list even when only the lists are asked for
   DBG_MANY_PASS = 32,     // predict: at least four item ranges
+  DBG_COARSE_SORT_KEY = 64,  // fit: the finishing sort keeps 24 bits of its keys, so almost every order is settled exactly
 };
 
 }  // namespace rpk

@@ -1237,38 +1237,411 @@ __global__ void __launch_bounds__(256) k_fit_merge(MergeParams p) {
   }
 }
 
-// Sorts the unsorted survivors of a row (written by k_fit_rows) with the exact order and writes the K best.
+// ------------------------------------------------------------------------------------------
+// Finishing kernel: exact top K of the deferred survivors, and the similarity values of every row
+// ------------------------------------------------------------------------------------------
+// c-fold left sum ((x + x) + x) + ... in float64, round to nearest even: scipy's csr_matmat adds the c identical
+// products of a cosine entry one at a time.  Inside one binade of the running sum s (fixed exponent, ulp u) every
+// step from a multiple of u adds the same multiple d of u -- x rounded to u -- while the result stays in the binade.
+// When x / u is a half-integer the tie goes to the even neighbour, so a step that starts inside the binade always
+// lands on an even multiple of u; from there every step adds the same even d.  A step that enters the binade may land
+// on an odd multiple, so the increment is read off two real steps after it, and the steps that stay below the binade's
+// top are taken at once.  Inside a binade the bit patterns are consecutive multiples of u, so this is integer
+// arithmetic on them.  About three real additions per binade: at most ~50 for c < 2^17.
+__device__ __forceinline__ double repeat_sum(double x, int c) {
+  double s = 0.0;
+  int r = 0;
+  while (r < c) {
+    const double s0 = s;
+    s = __dadd_rn(s, x);
+    ++r;
+    const long long b = __double_as_longlong(s);
+    if (r == c || s0 == 0.0 || (__double_as_longlong(s0) >> 52) != (b >> 52)) continue;
+    // s was reached by a step inside its binade
+    const double s1 = __dadd_rn(s, x);
+    ++r;
+    const long long b1 = __double_as_longlong(s1);
+    s = s1;
+    if (r == c || (b1 >> 52) != (b >> 52)) continue;
+    const long long d = b1 - b;                             // ulps per step until the binade ends
+    const long long room = (((b >> 52) + 1) << 52) - 1 - b1;  // ulps from s1 to the binade's largest value
+    long long t = c - r;
+    if (d > 0) {
+      // room, d < 2^53: the rounded quotient never reaches the next integer above the exact one
+      const long long q = (long long)((double)room / (double)d);
+      if (q < t) t = q;
+    }
+    s = __longlong_as_double(b1 + t * d);
+    r += (int)t;
+  }
+  return s;
+}
+
+// Similarity values in the reference's floating-point operation order (include/rpk.h).  Row factor of item i: cosine
+// a_i = 1/sqrt(n_i) -- sklearn row-normalises X^T (sparsefuncs_fast.pyx:578-604); conditional probability 1/n_i
+// (algorithms/util.py:132).
+__device__ __forceinline__ double row_factor(int mode, int n_i) {
+  return mode == 0 ? __ddiv_rn(1.0, __dsqrt_rn((double)n_i)) : __ddiv_rn(1.0, (double)n_i);
+}
+// Value of entry (i, j) with count c, f_i = row_factor(i).
+__device__ __forceinline__ double sim_value(int mode, double f_i, int n_j, int c, const double* pw, int j) {
+  if (mode == 0) {
+    // scipy's csr_matmat adds the c identical products fl(a_i a_j) one at a time
+    const double aj = __ddiv_rn(1.0, __dsqrt_rn((double)n_j));
+    return repeat_sum(__dmul_rn(f_i, aj), c);
+  }
+  double v = __dmul_rn(f_i, (double)c);    // A @ co_mat
+  if (mode == 2) v = __dmul_rn(v, pw[j]);  // ... @ A.power(pop_discount)
+  return v;
+}
+
+#ifdef RPK_PHASE_PROF
+// rows sorted, rows given values only, comparisons settled exactly, then cycles of the first thread of a group in the
+// phases of a sorted row: load + keys, select, compaction, sort, output + values
+__device__ unsigned long long g_fit_sort[8];
+#define SORT_MARK(k)                           \
+  do {                                         \
+    if (g == 0) {                              \
+      const long long t_now = clock64();       \
+      cyc[k] += (unsigned long long)(t_now - t_prev); \
+      t_prev = t_now;                          \
+    }                                          \
+  } while (0)
+#else
+#define SORT_MARK(k) do {} while (0)
+#endif
+
 struct SortParams {
-  SimKey sk;
+  const int* n;
+  const double* pw;
   const int* scr_idx;
   const int* scr_cnt;
   const int* scr_len;
-  int defer_max, K, cap, direct_cap;
-  int64_t nrows;
+  int* queue;  // next row to take (zeroed before the launch)
+  int defer_max, K, mode;
+  int64_t nrows, item_begin;
+  u64 key_mask;  // ~0, or the low 40 bits cleared (DBG_COARSE_SORT_KEY)
+  u64 margin;    // two sort keys further apart than this many bit patterns are in exact order
   int* out_idx;
   int* out_cnt;
   int* out_len;
+  double* out_val;  // null: no values asked for
 };
-__global__ void __launch_bounds__(256) k_fit_sort_rows(SortParams p) {
-  extern __shared__ __align__(16) unsigned char smem[];
-  Entry* list = reinterpret_cast<Entry*>(smem);
-  int* hist = reinterpret_cast<int*>(smem + sel_list_bytes(p.cap));
-  SelShared* sh = reinterpret_cast<SelShared*>(hist + SEL_BINS);
-  const int tid = threadIdx.x, nt = blockDim.x;
-  for (int64_t row = blockIdx.x; row < p.nrows; row += gridDim.x) {
-    const int m = p.scr_len[row];
-    if (m < 0) continue;  // already final
-    // exact selection + sort of the survivors with the precise keys (exact reciprocal popularity): the same
-    // routine as everywhere else, now on a list of a few hundred entries, many rows per SM at once
-    PairListSrc src{p.sk, p.scr_idx + row * p.defer_max, p.scr_cnt + row * p.defer_max, m};
-    const int keep = block_select_topk(src, p.K, list, p.cap, p.direct_cap, hist, sh);
-    for (int t = tid; t < p.K; t += nt) {
-      p.out_idx[row * p.K + t] = t < keep ? list[t].idx : -1;
-      p.out_cnt[row * p.K + t] = t < keep ? list[t].aux : 0;
-    }
-    if (tid == 0) p.out_len[row] = keep;
-    __syncthreads();
+
+constexpr int SORT_BINS = 256;  // radix of the threshold select
+struct SortGroupShared {
+  u64 w64[16];  // per-warp minima / maxima (256-thread groups)
+  int wsum[8];  // per-warp sums
+  u64 lo;       // the select's next bin
+  int above, n_in;
+  int row;
+};
+// per group: keys and (index, count) pairs of up to defer_max entries, the histogram, the scratch above
+__host__ __device__ __forceinline__ size_t sort_group_bytes(int defer_max) {
+  return (size_t)defer_max * 16 + SORT_BINS * 4 + (sizeof(SortGroupShared) + 15) / 16 * 16;
+}
+
+// The order of the deferred survivors.  Sort key: cosine fl((double)fl(c^2) / n_j) -- correctly rounded from exact
+// operands while c^2 < 2^53, so it never inverts two exact values there; for c up to 2^31 each of the two roundings
+// moves the key by at most 2^-53 relative, so two keys in the wrong order are at most 4 bit patterns apart (M = 4).
+// Conditional probability: the float64 key is the definition (M = 0).  Keys further apart than M decide; otherwise
+// the exact comparison (SimKey::cmp3), then the ascending index -- the canonical total order of the oracle.
+// The exact comparison takes n_j from the key itself: fl(fl(c^2) / k) is n_j within n_j 2^-51 < 2^-20 for
+// n_j, c < 2^31, so rounding it gives n_j exactly, without a global load in the sort.
+struct SortOrder {
+  u64 mask, M;
+  int mode;
+  __device__ __forceinline__ static u64 pop_of(u64 k, int c) {
+    if (c == 0) return 1ull;  // padding
+    return (u64)__double2ll_rn(__ddiv_rn((double)((u64)c * (u64)c), __longlong_as_double((long long)k)));
   }
+  __device__ __forceinline__ int exact(u64 ka, int ca, u64 kb, int cb) const {
+    if (mode != 0) return ka == kb ? 0 : (ka > kb ? 1 : -1);
+    // c_a^2 / n_a  vs  c_b^2 / n_b   <=>   c_a^2 * n_b  vs  c_b^2 * n_a   (128-bit exact); padding: c = 0
+    const u64 na = pop_of(ka, ca), nb = pop_of(kb, cb);
+    const u64 ca2 = (u64)(unsigned)ca * (u64)(unsigned)ca, cb2 = (u64)(unsigned)cb * (u64)(unsigned)cb;
+    const u64 l_lo = ca2 * nb, l_hi = __umul64hi(ca2, nb);
+    const u64 r_lo = cb2 * na, r_hi = __umul64hi(cb2, na);
+    if (l_hi != r_hi) return l_hi > r_hi ? 1 : -1;
+    if (l_lo != r_lo) return l_lo > r_lo ? 1 : -1;
+    return 0;
+  }
+  // true when a precedes b; keys are positive doubles (< 2^63 as patterns), so k + M does not wrap
+  __device__ __forceinline__ bool before(u64 ka, int ia, int ca, u64 kb, int ib, int cb, unsigned& n_exact) const {
+    const u64 a = ka & mask, b = kb & mask;
+    if (a > b + M) return true;
+    if (b > a + M) return false;
+    ++n_exact;
+    // the same key from the same count: the same n_j (cosine), the same value; padding against padding too
+    if (ka == kb && ca == cb) return ia < ib;
+    const int c3 = exact(ka, ca, kb, cb);
+    return c3 != 0 ? c3 > 0 : ia < ib;
+  }
+};
+
+// Group of GW threads: one warp, or a whole 256-thread block for the largest K.
+template <int GW>
+__device__ __forceinline__ void group_sync() {
+  if (GW == 32) __syncwarp();
+  else __syncthreads();
+}
+// Inclusive prefix sum over the group in thread order; *total = the group's sum.  wsum: GW / 32 ints of shared memory.
+template <int GW>
+__device__ __forceinline__ int group_scan(int v, int* wsum, int* total) {
+  const int lane = threadIdx.x & 31;
+  int incl = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int t = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += t;
+  }
+  if (GW == 32) {
+    *total = __shfl_sync(0xffffffffu, incl, 31);
+    return incl;
+  }
+  const int w = (threadIdx.x % GW) >> 5;
+  if (lane == 31) wsum[w] = incl;
+  __syncthreads();
+  int before = 0, tot = 0;
+#pragma unroll
+  for (int q = 0; q < GW / 32; ++q) {
+    const int s = wsum[q];
+    before += q < w ? s : 0;
+    tot += s;
+  }
+  __syncthreads();
+  *total = tot;
+  return incl + before;
+}
+template <int GW>
+__device__ __forceinline__ void group_min_max(u64& lo, u64& hi, u64* w64) {
+  lo = warp_min_u64(lo);
+  hi = warp_max_u64(hi);
+  if (GW == 32) return;
+  const int w = (threadIdx.x % GW) >> 5;
+  if ((threadIdx.x & 31) == 0) {
+    w64[w] = lo;
+    w64[GW / 32 + w] = hi;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int q = 0; q < GW / 32; ++q) {
+    lo = w64[q] < lo ? w64[q] : lo;
+    hi = w64[GW / 32 + q] > hi ? w64[GW / 32 + q] : hi;
+  }
+  __syncthreads();
+}
+
+// One group per row, rows taken from a counter.  A deferred row (scr_len >= 0: its survivors, unsorted, written by
+// k_fit_rows): keys into shared memory, a radix select of the K-th largest key tau, every survivor with key >= tau - M
+// kept (one below is beaten by at least K others), a bitonic sort of those with the exact order, the first K written
+// with their values.  A row already final (scr_len = -1): its values only.  GW = 32 for defer_max <= 1024 (K <= 512),
+// 256 above.
+template <int GW>
+__global__ void __launch_bounds__(GW == 32 ? 64 : 256) k_fit_sort_rows(SortParams p) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const int D = p.defer_max, K = p.K;
+  const int g = threadIdx.x % GW;
+  unsigned char* base = smem + (size_t)(threadIdx.x / GW) * sort_group_bytes(D);
+  u64* skey = reinterpret_cast<u64*>(base);
+  int2* sic = reinterpret_cast<int2*>(skey + D);  // (index, count)
+  int* hist = reinterpret_cast<int*>(sic + D);
+  SortGroupShared* gs = reinterpret_cast<SortGroupShared*>(hist + SORT_BINS);
+  const SortOrder ord{p.key_mask, p.margin, p.mode};
+  unsigned n_exact = 0;
+#ifdef RPK_PHASE_PROF
+  unsigned long long n_sorted = 0, n_values = 0, cyc[5] = {0, 0, 0, 0, 0};
+  long long t_prev = 0;
+#endif
+  for (;;) {
+    if (g == 0) gs->row = atomicAdd(p.queue, 1);
+    group_sync<GW>();
+    const int64_t row = gs->row;
+    group_sync<GW>();
+    if (row >= p.nrows) break;
+    const int m = p.scr_len[row];
+    const int i = (int)(p.item_begin + row);
+    const double f_i = row_factor(p.mode, p.n[i]);
+    int* o_idx = p.out_idx + row * K;
+    int* o_cnt = p.out_cnt + row * K;
+    double* o_val = p.out_val ? p.out_val + row * K : nullptr;
+    if (m < 0) {  // sorted by k_fit_rows or merged by k_fit_merge
+      if (!o_val) continue;
+      for (int t = g; t < K; t += GW) {
+        const int j = o_idx[t];
+        o_val[t] = j >= 0 ? sim_value(p.mode, f_i, p.n[j], o_cnt[t], p.pw, j) : 0.0;
+      }
+#ifdef RPK_PHASE_PROF
+      n_values++;
+#endif
+      continue;
+    }
+#ifdef RPK_PHASE_PROF
+    n_sorted++;
+    if (g == 0) t_prev = clock64();
+#endif
+    const int* r_idx = p.scr_idx + row * D;
+    const int* r_cnt = p.scr_cnt + row * D;
+#pragma unroll 4
+    for (int t = g; t < m; t += GW) sic[t] = make_int2(r_idx[t], r_cnt[t]);
+    group_sync<GW>();
+    u64 kmin = ~0ull, kmax = 0ull;
+#pragma unroll 4
+    for (int t = g; t < m; t += GW) {
+      const int2 e = sic[t];
+      u64 k;
+      if (p.mode == 0) k = (u64)__double_as_longlong(__ddiv_rn((double)((u64)e.y * (u64)e.y), (double)p.n[e.x]));
+      else if (p.mode == 1) k = (u64)__double_as_longlong((double)e.y);
+      else k = (u64)__double_as_longlong(__dmul_rn((double)e.y, p.pw[e.x]));
+      skey[t] = k;
+      const u64 km = k & p.key_mask;
+      kmin = km < kmin ? km : kmin;
+      kmax = km > kmax ? km : kmax;
+    }
+    SORT_MARK(0);
+    int kept = m;
+    if (m > K) {
+      // ---- radix select: narrow [lo, hi] to the bin of the K-th largest key until at most `room` keys lie at or
+      //      above lo (or the bin is one key); g_above = keys above hi, n_in = keys in [lo, hi]
+      group_min_max<GW>(kmin, kmax, gs->w64);
+      int room = 1;
+      while (room < K + K / 16 + 1) room <<= 1;
+      u64 lo = kmin, hi = kmax;
+      int g_above = 0, n_in = m;
+      while (g_above + n_in > room && lo < hi) {
+        int shift, nb;
+        bin_geometry<8>(lo, hi, shift, nb);
+        for (int b = g; b < nb; b += GW) hist[b] = 0;
+        group_sync<GW>();
+        for (int t = g; t < m; t += GW) {
+          const u64 k = skey[t] & p.key_mask;
+          if (k >= lo && k <= hi) atomicAdd(&hist[(int)((k - lo) >> shift)], 1);
+        }
+        group_sync<GW>();
+        // the bin holding the K-th largest key, scanning from the top: thread g owns bins [b0, b1)
+        const int per = (nb + GW - 1) / GW;
+        const int b0 = min(nb, g * per), b1 = min(nb, b0 + per);
+        int tsum = 0;
+        for (int b = b0; b < b1; ++b) tsum += hist[b];
+        int total;
+        const int incl = group_scan<GW>(tsum, gs->wsum, &total);
+        int above = g_above + total - incl;  // keys in bins of higher threads
+        if (above < K && above + tsum >= K) {
+          for (int b = b1 - 1; b >= b0; --b) {
+            if (above + hist[b] >= K) {
+              gs->lo = lo + ((u64)b << shift);
+              gs->above = above;
+              gs->n_in = hist[b];
+              break;
+            }
+            above += hist[b];
+          }
+        }
+        group_sync<GW>();
+        const u64 nlo = gs->lo;
+        g_above = gs->above;
+        n_in = gs->n_in;
+        group_sync<GW>();
+        u64 nhi = nlo + ((1ull << shift) - 1);
+        if (nhi > hi || nhi < nlo) nhi = hi;
+        lo = nlo;
+        hi = nhi;
+      }
+      const u64 thr = lo > p.margin ? lo - p.margin : 0ull;
+      SORT_MARK(1);
+      // ---- keep the survivors with key >= thr: stable compaction in place (a kept entry moves to a lower or its own
+      //      position; each round reads its GW entries before any of them is overwritten)
+      kept = 0;
+      for (int r0 = 0; r0 < m; r0 += GW) {
+        const int t = r0 + g;
+        u64 k = 0;
+        int2 e = make_int2(0, 0);
+        bool keep = false;
+        if (t < m) {
+          k = skey[t];
+          e = sic[t];
+          keep = (k & p.key_mask) >= thr;
+        }
+        int total, pos;
+        if (GW == 32) {
+          const unsigned ball = __ballot_sync(0xffffffffu, keep);
+          total = __popc(ball);
+          pos = kept + __popc(ball & ((1u << g) - 1u));
+        } else {
+          pos = kept + group_scan<GW>(keep ? 1 : 0, gs->wsum, &total) - 1;
+        }
+        group_sync<GW>();
+        if (keep) {
+          skey[pos] = k;
+          sic[pos] = e;
+        }
+        kept += total;
+        group_sync<GW>();
+      }
+      SORT_MARK(2);
+    }
+    // ---- bitonic sort of the kept entries, best first; padding (key 0, count 0, index SENTINEL_IDX) sorts last
+    int n2 = 1;
+    while (n2 < kept) n2 <<= 1;
+    for (int t = kept + g; t < n2; t += GW) {
+      skey[t] = 0ull;
+      sic[t] = make_int2(SENTINEL_IDX, 0);
+    }
+    group_sync<GW>();
+    for (int k2 = 2; k2 <= n2; k2 <<= 1) {
+      for (int j2 = k2 >> 1; j2 > 0; j2 >>= 1) {
+#pragma unroll 4
+        for (int q = g; q < (n2 >> 1); q += GW) {
+          const int a = ((q & ~(j2 - 1)) << 1) | (q & (j2 - 1)), b = a + j2;
+          const u64 ka = skey[a], kb = skey[b];
+          const int2 ea = sic[a], eb = sic[b];
+          const bool up = (a & k2) == 0;
+          if (ord.before(kb, eb.x, eb.y, ka, ea.x, ea.y, n_exact) == up) {
+            skey[a] = kb;
+            skey[b] = ka;
+            sic[a] = eb;
+            sic[b] = ea;
+          }
+        }
+        group_sync<GW>();
+      }
+    }
+    SORT_MARK(3);
+    const int keep = kept < K ? kept : K;
+    // four entries per thread at a time, so that their popularity loads overlap
+    for (int t0 = g; t0 < K; t0 += 4 * GW) {
+      int2 e[4];
+      int nj[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int t = t0 + u * GW;
+        e[u] = t < keep ? sic[t] : make_int2(-1, 0);
+        nj[u] = e[u].x >= 0 ? p.n[e[u].x] : 1;
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int t = t0 + u * GW;
+        if (t < K) {
+          o_idx[t] = e[u].x;
+          o_cnt[t] = e[u].y;
+          if (o_val) o_val[t] = e[u].x >= 0 ? sim_value(p.mode, f_i, nj[u], e[u].y, p.pw, e[u].x) : 0.0;
+        }
+      }
+    }
+    if (g == 0) p.out_len[row] = keep;
+    group_sync<GW>();
+    SORT_MARK(4);
+  }
+#ifdef RPK_PHASE_PROF
+  if (g == 0) {
+    atomicAdd(&g_fit_sort[0], n_sorted);
+    atomicAdd(&g_fit_sort[1], n_values);
+    for (int k = 0; k < 5; ++k) atomicAdd(&g_fit_sort[3 + k], cyc[k]);
+  }
+  atomicAdd(&g_fit_sort[2], (unsigned long long)n_exact);
+#else
+  (void)n_exact;
+#endif
 }
 
 // Stable split of the heaviest-first row order into rows whose counts fit 16 bits and the rest (one block).
@@ -1311,35 +1684,6 @@ __global__ void __launch_bounds__(1024) k_split_rows(const int* __restrict__ ord
     counts[0] = nl;
     counts[1] = nh;
   }
-}
-
-// Similarity values with the reference's floating-point operation order (see include/rpk.h).
-__global__ void k_fit_values(const int* __restrict__ idx, const int* __restrict__ cnt, const int* __restrict__ n,
-                             const double* __restrict__ pw, int mode, int64_t item_begin, int64_t nrows, int K,
-                             double* __restrict__ val) {
-  int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= nrows * K) return;
-  const int j = idx[t];
-  double v = 0.0;
-  if (j >= 0) {
-    const int i = (int)(item_begin + t / K);
-    const int c = cnt[t];
-    if (mode == 0) {
-      // sklearn row-normalises X^T: a = 1/sqrt(n) (sparsefuncs_fast.pyx:578-604); scipy's csr_matmat then
-      // adds the c identical products one at a time
-      const double ai = __ddiv_rn(1.0, __dsqrt_rn((double)n[i]));
-      const double aj = __ddiv_rn(1.0, __dsqrt_rn((double)n[j]));
-      const double prod = __dmul_rn(ai, aj);
-      double s = 0.0;
-      for (int r = 0; r < c; ++r) s = __dadd_rn(s, prod);
-      v = s;
-    } else {
-      const double inv = __ddiv_rn(1.0, (double)n[i]);  // algorithms/util.py:132
-      v = __dmul_rn(inv, (double)c);                   // A @ co_mat
-      if (mode == 2) v = __dmul_rn(v, pw[j]);          // ... @ A.power(pop_discount)
-    }
-  }
-  val[t] = v;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1788,31 +2132,56 @@ static void fit_range(rpk_ctx* c, int64_t U, int64_t I, int64_t nnz, const int64
 #endif
     c->mark("fit: row kernels");
     c->span_end(1);  // the row kernels end here (rpk_last_timings); the deferred sort is timed with the rest of the fit
-    if (any_deferred) {
+    if (any_deferred || o_val.dev) {
+      // one finishing launch: the deferred rows are selected and sorted, every row gets its values
+      const bool coarse = (c->flags & DBG_COARSE_SORT_KEY) != 0;  // test hook: nearly every order settled exactly
+      int* queue = c->buf<int>("fit_sort_queue", 1);
+      RPK_CUDA(cudaMemsetAsync(queue, 0, sizeof(int), st));
       SortParams sp;
-      sp.sk = sk;
+      sp.n = n;
+      sp.pw = pw;
       sp.scr_idx = scr_idx;
       sp.scr_cnt = scr_cnt;
       sp.scr_len = scr_len;
+      sp.queue = queue;
       sp.defer_max = defer_max;
       sp.K = K;
-      sp.cap = std::max(256, next_pow2(2 * K));
-      sp.direct_cap = std::min(sp.cap, std::max(K + K / 4, 64));
+      sp.mode = mode;
       sp.nrows = nrows;
+      sp.item_begin = item_begin;
+      sp.key_mask = coarse ? ~((1ull << 40) - 1) : ~0ull;
+      sp.margin = coarse ? (1ull << 40) : (mode == 0 ? 4ull : 0ull);
       sp.out_idx = o_idx.dev;
       sp.out_cnt = cnt_dev;
       sp.out_len = o_len.dev;
-      const size_t ssm = sel_smem_bytes(sp.cap);
-      RPK_CUDA(cudaFuncSetAttribute(k_fit_sort_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm));
+      sp.out_val = o_val.dev;
+#ifdef RPK_PHASE_PROF
+      static const unsigned long long sort_zero[8] = {};
+      RPK_CUDA(cudaMemcpyToSymbolAsync(g_fit_sort, sort_zero, sizeof(sort_zero), 0, cudaMemcpyHostToDevice, st));
+#endif
+      // one warp per row while the survivors fit 1,024 (K <= 512), a 256-thread block per row above
+      const bool warp_rows = defer_max <= 1024;
+      auto kern = warp_rows ? k_fit_sort_rows<32> : k_fit_sort_rows<256>;
+      const int nt = warp_rows ? 64 : 256;
+      const size_t ssm = sort_group_bytes(defer_max) * (nt / (warp_rows ? 32 : 256));
+      RPK_REQUIRE(ssm <= (size_t)c->smem_max, "K too large for shared memory");
+      RPK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssm));
       int socc = 0;
-      RPK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&socc, k_fit_sort_rows, 256, ssm));
-      const int sgrid = (int)std::min<int64_t>(nrows, (int64_t)c->sm_count * std::max(socc, 1));
-      k_fit_sort_rows<<<sgrid, 256, ssm, st>>>(sp);
+      RPK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&socc, kern, nt, ssm));
+      const int rows_per_block = warp_rows ? nt / 32 : 1;
+      const int sgrid = (int)std::max<int64_t>(1, std::min<int64_t>((nrows + rows_per_block - 1) / rows_per_block,
+                                                                      (int64_t)c->sm_count * std::max(socc, 1)));
+      kern<<<sgrid, nt, ssm, st>>>(sp);
       RPK_LAUNCH_CHECK(c);
-    }
-    if (o_val.dev) {
-      k_fit_values<<<ceil_div(nrows * K, 256), 256, 0, st>>>(o_idx.dev, cnt_dev, n, pw, mode, item_begin, nrows, K, o_val.dev);
-      RPK_LAUNCH_CHECK(c);
+#ifdef RPK_PHASE_PROF
+      unsigned long long fs[8];
+      RPK_CUDA(cudaMemcpyFromSymbolAsync(fs, g_fit_sort, sizeof(fs), 0, cudaMemcpyDeviceToHost, st));
+      RPK_CUDA(cudaStreamSynchronize(st));
+      const double rs = fs[0] ? (double)fs[0] : 1.0;
+      fprintf(stderr, "[fit sort] sorted=%llu values_only=%llu exact_cmp=%llu coarse=%d  cycles/sorted row: load %.0f select %.0f "
+              "compact %.0f sort %.0f out %.0f\n", fs[0], fs[1], fs[2], (int)coarse, fs[3] / rs, fs[4] / rs, fs[5] / rs, fs[6] / rs,
+              fs[7] / rs);
+#endif
     }
   }
   c->mark("fit: sort + values");
