@@ -21,6 +21,8 @@
  *                       EASE._fit and its dense X @ B predict (recpack/algorithms/ease.py:63-95)
  *   rpk_embed_topk      the similarity_matrix_ of Prod2Vec (cosine_similarity of the item embeddings +
  *                       get_top_K_values) and of any item-factor matrix
+ *   rpk_factor_*        FactorizationAlgorithm._predict (recpack/algorithms/base.py:307-369; SVD, NMF):
+ *                       user_embedding_ @ item_embedding_.T for the users with history
  *
  * Conventions
  *   - plain C types only; every call returns 0 on success, non-zero on failure, with a
@@ -338,6 +340,32 @@ RPK_EXPORT int rpk_predict_dense_full(rpk_ctx* ctx, int64_t U, int64_t nnz, cons
 RPK_EXPORT int rpk_embed_topk(rpk_ctx* ctx, int64_t I, int D, const double* E, int similarity, int K,
                    int64_t item_begin, int64_t item_end, int32_t* out_idx, double* out_val, int32_t* out_len);
 RPK_EXPORT int rpk_embed_screen_f32(rpk_ctx* ctx, int64_t I, int D, const double* E, int similarity, float* out_S);
+
+/*
+ * Factor models (DESIGN.md 2, "Factor models"): user factors P (float64 [U x D], one row per row of X), item factors Q
+ * (float64 [I x D]), both row-major and finite; 1 <= D <= 1024, I < 2^24, every squared row norm below 2^1020.  X is the
+ * CSR of the rows scored (indptr int64[U+1], indices int32[nnz], ascending unique columns per row; structure only).
+ *   s_uj = left fold over d = 0 .. D-1 of fl(p_ud * q_jd), starting from the first product, separate multiply and add.
+ * Only users with at least one entry in X are scored; every other row is empty (len 0 / all 0.0).  A score of exactly
+ * 0.0 is not stored.  mask_history removes the user's own columns, then the item filter of rpk_predict_item_filter
+ * (when set, for I items) removes the filtered columns.
+ *   rpk_factor_topn        the N largest stored scores per user (1 <= N <= 1024) by (score desc, column asc), negative
+ *                          ones included when fewer than N larger ones exist; outputs as rpk_predict_topn: out_idx int32
+ *                          [U x N] (-1 padded), out_val float64 (0 padded, may be NULL), out_len int32 [U].  The tensor
+ *                          cores (tf32) only screen candidates under the bound of DESIGN.md 4.10; every value and order
+ *                          decision is made in float64 on the definition.
+ *   rpk_factor_full        every score, out_scores float64 [U x I] (0.0 = not stored), as the reference's dense product.
+ *   rpk_factor_screen_f32  the screen's approximate matrix, out_S float32 [U x I] (U, I <= 65536), in the units of s.
+ *                          For verification of the bound only.
+ * NaN / inf, a malformed X and arguments outside the limits fail the call.  Synchronises once (the checks).
+ * P, Q and X may be host or device memory.
+ */
+RPK_EXPORT int rpk_factor_topn(rpk_ctx* ctx, int64_t U, int64_t I, int D, const double* P, const double* Q, int64_t nnz,
+                    const int64_t* indptr, const int32_t* indices, int N, int mask_history,
+                    int32_t* out_idx, double* out_val, int32_t* out_len);
+RPK_EXPORT int rpk_factor_full(rpk_ctx* ctx, int64_t U, int64_t I, int D, const double* P, const double* Q, int64_t nnz,
+                    const int64_t* indptr, const int32_t* indices, int mask_history, double* out_scores);
+RPK_EXPORT int rpk_factor_screen_f32(rpk_ctx* ctx, int64_t U, int64_t I, int D, const double* P, const double* Q, float* out_S);
 
 /* Device time (CUDA events on the context's stream) of the dominant kernels of the last calls:
  * out_ms[0] = tensor-core Gram of the last fit, out_ms[1] = sparse fit kernels of the last fit,

@@ -66,6 +66,11 @@ _SIGNATURES = {
     "rpk_embed_topk": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _f64p, C.c_int, C.c_int, C.c_int64, C.c_int64, _i32p, _f64p,
                                  _i32p]),
     "rpk_embed_screen_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _f64p, C.c_int, _vp]),
+    "rpk_factor_topn": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, _f64p, _f64p, C.c_int64, _i64p, _i32p, C.c_int,
+                                  C.c_int, _i32p, _f64p, _i32p]),
+    "rpk_factor_full": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, _f64p, _f64p, C.c_int64, _i64p, _i32p, C.c_int,
+                                  _f64p]),
+    "rpk_factor_screen_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, _f64p, _f64p, _vp]),
     "rpk_metrics_topn": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _i32p, _i32p, _i64p, _i32p, C.c_int64, C.c_int,
                                    _i32p, _i32p, _f64p, _f64p, C.c_int, _f64p, _f64p, _i64p]),
 }

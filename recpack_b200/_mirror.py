@@ -59,6 +59,19 @@ class TopKItemSimilarityMatrixAlgorithm(ItemSimilarityMatrixAlgorithm):
         self.K = K
 
 
+class FactorizationAlgorithm(Algorithm):
+    """Constructor and fit check of recpack/algorithms/base.py:307-369."""
+
+    def __init__(self, num_components=100):
+        super().__init__()
+        self.num_components = num_components
+
+    def _check_fit_complete(self):
+        super()._check_fit_complete()
+        assert hasattr(self, "user_embedding_")
+        assert hasattr(self, "item_embedding_")
+
+
 class ItemKNNArgs(TopKItemSimilarityMatrixAlgorithm):
     """Constructor contract of recpack/algorithms/nearest_neighbour.py:170-202."""
 

@@ -30,7 +30,37 @@ else:
     _TopKBase = _mirror.TopKItemSimilarityMatrixAlgorithm
 
 
-class GpuSimilarityMixin:
+class GpuPredictMixin:
+    """What every GPU ``_predict`` of this package adds to the reference's contract: ``predict_topK``,
+    ``remove_history`` and ``set_postfilters`` (below), the predict input coercion (structure only, memoised per
+    matrix) and the reference's "failed to recommend" check computed from row pointers."""
+
+    predict_topK = None
+    remove_history = False
+    _postfilters = ()
+
+    def set_postfilters(self, filters):
+        """Post-filters (``recpack_b200.postprocessing.ExcludeItems`` / ``SelectItems``) applied inside predict,
+        before the truncation to ``predict_topK``: the filtered items are never recommended and the lists are
+        refilled from the items that remain (postprocessing/filters.py:58-101 on an untruncated matrix)."""
+        self._postfilters = tuple(filters or ())
+        return self
+
+    def _transform_predict_input(self, X):
+        return to_csr_matrix(X, binary=True)
+
+    def _check_prediction(self, X_pred: csr_matrix, X: csr_matrix) -> None:
+        """Warn when a user with history got no recommendation (base.py:108-127)."""
+        has_hist = np.diff(X.indptr) > 0
+        has_pred = np.diff(X_pred.indptr) > 0
+        if X_pred.nnz and not np.all(X_pred.data):  # explicit zeros do not count as recommendations
+            has_pred = np.asarray((X_pred != 0).sum(axis=1)).ravel() > 0
+        missing = int(np.count_nonzero(has_hist & ~has_pred))
+        if missing > 0:
+            warnings.warn(f"{self.name} failed to recommend any items for {missing} users")
+
+
+class GpuSimilarityMixin(GpuPredictMixin):
     """GPU implementation of the ``ItemSimilarityMatrixAlgorithm`` contract (base.py:220-279): predict =
     X @ similarity_matrix_.
 
@@ -51,17 +81,6 @@ class GpuSimilarityMixin:
     over the user's history items in ascending order; sums of exactly 0.0 are not stored), and ``predict_topK``
     keeps the N largest stored scores, negative ones included when fewer than N positive ones exist (DESIGN.md 2).
     Similarity values must be finite."""
-
-    predict_topK = None
-    remove_history = False
-    _postfilters = ()
-
-    def set_postfilters(self, filters):
-        """Post-filters (``recpack_b200.postprocessing.ExcludeItems`` / ``SelectItems``) applied inside predict,
-        before the truncation to ``predict_topK``: the filtered items are never recommended and the lists are
-        refilled from the items that remain (postprocessing/filters.py:58-101 on an untruncated matrix)."""
-        self._postfilters = tuple(filters or ())
-        return self
 
     def truncated(self, K: int):
         """The same model cut to the K (<= self.K) best neighbours per item, without fitting again: the fitted lists
@@ -170,19 +189,6 @@ class GpuSimilarityMixin:
     def _transform_fit_input(self, X):
         return to_csr_matrix(X, binary=True)
 
-    def _transform_predict_input(self, X):
-        return to_csr_matrix(X, binary=True)
-
-    def _check_prediction(self, X_pred: csr_matrix, X: csr_matrix) -> None:
-        """Warn when a user with history got no recommendation (base.py:108-127)."""
-        has_hist = np.diff(X.indptr) > 0
-        has_pred = np.diff(X_pred.indptr) > 0
-        if X_pred.nnz and not np.all(X_pred.data):  # explicit zeros do not count as recommendations
-            has_pred = np.asarray((X_pred != 0).sum(axis=1)).ravel() > 0
-        missing = int(np.count_nonzero(has_hist & ~has_pred))
-        if missing > 0:
-            warnings.warn(f"{self.name} failed to recommend any items for {missing} users")
-
     def _check_fit_complete(self):
         """check_is_fitted + "missing similar items" (base.py:257-279); the device-resident fit result answers
         from its row lengths without building the host matrix."""
@@ -241,10 +247,15 @@ def predict_with_model(engine, ensure_model, X: csr_matrix, I: int, predict_topK
         X, _, _, ptr_d, idx_d = device_structure(X, engine.device)
         top = engine.predict_topn(U, ptr_d, idx_d, N, mask_history=bool(remove_history))
         engine.sync()
+    return topn_result(top, I, engine.device)
+
+
+def topn_result(top, I: int, device: int) -> csr_matrix:
+    """The CSR of device-resident top-N lists (dict(idx, val, len), rank order) that carries them for the metrics."""
     idx, val, ln = to_host(top["idx"], top["val"], top["len"])
     M = lists_to_csr(idx, val, ln, I, attach=True)
     # the metrics read the lists where they are, as long as the matrix still is what predict returned
-    M._rpk_topn_dev = (top["idx"], top["len"], engine.device)
+    M._rpk_topn_dev = (top["idx"], top["len"], device)
     M._rpk_topn_sig = matrix_signature(M)
     return M
 

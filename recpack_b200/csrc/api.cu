@@ -308,6 +308,27 @@ int rpk_embed_screen_f32(rpk_ctx* ctx, int64_t I, int D, const double* E, int si
   RPK_API_END(ctx)
 }
 
+int rpk_factor_topn(rpk_ctx* ctx, int64_t U, int64_t I, int D, const double* P, const double* Q, int64_t nnz,
+                    const int64_t* indptr, const int32_t* indices, int N, int mask_history, int32_t* out_idx, double* out_val,
+                    int32_t* out_len) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_factor_topn(ctx, U, I, D, P, Q, nnz, indptr, indices, N, mask_history, out_idx, out_val, out_len);
+  RPK_API_END(ctx)
+}
+
+int rpk_factor_full(rpk_ctx* ctx, int64_t U, int64_t I, int D, const double* P, const double* Q, int64_t nnz,
+                    const int64_t* indptr, const int32_t* indices, int mask_history, double* out_scores) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_factor_full(ctx, U, I, D, P, Q, nnz, indptr, indices, mask_history, out_scores);
+  RPK_API_END(ctx)
+}
+
+int rpk_factor_screen_f32(rpk_ctx* ctx, int64_t U, int64_t I, int D, const double* P, const double* Q, float* out_S) {
+  RPK_API_BEGIN(ctx)
+  rpk::run_factor_screen_f32(ctx, U, I, D, P, Q, out_S);
+  RPK_API_END(ctx)
+}
+
 int rpk_last_timings(rpk_ctx* ctx, double* out_ms) {
   RPK_API_BEGIN(ctx)
   if (!out_ms) throw rpk::Error("out_ms must not be null");

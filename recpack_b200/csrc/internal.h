@@ -72,5 +72,11 @@ void run_gram_dense_tc(rpk_ctx* c, const unsigned char* A, int64_t rows_pad, int
 void run_embed_topk(rpk_ctx* c, int64_t I, int D, const double* E, int similarity, int K, int64_t item_begin,
                     int64_t item_end, int32_t* out_idx, double* out_val, int32_t* out_len);
 void run_embed_screen_f32(rpk_ctx* c, int64_t I, int D, const double* E, int similarity, float* out_S);
+void run_factor_topn(rpk_ctx* c, int64_t U, int64_t I, int D, const double* P, const double* Q, int64_t nnz,
+                     const int64_t* indptr, const int32_t* indices, int N, int mask_history, int32_t* out_idx,
+                     double* out_val, int32_t* out_len);
+void run_factor_full(rpk_ctx* c, int64_t U, int64_t I, int D, const double* P, const double* Q, int64_t nnz,
+                     const int64_t* indptr, const int32_t* indices, int mask_history, double* out_scores);
+void run_factor_screen_f32(rpk_ctx* c, int64_t U, int64_t I, int D, const double* P, const double* Q, float* out_S);
 
 }  // namespace rpk

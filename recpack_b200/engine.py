@@ -243,6 +243,42 @@ class Engine:
                                                    _addr(out, np.float32)))
         return out
 
+    # -- factor models: user x item factor products ----------------------------------------
+    def factor_topn(self, P, Q, indptr, indices, N, mask_history=True, want_val=True):
+        """rpk_factor_topn: the N best stored scores of P @ Q.T per user with history in X (indptr / indices), float64
+        factors [U, D] / [I, D].  Returns dict(idx, val, len), rank order, next to the factors (torch CUDA or numpy)."""
+        U, D = (int(n) for n in P.shape)
+        I = int(Q.shape[0])
+        out = {
+            "idx": _empty_like_kind(P, (U, N), np.int32),
+            "val": _empty_like_kind(P, (U, N), np.float64) if want_val else None,
+            "len": _empty_like_kind(P, (U,), np.int32),
+        }
+        self._check(self._lib.rpk_factor_topn(
+            self._h, U, I, D, _addr(P, np.float64), _addr(Q, np.float64), int(indices.shape[0]), _addr(indptr, np.int64),
+            _addr(indices, np.int32), int(N), int(bool(mask_history)), _addr(out["idx"], np.int32),
+            _addr(out["val"], np.float64, allow_none=True), _addr(out["len"], np.int32)))
+        return out
+
+    def factor_full(self, P, Q, indptr, indices, mask_history=False):
+        """rpk_factor_full: every score as float64 [U, I] (0.0 = not stored) next to the factors."""
+        U, D = (int(n) for n in P.shape)
+        I = int(Q.shape[0])
+        out = _empty_like_kind(P, (U, I), np.float64)
+        self._check(self._lib.rpk_factor_full(
+            self._h, U, I, D, _addr(P, np.float64), _addr(Q, np.float64), int(indices.shape[0]), _addr(indptr, np.int64),
+            _addr(indices, np.int32), int(bool(mask_history)), _addr(out, np.float64)))
+        return out
+
+    def factor_screen_f32(self, P, Q):
+        """rpk_factor_screen_f32: the screen's approximate [U, I] float32 matrix (verification entry)."""
+        U, D = (int(n) for n in P.shape)
+        I = int(Q.shape[0])
+        out = _empty_like_kind(P, (U, I), np.float32)
+        self._check(self._lib.rpk_factor_screen_f32(self._h, U, I, D, _addr(P, np.float64), _addr(Q, np.float64),
+                                                    _addr(out, np.float32)))
+        return out
+
     # -- EASE: dense Gram, closed-form model, dense scoring ----------------------------------
     def gram_dense_f64(self, U, I, indptr, indices):
         """rpk_gram_dense_f64: exact X^T X of all users as float64 [I, I] (torch CUDA tensor when the inputs are)."""
